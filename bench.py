@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the liuzhou_b200 hot path (contract: see README / DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload selfplay|playout] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by the driver through torchrun (one rank per GPU, NCCL); games are independent, so ranks
 shard the games with no data-path collective ("scaling": "weak").  Rank 0 prints ONE JSON line.
@@ -165,6 +166,36 @@ class L2Flusher:
 
     def flush(self):
         self.buf.add_(1)
+
+
+DUMP_LIMIT_BYTES = 60 << 20          # array data; with the .npy headers a dump stays under 64 MB (64e6 bytes)
+
+
+def dump_outputs(out_dir: str, per_game: dict, other: dict) -> None:
+    """--dump-outputs: write what the timed path computed as DIR/<name>.npy -- float64 for 64-bit sources, float32
+    otherwise (exact for every array dumped here) -- so that two builds can be compared output for output.  The arrays
+    of `per_game` share their first dimension (the game); if everything would exceed DUMP_LIMIT_BYTES, the same fixed,
+    seeded sample of games is kept in each of them and its indices are written as games.npy."""
+    import numpy as np
+    import torch
+
+    def host(t):
+        wide = t.dtype in (torch.int64, torch.float64)
+        return t.detach().to("cpu", torch.float64 if wide else torch.float32).numpy()
+
+    rows = {k: host(v) for k, v in per_game.items()}
+    rest = {k: host(v) for k, v in other.items()}
+    n = next(iter(rows.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in rows.values())
+    keep = (DUMP_LIMIT_BYTES - sum(a.nbytes for a in rest.values())) // (row_bytes + 8)
+    if keep < n:
+        games = np.sort(np.random.default_rng(SEED).choice(n, keep, replace=False))
+        rows = {k: a[games] for k, a in rows.items()}
+        rest["games"] = games.astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in {**rows, **rest}.items():
+        np.save(out / f"{k}.npy", a)
 
 
 def reference_gpu_line(games: int, sims: int, device_index: int, timeout_s: float = 600.0) -> dict:
@@ -815,6 +846,17 @@ def run_selfplay(args, world, rank, local_rank):
     e1.synchronize()
     barrier_sync(world)
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        # the last timed ply: its trajectory rows (reference format), the positions after the move (finished games
+        # refilled), the ply counters and the running outcome counts
+        from liuzhou_b200 import native
+        from liuzhou_b200._lib import STATE_FIELDS
+
+        planes, legal, policy, sign = stepper.trajectory_block()
+        state = {f"state_{k}": t for k, t in zip(STATE_FIELDS, native.unpack_states(stepper.states))}
+        dump_outputs(args.dump_outputs, {"trajectory_planes": planes, "trajectory_legal_mask": legal,
+                                         "trajectory_policy": policy, "trajectory_sign": sign, **state,
+                                         "plies": stepper.plies}, {"outcomes": stepper.outcomes})
     # graph replays re-launch the captured kernels: our kernels inside the root / wave graphs were counted at capture
     waves = stepper.mcts.waves
     launches = (_lib.launch_count() - launches0) + args.steps * (waves * stepper.mcts.wave_graph_launches
@@ -1088,7 +1130,7 @@ def run_selfplay_root(args, world, rank, local_rank):
     if rank == 0:
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     positions = 0
     last = None
     e0.record(stream)
@@ -1396,14 +1438,27 @@ def main() -> int:
                     help="1: also time the UNMODIFIED v1 reference (its python + its v0_core CUDA) on the same GPU (N = 1)")
     ap.add_argument("--legacy-cpu", type=int, default=1, help="1: also time BASELINE configs[0] (legacy src/ self-play, CPU)")
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 5); config4 and eval time one whole run, so only 1 is accepted there")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--workload", choices=["playout", "selfplay", "eval", "config4"], default="selfplay")
     ap.add_argument("--eval-games", type=int, default=2000)
     ap.add_argument("--eval-sims", type=int, default=64)
     ap.add_argument("--eval-rr-games", type=int, default=256)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (default self-play "
+                         "workload; rank 0's games)")
     args = ap.parse_args()
+    if args.workload in ("config4", "eval") and args.impl == "ours":
+        if args.steps not in (None, 1):
+            ap.error(f"--workload {args.workload} times one whole run: --steps must be 1")
+        args.steps = 1
+    args.steps = 5 if args.steps is None else args.steps
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl, args.workload, args.search) != ("ours", "selfplay", "tree"):
+        ap.error("--dump-outputs is implemented for the default workload (--impl ours --workload selfplay --search tree)")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":

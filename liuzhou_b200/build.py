@@ -7,6 +7,8 @@ nvcc cross-compiles without a GPU; the resulting .so travels to the GPU box with
 from __future__ import annotations
 
 import argparse
+import os
+import shutil
 import subprocess
 import sys
 from concurrent.futures import ThreadPoolExecutor
@@ -20,6 +22,17 @@ NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",
 ]
+
+
+def nvcc() -> str:
+    """nvcc from PATH, else from $CUDA_HOME or the toolkit's default location."""
+    found = shutil.which("nvcc")
+    if found:
+        return found
+    for home in (os.environ.get("CUDA_HOME"), "/usr/local/cuda"):
+        if home and (Path(home) / "bin" / "nvcc").is_file():
+            return str(Path(home) / "bin" / "nvcc")
+    raise RuntimeError("nvcc not found: put the CUDA toolkit's bin directory on PATH or set CUDA_HOME")
 
 
 def sources() -> list[Path]:
@@ -45,7 +58,7 @@ def build(force: bool = False, verbose: bool = False) -> Path:
     for src in sources():
         obj = src.with_suffix(".o")
         objs.append(str(obj))
-        cmd = ["nvcc", *NVCC_FLAGS, f"-I{INCLUDE}", "-c", str(src), "-o", str(obj)]
+        cmd = [nvcc(), *NVCC_FLAGS, f"-I{INCLUDE}", "-c", str(src), "-o", str(obj)]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
         cmds.append(cmd)
@@ -59,7 +72,7 @@ def build(force: bool = False, verbose: bool = False) -> Path:
 
     with ThreadPoolExecutor(max_workers=8) as pool:
         list(pool.map(run, cmds))
-    run(["nvcc", "-shared", "-gencode", "arch=compute_100a,code=sm_100a", *objs, "-o", str(LIB)])
+    run([nvcc(), "-shared", "-gencode", "arch=compute_100a,code=sm_100a", *objs, "-o", str(LIB)])
     return LIB
 
 

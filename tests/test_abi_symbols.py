@@ -31,7 +31,8 @@ def test_library_is_sm100a_only():
 
     from liuzhou_b200 import build
 
-    out = subprocess.run(["cuobjdump", "-lelf", str(build.build())], capture_output=True, text=True).stdout
+    cuobjdump = str(Path(build.nvcc()).with_name("cuobjdump"))
+    out = subprocess.run([cuobjdump, "-lelf", str(build.build())], capture_output=True, text=True, check=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 

@@ -85,13 +85,48 @@ def test_scalar_api_errors_and_per_phase_functions():
     assert back[0] == s and back[1] == s2 and back[2] == s3 and back[2].move_count == 1
 
 
+def _stored_reference_playouts(v):
+    """tests/golden/scalar_playouts.npz -- 24 playouts decided by the reference's scalar engine: every state's legal
+    action indices and the state each chosen move led to -- through generate_all_legal_moves_struct / apply_move_struct."""
+    z = load_golden("scalar_playouts")
+    st = {k: z[k] for k in STATE_FIELDS}
+
+    def state(i):
+        s = v.GameState()
+        s.board = [[int(x) for x in row] for row in st["board"][i]]
+        s.marked_black = [(int(r), int(c)) for r, c in zip(*np.nonzero(st["marks_black"][i]))]
+        s.marked_white = [(int(r), int(c)) for r, c in zip(*np.nonzero(st["marks_white"][i]))]
+        s.phase, s.current_player = v.Phase(int(st["phase"][i])), v.Player(int(st["current_player"][i]))
+        for k in STATE_FIELDS[5:]:
+            setattr(s, k, int(st[k][i]))
+        return s
+
+    gp, checked = z["game_ptr"], 0
+    for g in range(len(gp) - 1):
+        for i in range(gp[g], gp[g + 1] - 1, 3):
+            s, nxt = state(i), state(i + 1)
+            moves = v.generate_all_legal_moves_struct(s)
+            assert sorted(m.action_index() for m in moves) == list(z["legal_idx"][z["legal_ptr"][i]:z["legal_ptr"][i + 1]])
+            got = v.apply_move_struct(s, next(m for m in moves if m.action_index() == int(z["chosen"][i])))
+            assert got.board == nxt.board and int(got.phase) == int(nxt.phase)
+            assert sorted(got.marked_black) == sorted(nxt.marked_black)
+            assert sorted(got.marked_white) == sorted(nxt.marked_white)
+            assert int(got.current_player) == int(nxt.current_player)
+            for k in STATE_FIELDS[5:]:
+                assert getattr(got, k) == getattr(nxt, k), (i, k)
+            checked += 1
+    assert checked > 500
+
+
 def test_scalar_api_vs_reference_objects():
-    """Call for call against the reference's own v0_core objects on states of oracle playouts (all phases)."""
+    """Call for call against the reference's own v0_core objects on states of oracle playouts (all phases); without
+    oracle/_ref, against the playouts the reference's scalar engine stored in tests/golden."""
+    from liuzhou_b200 import v0_core as v
+
     ref = load_ref()
     if ref is None:
-        pytest.skip("oracle/_ref not built")
+        return _stored_reference_playouts(v)
     rv, _ = ref
-    from liuzhou_b200 import v0_core as v
 
     def to_ref(s):
         r = rv.GameState()

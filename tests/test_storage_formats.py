@@ -1,7 +1,8 @@
 """Self-play payload files (SURVEY 8b: `run_self_play_worker` + `v1_sharded_shard` / `v1_worker_chunk_manifest` /
 `v1_sharded_manifest`; 8f-2 asynchronous writer).  CPU tests: our helpers vs golden vectors produced by the reference's
-python (tests/golden/make_storage_golden.py) and -- when /root/reference is present -- the reference's own loader
-opening the files we write.  GPU test: the worker end to end on a tiny configuration."""
+python (tests/golden/make_storage_golden.py) and -- when oracle/build_ref.py has put the reference's build and python
+copy into oracle/_ref -- the reference's own loader opening the files we write.  GPU test: the worker end to end on a
+tiny configuration."""
 import json
 import os
 import sys
@@ -14,7 +15,7 @@ from liuzhou_b200 import self_play_storage as st
 from liuzhou_b200.trajectory_buffer import TensorSelfPlayBatch
 
 GOLDEN = Path(__file__).resolve().parent / "golden" / "storage_formats.json"
-REFERENCE = Path("/root/reference")
+REF_DIR = Path(__file__).resolve().parents[1] / "oracle" / "_ref"
 
 PLAN_GRID = [
     dict(total_samples=0, num_shards=4),
@@ -248,16 +249,14 @@ def test_worker_manifest_merge_and_reference_loader(tmp_path):
     assert man["metadata"]["value_target_summary"]["total"] == 733
     loaded, stats, meta = st.load_self_play_payload(out)
     _eq_batches(loaded, st.concat_batches([b0, b1]))          # worker-major, chunk order
-    if not REFERENCE.is_dir():
-        pytest.skip("reference python not present: cross-loading by the reference's own loader skipped")
+    if not (REF_DIR / "pysrc" / "v1").is_dir():
+        pytest.skip("oracle/_ref/pysrc not present: cross-loading by the reference's own loader skipped")
     saved_path = list(sys.path)
-    sys.path[:0] = [str(REFERENCE), str(Path(__file__).resolve().parents[1] / "oracle" / "_ref")]
+    sys.path[:0] = [str(REF_DIR / "pysrc"), str(REF_DIR)]
     try:
         import v1.train as T
         from v1.python.self_play_types import SelfPlayV1Stats as RefStats
         from v1.python.trajectory_buffer import TensorSelfPlayBatch as RefBatch
-    except Exception as exc:                                   # pragma: no cover - reference import needs oracle/_ref
-        pytest.skip(f"reference v1.train not importable: {exc}")
     finally:
         sys.path[:] = saved_path
     ref_batch, ref_stats, ref_meta = T._load_self_play_payload(out)
