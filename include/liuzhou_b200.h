@@ -328,17 +328,11 @@ LZB_API int lzb_conv_bf16(const void *x, const void *w, int64_t n, int32_t cin, 
  * memory / tensor memory across all layers; the residual stream is kept in fp32.
  * planes bf16 [n,6,6,64] (lzb_encode_inputs_packed layout 2; channels 16..63 MUST be zero -- the stem only multiplies the
  * first 16 channels, the network has 11); w_stem bf16 [9][128][64]; w_trunk bf16 [2*blocks*9+1][128][128]
- * (conv1_0, conv2_0, ..., heads 1x1; tap-major, K-major rows, BatchNorm folded where it follows a conv), stored w_copies
- * times back to back (cluster c streams copy c % w_copies: spreads the L2 traffic of the hot weight lines); params f32 in
+ * (conv1_0, conv2_0, ..., heads 1x1; tap-major, K-major rows, BatchNorm folded where it follows a conv); params f32 in
  * DEVICE memory, compact: stem bias | scale | shift (384), per block conv1 bias (128) + conv2 scale | shift (256), heads
  * conv bias (128) -- copied to constant memory in stream order at every launch; blocks <= 10; out bf16 [n,6,6,128]. */
-LZB_API int lzb_trunk_bf16(const void *planes, int64_t n, const void *w_stem, const void *w_trunk, int32_t w_copies,
-                           const float *params, int32_t blocks, void *out, void *stream);
-/* lzb_trunk_bf16 that also publishes per-tile completion for an overlapped heads launch: tile_done = device int32
- * [ceil(n / 3) + 1], ALL ZERO on entry; entry i becomes 1 when boards [3 i, 3 i + 3) of `out` are complete.  Consumed and
- * zeroed again by lzb_heads_tail_overlapped, which must be the next launch on the stream. */
-LZB_API int lzb_trunk_bf16_signal(const void *planes, int64_t n, const void *w_stem, const void *w_trunk, int32_t w_copies,
-                                  const float *params, int32_t blocks, void *out, int32_t *tile_done, void *stream);
+LZB_API int lzb_trunk_bf16(const void *planes, int64_t n, const void *w_stem, const void *w_trunk, const float *params,
+                           int32_t blocks, void *out, void *stream);
 
 /* Fused network heads: everything of PolicyHead / ValueHead after their 1x1 convolutions
  * (src/neural_network.py:98-151: global pooling, gpool_linear, bn2 + relu, the three output convs,
@@ -355,14 +349,6 @@ LZB_API int lzb_heads_tail(const void *pv, int64_t n, int32_t pc, int32_t vc, in
                            const float *wfc1_t, const float *bfc1, const float *wfc2_t, const float *bfc2,
                            const uint64_t *states, float *priors, float *values, float *log_heads,
                            float *value_logits, void *stream);
-/* lzb_heads_tail as a programmatic dependent of the preceding lzb_trunk_bf16_signal launch: blocks start as trunk CTAs
- * finish and wait per 8-state tile for the producer's tile_done flags, so the heads of finished tiles run under the trunk
- * kernel's tail (its last scheduling round leaves most SMs idle).  The last block zeroes tile_done again. */
-LZB_API int lzb_heads_tail_overlapped(const void *pv, int64_t n, int32_t pc, int32_t vc, int32_t mlp, int32_t bins,
-                                      const float *wgl_t, const float *bn2_scale, const float *bn2_shift, const float *wout,
-                                      const float *wfc1_t, const float *bfc1, const float *wfc2_t, const float *bfc2,
-                                      const uint64_t *states, float *priors, float *values, float *log_heads,
-                                      float *value_logits, int32_t *tile_done, void *stream);
 
 #ifdef __cplusplus
 }

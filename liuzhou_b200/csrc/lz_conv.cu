@@ -1,42 +1,49 @@
 // lz_conv.cu -- the network's 3x3 / 1x1 convolutions as hand-written tcgen05 implicit GEMMs (sm_100a) with the
 // whole pre-activation-ResNet epilogue fused in (replaces cuDNN conv + our bn_relu pass; src/neural_network.py:83-96).
+// The fused trunk kernel (lz_trunk.cu) runs a net of up to 10 blocks in one launch; this per-layer path runs deeper nets.
 //
 // One launch = one convolution layer over the whole wave batch:
 //     D[rows = n*36, 128] = sum over taps (ky,kx) of  A_tap[rows, Cin] * W_tap[Cin, 128]        (bf16 x bf16 -> fp32)
-// * A operand: activations bf16 NHWC [n,6,6,Cin]; each tap's shifted, zero-padded [128 rows x 64 ch] tile is fetched
-//   by ONE TMA im2col load (cp.async.bulk.tensor.4d.im2col, SWIZZLE_128B) -- the hardware does the halo.
-// * B operand: the layer's weights [tap][cout][cin] stay RESIDENT in shared memory for the whole launch: a CTA
-//   pair (cta_group::2, cluster of 2) splits Cout, so each CTA holds 9 x 64 x 128 bf16 = 147 KB.  Only A streams.
+// * A operand: all taps are served from shared-memory-resident padded boards.  A CTA tile is 3 WHOLE boards kept in a
+//   padded row space,
+//       row(b, y, x) = b * 42 + (y + 1) * 6 + x,     y = -1 .. 5   (y = -1: a zero row above every board),
+//   and a tap (dy, dx) is an MMA whose A descriptor simply STARTS 6 * (dy + 1) rows into that buffer: the tensor core
+//   applies the 128-byte swizzle on absolute shared-memory address bits, so a descriptor may start on any 128-byte row
+//   (measured, tools/probe/umma_shift_probe.cu: base_offset = 0 works for every row shift).  The x shift cannot share
+//   rows (no pad column: that would cost 1/7 of the MMA rows again), so there is one copy per dx, each written by ONE
+//   tiled TMA load whose box starts at x = dx, y = -1: the out-of-bounds column / row arrive as zeros.  A tile therefore
+//   loads 3 copies instead of 9 taps (83 KB instead of 288 KB of real bytes per CTA), the rows b * 42 + 36 .. 41 of the
+//   accumulator are junk (the price: 108 useful rows of 128), rows 126 .. 135 of every copy are a zero block written once.
+//   The three dx copies are the A pipeline stages (the producer runs one tile ahead).
+// * B operand: a ring of weight stages (one tap each); a CTA pair (cta_group::2, cluster of 2) splits Cout, so each CTA
+//   loads its 64-cout half of every tap.
 // * MMA: tcgen05.mma.cta_group::2.kind::f16, M = 256 (128 rows per CTA), N = 128, K = 16; fp32 accumulators in
 //   TMEM, double buffered (2 x 128 columns) so the epilogue of tile i overlaps the MMAs of tile i+1.
-// * Persistent: 74 clusters walk the 256-row tiles round-robin.  Warp roles per CTA: warp 0 = TMA producer,
+// * Persistent: up to 74 clusters walk the pair tiles round-robin.  Warp roles per CTA: warp 0 = TMA producer,
 //   warp 1 = TMEM allocator + (leader CTA) MMA issuer, warps 2-9 = epilogue (TMEM lane quarter x column half).
 // * Epilogue (per row, fp32): v = acc + bias[c] (+ residual[row][c]); optional ReLU; out1 = bf16(v);
 //   out2 = bf16(relu(scale[c] * float(out1) + shift[c])).  With BatchNorm folded this covers
 //       conv1 of a block : out1 = relu(bn2(conv1(a)))                      (bias, relu)
 //       conv2 of a block : out1 = x + conv2(h) ; out2 = relu(bn1_next(out1)) (residual, both outputs)
 //       stem             : out1 = relu(stem_bn(conv(x))) ; out2 = relu(bn1_0(out1)).
-// Algorithmic work per launch (C = 128): 2 * rows * 128 * 1152 FLOP; bytes: rows * 256 B read (x9 from L2) +
-// rows * 256 B per output (+ residual).
+// Algorithmic work per launch (C = 128): 2 * rows * 128 * 1152 FLOP; bytes: rows * 256 B read + rows * 256 B per
+// output (+ residual).
 #include <cuda.h>
-#include <stdlib.h>
 #include <cuda_bf16.h>
 
 #include "lz_common.cuh"
+#include "lz_tc.cuh"
 
 namespace lzb {
 namespace {
+using namespace tc;
 
 constexpr int kConvThreads = 320;                // warp 0 producer, warp 1 MMA, warps 2-9 epilogue
-constexpr int kStages = 4;                       // pipeline depth (one stage = one tap: A [128 x Cin] + this CTA's half of W_tap)
-constexpr int kTileM = 128;                      // rows per CTA (256 per CTA pair)
 constexpr int kCout = 128;
-constexpr int kKC = 64;                          // channels per pipeline stage: 64 bf16 = one 128 B swizzle row
-constexpr uint32_t kChunkBytes = kTileM * kKC * 2;        // 16 KB: [128 rows x 64 ch], one TMA im2col load
+constexpr int kKC = 64;                          // channels per 128 B swizzle row
 constexpr uint32_t kWSlotBytes = (kCout / 2) * kKC * 2;   // 8 KB: 64 couts (this CTA's half) x 64 cin
 constexpr int kAccStages = 2;
 constexpr uint32_t kTmemCols = kAccStages * kCout;        // 256 fp32 columns
-constexpr uint64_t kWatchdogCycles = 4000000000ull;       // ~2 s: a lost arrival traps instead of hanging the GPU
 
 struct ConvParams {
     const float* bias;                 // [128] or null
@@ -45,365 +52,10 @@ struct ConvParams {
     const float* shift;
     __nv_bfloat16* out1;               // [rows,128] or null
     __nv_bfloat16* out2;               // [rows,128] or null
-    int64_t rows;                      // n * 36, multiple of 256
     int relu1;
     int images;                        // n
-    unsigned long long* trace;         // debug: clock64 stamps of cluster 0's leader (MMA thread: [0,4096), producer: [4096,8192))
-    int debug;                         // bit 0: epilogue drains TMEM but skips global loads / stores (timing experiments)
 };
 
-// ---- PTX wrappers -------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ uint32_t mapa_rank(uint32_t addr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// Relaxed on purpose: this arrive only hands a TMEM accumulator back (ordered by tcgen05.fence::before_thread_sync);
-// a .release here is a MEMBAR.GPU that waits for the thread's outstanding global stores (~2,000 cycles per tile).
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
-    asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    return done;
-}
-__device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity) {
-    const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
-        if ((uint64_t)(clock64() - t0) > kWatchdogCycles) {
-            printf("lz_conv: mbarrier wait timed out (block %d thread %d bar 0x%x parity %u)\n", (int)blockIdx.x,
-                   (int)threadIdx.x, bar, parity);
-            __trap();
-        }
-    }
-}
-// fast path: one try_wait (which itself suspends the thread for a while); the watchdog only starts after it fails
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    if (!mbar_try_wait(bar, parity)) mbar_wait_slow(bar, parity);
-}
-// One lane of the (converged) warp; the compiler then knows the guarded region runs single-threaded and keeps the
-// tcgen05 / TMA operands in uniform registers (a plain `lane == 0` test makes it wrap every UTCHMMA / UTMALDG in a
-// divergence "waterfall" loop: ~80 cycles per instruction instead of ~10).
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void prefetch_tmap(const CUtensorMap* m) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
-}
-constexpr uint64_t kL2Default = 0x1000000000000000ull;   // the default L2 cache-hint descriptor
-
-// im2col load of [128 pixels x 64 ch] starting at base pixel (w, h, n) with filter offsets (off_w, off_h); the
-// transaction bytes are signalled on `bar` (an address in the LEADER CTA's window: cta_group::2).
-__device__ __forceinline__ void tma_im2col_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c, int w, int h, int n,
-                                               uint16_t off_w, uint16_t off_h) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.im2col.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-        " [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8}, %9;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h),
-          "l"(kL2Default)
-        : "memory");
-}
-__device__ __forceinline__ void tma_tile2d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-        " [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "l"(kL2Default)
-        : "memory");
-}
-
-// K-major, SWIZZLE_128B shared-memory matrix descriptor (rows of 128 B, 8-row groups 1024 B apart).
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) {
-    return (uint64_t)((saddr >> 4) & 0x3FFFu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
-// kind::f16 instruction descriptor: D = f32, A = B = bf16, both K-major, N = 128, M = 256 (cta_group::2).
-constexpr uint32_t kInstrDesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kCout >> 3) << 17) | ((256u >> 4) << 24);
-
-__device__ __forceinline__ void umma_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(kInstrDesc), "r"(accumulate)
-        : "memory");
-}
-// all MMAs issued so far by this thread -> one arrival on `bar` in every CTA of `mask` when they complete
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-          "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-          "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<const uint32_t*>(&h);
-}
-
-// ---- the kernel ---------------------------------------------------------------------------------------------
-// TAPS = 9 (3x3, pad 1) or 1 (1x1); KCH = Cin / 64.
-template <int TAPS, int KCH>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kConvThreads, 1)
-conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, const ConvParams P) {
-    constexpr uint32_t kABytes = KCH * kChunkBytes;         // 32 KB
-    constexpr uint32_t kStageBytes = kABytes + KCH * kWSlotBytes;   // + 16 KB of weights = 48 KB
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;          // SWIZZLE_128B atoms need 1024 B alignment
-    const uint32_t a_smem = base;
-    const uint32_t bar0 = a_smem + kStages * kStageBytes;
-    // barriers (8 B each)
-    const uint32_t full_bar = bar0;                         // [kStages]    leader: A stage landed (both CTAs' bytes)
-    const uint32_t empty_bar = full_bar + 8 * kStages;      // [kStages]    both  : MMAs that read the stage are done
-    const uint32_t tfull_bar = empty_bar + 8 * kStages;     // [kAccStages] both  : accumulator complete
-    const uint32_t tempty_bar = tfull_bar + 8 * kAccStages; // [kAccStages] leader: epilogue of both CTAs drained it
-    const uint32_t tmem_slot = tempty_bar + 8 * kAccStages; // u32
-    const uint32_t vec_smem = (tmem_slot + 16 + 15u) & ~15u; // bias | scale | shift : 3 x 128 f32
-    const uint32_t stage_smem = vec_smem + 3 * kCout * 4;   // epilogue staging: 8 warps x 32 rows x 128 B (fp32)
-    uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
-    float* vec = reinterpret_cast<float*>(gen + (vec_smem - base));
-    volatile uint32_t* tmem_slot_p = reinterpret_cast<volatile uint32_t*>(gen + (tmem_slot - base));
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const bool leader = rank == 0;
-    const int cluster_id = blockIdx.x >> 1, num_clusters = gridDim.x >> 1;
-    const int64_t pair_tiles = P.rows / (2 * kTileM);
-
-    if (threadIdx.x == 0) {
-        prefetch_tmap(&tmA);
-        prefetch_tmap(&tmW);
-        for (int i = 0; i < kStages; ++i) { mbar_init(full_bar + 8 * i, 1); mbar_init(empty_bar + 8 * i, 1); }
-        for (int i = 0; i < kAccStages; ++i) { mbar_init(tfull_bar + 8 * i, 1); mbar_init(tempty_bar + 8 * i, 16); }
-        fence_barrier_init();
-    }
-    if (warp == 1) {   // TMEM: one warp per CTA, the pair allocates together
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    for (int i = threadIdx.x; i < kCout; i += kConvThreads) {
-        vec[i] = P.bias ? P.bias[i] : 0.0f;
-        vec[kCout + i] = P.scale ? P.scale[i] : 1.0f;
-        vec[2 * kCout + i] = P.shift ? P.shift[i] : 0.0f;
-    }
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();            // the peer's barriers exist before any remote arrive / multicast commit
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot_p;
-    // Programmatic dependent launch: everything above touched only constants and on-chip state.  Let the next
-    // layer's grid be scheduled as our SMs free up, and wait here until the previous layer's outputs are complete.
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-
-    if (warp == 0) {
-        // ===================== TMA producer (whole warp loops, one elected lane issues; both CTAs) ============
-        const uint32_t full_leader = mapa_rank(full_bar, 0);
-        uint32_t stage = 0, phase = 0;
-        int tr_p = 0;
-        for (int64_t pt = cluster_id; pt < pair_tiles; pt += num_clusters) {
-            const int64_t p0 = (2 * pt + rank) * kTileM;
-            const int n0 = (int)(p0 / 36), rem = (int)(p0 - (int64_t)n0 * 36), h0 = rem / 6, w0 = rem - h0 * 6;
-            for (int tap = 0; tap < TAPS; ++tap) {
-                const int off_w = TAPS == 9 ? tap % 3 : 0, off_h = TAPS == 9 ? tap / 3 : 0;
-                const int lo = TAPS == 9 ? -1 : 0;
-                mbar_wait(empty_bar + 8 * stage, phase ^ 1);
-                if (elect_one()) {
-                    if (P.trace && blockIdx.x == 0 && tr_p < 4096) P.trace[4096 + tr_p++] = clock64();
-                    if (P.debug & 2) {   // timing experiment: no loads, the MMAs chew on whatever is in smem
-                        if (leader) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(full_bar + 8 * stage) : "memory");
-                    } else {
-                        if (leader) mbar_arrive_expect_tx(full_bar + 8 * stage, 2 * kStageBytes);
-#pragma unroll
-                        for (int kc = 0; kc < KCH; ++kc) {
-                            tma_im2col_2sm(a_smem + stage * kStageBytes + kc * kChunkBytes, &tmA, full_leader + 8 * stage,
-                                           kc * kKC, w0 + lo, h0 + lo, n0, (uint16_t)off_w, (uint16_t)off_h);
-                            // this tap's weights: our half of Cout (the pair's MMA reads the other half from the peer)
-                            tma_tile2d_2sm(a_smem + stage * kStageBytes + kABytes + kc * kWSlotBytes, &tmW,
-                                           full_leader + 8 * stage, kc * kKC, tap * kCout + (int)rank * (kCout / 2));
-                        }
-                    }
-                }
-                __syncwarp();
-                if (++stage == kStages) { stage = 0; phase ^= 1; }
-            }
-        }
-    } else if (warp == 1) {
-        // ===================== MMA issuer (leader CTA; whole warp loops, one elected lane issues) =============
-        if (leader) {
-            uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
-            int tr_m = 0;
-            for (int64_t pt = cluster_id; pt < pair_tiles; pt += num_clusters) {
-                mbar_wait(tempty_bar + 8 * acc, acc_phase ^ 1);
-                tc_fence_after();
-                const uint32_t d_tmem = tmem_base + acc * kCout;
-                for (int tap = 0; tap < TAPS; ++tap) {
-                    mbar_wait(full_bar + 8 * stage, phase);
-                    tc_fence_after();
-                    if (elect_one()) {
-                        if (P.trace && blockIdx.x == 0 && tr_m < 4000) P.trace[tr_m++] = clock64();
-#pragma unroll
-                        for (int kc = 0; kc < KCH; ++kc) {
-                            const uint64_t adesc = umma_desc_sw128(a_smem + stage * kStageBytes + kc * kChunkBytes);
-                            const uint64_t bdesc = umma_desc_sw128(a_smem + stage * kStageBytes + kABytes + kc * kWSlotBytes);
-#pragma unroll
-                            for (int k = 0; k < kKC / 16; ++k)   // +32 B per K = 16 step inside the 128 B swizzle row
-                                if (!(P.debug & 4)) umma_2sm(d_tmem, adesc + 2 * k, bdesc + 2 * k, (uint32_t)((tap | kc | k) != 0));
-                        }
-                        umma_commit_2sm(empty_bar + 8 * stage, 3);              // frees the stage in both CTAs
-                        if (tap == TAPS - 1) umma_commit_2sm(tfull_bar + 8 * acc, 3);   // accumulator ready in both CTAs
-                        if (P.trace && blockIdx.x == 0 && tr_m < 4000) P.trace[tr_m++] = clock64();
-                    }
-                    __syncwarp();
-                    if (++stage == kStages) { stage = 0; phase ^= 1; }
-                }
-                if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
-            }
-        }
-    } else {
-        // ===================== epilogue: warps 2..9 =====================
-        // TMEM lane quarter = warp % 4 (hardware rule), column half = (warp - 2) / 4: each warp owns 32 rows x 64
-        // channels of the tile.  Per 32-column chunk: TMEM -> registers (lane = row) -> fp32 staging tile in shared
-        // memory (XOR-swizzled 16 B slots, conflict-free both ways) -> re-read so that 4 consecutive lanes own 32
-        // consecutive channels of one row: residual loads and both output stores are then full 32 B sectors,
-        // 8 rows per instruction.  The residual is prefetched into registers BEFORE waiting for the accumulator.
-        const int q = warp & 3, half = (warp - 2) >> 2;
-        const uint32_t tempty_leader = mapa_rank(tempty_bar, 0);
-        uint32_t acc = 0, acc_phase = 0;
-        float4* stg = reinterpret_cast<float4*>(gen + (stage_smem - base)) + (warp - 2) * (32 * 8);   // [32 rows][8 x 16 B]
-        const int sub = lane & 3, rsub = lane >> 2;          // channel octet within the chunk, row within a group of 8
-        const bool relu1 = P.relu1 != 0;
-        const bool no_io = (P.debug & 1) != 0;
-        int tr_e = 0;
-        for (int64_t pt = cluster_id; pt < pair_tiles; pt += num_clusters) {
-            const int64_t row0 = (2 * pt + rank) * kTileM + q * 32;
-            uint4 resv[2][4];
-            if (P.residual) {
-#pragma unroll
-                for (int jj = 0; jj < 2; ++jj)
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        resv[jj][k] = __ldg(reinterpret_cast<const uint4*>(P.residual) +
-                                            (((row0 + rsub + 8 * k) * kCout + half * 64 + jj * 32 + sub * 8) >> 3));
-            }
-            mbar_wait(tfull_bar + 8 * acc, acc_phase);
-            if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 2000) P.trace[2048 + tr_e++] = clock64();
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * kCout + half * 64;
-            uint32_t v[2][32];
-            tmem_ld32(taddr, v[0]);
-            tmem_ld32(taddr + 32, v[1]);
-            tmem_ld_wait();
-            if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 2000) P.trace[2048 + tr_e++] = clock64();
-            // the accumulator is in registers: hand the TMEM stage back to the MMA warp right away
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(tempty_leader + 8 * acc);
-            if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
-            if (no_io) continue;
-#pragma unroll
-            for (int jj = 0; jj < 2; ++jj) {
-                const int c0 = half * 64 + jj * 32 + sub * 8;
-                const float4 b0 = *reinterpret_cast<const float4*>(vec + c0), b1 = *reinterpret_cast<const float4*>(vec + c0 + 4);
-                const float4 s0 = *reinterpret_cast<const float4*>(vec + kCout + c0), s1 = *reinterpret_cast<const float4*>(vec + kCout + c0 + 4);
-                const float4 t0 = *reinterpret_cast<const float4*>(vec + 2 * kCout + c0), t1 = *reinterpret_cast<const float4*>(vec + 2 * kCout + c0 + 4);
-                const float2 bias2[4] = {make_float2(b0.x, b0.y), make_float2(b0.z, b0.w), make_float2(b1.x, b1.y), make_float2(b1.z, b1.w)};
-                const float2 scale2[4] = {make_float2(s0.x, s0.y), make_float2(s0.z, s0.w), make_float2(s1.x, s1.y), make_float2(s1.z, s1.w)};
-                const float2 shift2[4] = {make_float2(t0.x, t0.y), make_float2(t0.z, t0.w), make_float2(t1.x, t1.y), make_float2(t1.z, t1.w)};
-                __syncwarp();                                   // previous chunk's readers are done with the staging tile
-#pragma unroll
-                for (int f = 0; f < 8; ++f)
-                    stg[lane * 8 + (f ^ (lane & 7))] = make_float4(__uint_as_float(v[jj][4 * f]), __uint_as_float(v[jj][4 * f + 1]),
-                                                                   __uint_as_float(v[jj][4 * f + 2]), __uint_as_float(v[jj][4 * f + 3]));
-                __syncwarp();
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const int r = rsub + 8 * k;
-                    const float4 x0 = stg[r * 8 + ((2 * sub) ^ (r & 7))], x1 = stg[r * 8 + ((2 * sub + 1) ^ (r & 7))];
-                    float2 x[4] = {make_float2(x0.x, x0.y), make_float2(x0.z, x0.w), make_float2(x1.x, x1.y), make_float2(x1.z, x1.w)};
-                    const int64_t off = ((row0 + r) * kCout + c0) >> 3;            // in 16-byte units
-                    if (P.residual) {
-                        const uint32_t* rw = reinterpret_cast<const uint32_t*>(&resv[jj][k]);
-#pragma unroll
-                        for (int h = 0; h < 4; ++h)      // bf16 pair -> two floats: low half << 16, high half masked
-                            x[h] = __fadd2_rn(x[h], make_float2(__uint_as_float(rw[h] << 16), __uint_as_float(rw[h] & 0xffff0000u)));
-                    }
-                    uint32_t p1[4], p2[4];
-#pragma unroll
-                    for (int h = 0; h < 4; ++h) {
-                        float2 f = __fadd2_rn(x[h], bias2[h]);
-                        if (relu1) { f.x = fmaxf(f.x, 0.0f); f.y = fmaxf(f.y, 0.0f); }
-                        p1[h] = pack_bf16(f.x, f.y);
-                        // BN reads the stored (bf16) value: unpack the pair we just rounded
-                        const float2 sv = make_float2(__uint_as_float(p1[h] << 16), __uint_as_float(p1[h] & 0xffff0000u));
-                        const float2 g = __ffma2_rn(scale2[h], sv, shift2[h]);
-                        p2[h] = pack_bf16(fmaxf(g.x, 0.0f), fmaxf(g.y, 0.0f));
-                    }
-                    if (P.out1) reinterpret_cast<uint4*>(P.out1)[off] = make_uint4(p1[0], p1[1], p1[2], p1[3]);
-                    if (P.out2) reinterpret_cast<uint4*>(P.out2)[off] = make_uint4(p2[0], p2[1], p2[2], p2[3]);
-                }
-                if (jj == 0 && P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 2000) P.trace[2048 + tr_e++] = clock64();
-            }
-            if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 2000) P.trace[2048 + tr_e++] = clock64();
-        }
-    }
-
-    // teardown: every MMA / TMEM read of the pair is done before the pair frees TMEM
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-    }
-}
-
-// ---- second-generation kernel: all taps served from shared-memory-resident padded boards -------------------------------
-// The im2col kernel above fetches the A operand once per tap: 9 x 32 KB per 128-row tile, which makes the launch
-// operand-delivery bound (L2 -> SM), not tensor bound (profiles/r02_conv_decompose_v1.txt: MMAs alone 26 us, loads
-// alone 25 us, full kernel 38-54 us).  Here a CTA tile is 3 WHOLE boards kept in a padded row space,
-//     row(b, y, x) = b * 42 + (y + 1) * 6 + x,     y = -1 .. 5   (y = -1: a zero row above every board),
-// and a tap (dy, dx) is an MMA whose A descriptor simply STARTS 6 * (dy + 1) rows into that buffer: the tensor core
-// applies the 128-byte swizzle on absolute shared-memory address bits, so a descriptor may start on any 128-byte row
-// (measured, tools/probe/umma_shift_probe.cu: base_offset = 0 works for every row shift).  The x shift cannot share
-// rows (no pad column: that would cost 1/7 of the MMA rows again), so there is one copy per dx, each written by ONE
-// tiled TMA load whose box starts at x = dx, y = -1: the out-of-bounds column / row arrive as zeros.  A tile therefore
-// loads 3 copies instead of 9 taps (83 KB instead of 288 KB of real bytes per CTA), the rows b * 42 + 36 .. 41 of the
-// accumulator are junk (the price: 108 useful rows of 128), rows 126 .. 131 of every copy are a zero block written once.
-// Pipelines: 3 A stages = the dx copies (the producer runs one tile ahead), a separate ring of weight stages (one tap
-// each), TMEM accumulators double buffered; warp roles and the fused epilogue are those of the kernel above.
 constexpr int kBoards = 3;                               // boards per CTA tile
 constexpr int kBoardRows = 42;                           // padded rows per board
 constexpr int kBoxRows = kBoards * kBoardRows;           // 126 rows written by one TMA box
@@ -411,14 +63,6 @@ constexpr int kBufRows = 136;                            // rows per chunk buffe
 constexpr uint32_t kPChunkBytes = kBufRows * 128;        // 17,408 B = 17 x 1024
 constexpr uint32_t kPBoxBytes = kBoxRows * 128;          // 16,128 B per TMA load
 constexpr int kWStages = 4;
-
-__device__ __forceinline__ void tma_tile4d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c, int w, int h, int n) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-        " [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c), "r"(w), "r"(h), "r"(n), "l"(kL2Default)
-        : "memory");
-}
 
 template <int TAPS, int KCH>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kConvThreads, 1)
@@ -494,15 +138,11 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             for (int dxi = 0; dxi < NDX; ++dxi) {
                 mbar_wait(aempty_bar + 8 * dxi, aph ^ 1);
                 if (elect_one()) {
-                    if (P.debug & 2) {
-                        if (leader) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(afull_bar + 8 * dxi) : "memory");
-                    } else {
-                        if (leader) mbar_arrive_expect_tx(afull_bar + 8 * dxi, 2 * KCH * kPBoxBytes);
+                    if (leader) mbar_arrive_expect_tx(afull_bar + 8 * dxi, 2 * KCH * kPBoxBytes);
 #pragma unroll
-                        for (int kc = 0; kc < KCH; ++kc)     // box (64 ch, 6 x, 7 y, 3 boards) at x = dx, y = -1: zeros outside
-                            tma_tile4d_2sm(a_smem + dxi * kACopyBytes + kc * kPChunkBytes, &tmA, afull_leader + 8 * dxi,
-                                           kc * kKC, TAPS == 9 ? dxi - 1 : 0, -1, board0);
-                    }
+                    for (int kc = 0; kc < KCH; ++kc)     // box (64 ch, 6 x, 7 y, 3 boards) at x = dx, y = -1: zeros outside
+                        tma_tile4d_2sm(a_smem + dxi * kACopyBytes + kc * kPChunkBytes, &tmA, afull_leader + 8 * dxi,
+                                       kc * kKC, TAPS == 9 ? dxi - 1 : 0, -1, board0);
                 }
                 __syncwarp();
 #pragma unroll
@@ -510,15 +150,11 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                     const int tap = TAPS == 9 ? dyi * 3 + dxi : 0;
                     mbar_wait(wempty_bar + 8 * wst, wph ^ 1);
                     if (elect_one()) {
-                        if (P.debug & 2) {
-                            if (leader) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(wfull_bar + 8 * wst) : "memory");
-                        } else {
-                            if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * kWStageBytes);
+                        if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * kWStageBytes);
 #pragma unroll
-                            for (int kc = 0; kc < KCH; ++kc)
-                                tma_tile2d_2sm(w_smem + wst * kWStageBytes + kc * kWSlotBytes, &tmW, wfull_leader + 8 * wst,
-                                               kc * kKC, tap * kCout + (int)rank * (kCout / 2));
-                        }
+                        for (int kc = 0; kc < KCH; ++kc)
+                            tma_tile2d_2sm(w_smem + wst * kWStageBytes + kc * kWSlotBytes, &tmW, wfull_leader + 8 * wst,
+                                           kc * kKC, tap * kCout + (int)rank * (kCout / 2));
                     }
                     __syncwarp();
                     if (++wst == kWStages) { wst = 0; wph ^= 1; }
@@ -551,7 +187,7 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                                 const uint64_t bdesc = umma_desc_sw128(w_smem + wst * kWStageBytes + kc * kWSlotBytes);
 #pragma unroll
                                 for (int k = 0; k < kKC / 16; ++k)
-                                    if (!(P.debug & 4)) umma_2sm(d_tmem, adesc + 2 * k, bdesc + 2 * k, (uint32_t)((dxi | dyi | kc | k) != 0));
+                                    umma_2sm(d_tmem, adesc + 2 * k, bdesc + 2 * k, (uint32_t)((dxi | dyi | kc | k) != 0));
                             }
                             umma_commit_2sm(wempty_bar + 8 * wst, 3);
                             if (dyi == NDY - 1) umma_commit_2sm(aempty_bar + 8 * dxi, 3);      // the copy is free in both CTAs
@@ -567,7 +203,12 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         }
     } else {
         // ===================== epilogue: warps 2..9 =====================
-        // as above; accumulator row i = b * 42 + y * 6 + x of the tile <-> global pixel row (board0 + b) * 36 + y * 6 + x,
+        // TMEM lane quarter = warp % 4 (hardware rule), column half = (warp - 2) / 4: each warp owns 32 rows x 64
+        // channels of the tile.  Per 32-column chunk: TMEM -> registers (lane = row) -> fp32 staging tile in shared
+        // memory (XOR-swizzled 16 B slots, conflict-free both ways) -> re-read so that 4 consecutive lanes own 32
+        // consecutive channels of one row: residual loads and both output stores are then full 32 B sectors,
+        // 8 rows per instruction.  The residual is prefetched into registers BEFORE waiting for the accumulator.
+        // Accumulator row i = b * 42 + y * 6 + x of the tile <-> global pixel row (board0 + b) * 36 + y * 6 + x,
         // rows with i % 42 >= 36 (the pad row between boards), i >= 126 or a board beyond the batch are junk: skipped
         const int q = warp & 3, half = (warp - 2) >> 2;
         const uint32_t tempty_leader = mapa_rank(tempty_bar, 0);
@@ -575,7 +216,6 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         float4* stg = reinterpret_cast<float4*>(gen + (stage_smem - base)) + (warp - 2) * (32 * 8);
         const int sub = lane & 3, rsub = lane >> 2;
         const bool relu1 = P.relu1 != 0;
-        const bool no_io = (P.debug & 1) != 0;
         int rem4[4], b4[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -612,7 +252,6 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(tempty_leader + 8 * acc);
             if (++acc == kAccStages) { acc = 0; acc_phase ^= 1; }
-            if (no_io) continue;
 #pragma unroll
             for (int jj = 0; jj < 2; ++jj) {
                 const int c0 = half * 64 + jj * 32 + sub * 8;
@@ -670,81 +309,10 @@ conv_pad_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-typedef CUresult (*EncodeIm2colFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                   const int*, const int*, cuuint32_t, cuuint32_t, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 bool driver_entry(const char* name, void** fn) {
     cudaDriverEntryPointQueryResult st;
     return cudaGetDriverEntryPoint(name, fn, cudaEnableDefault, &st) == cudaSuccess && st == cudaDriverEntryPointSuccess &&
            *fn != nullptr;
-}
-
-template <int TAPS, int KCH>
-int launch_conv(const void* x, const void* w, const ConvParams& P, cudaStream_t stream) {
-    static EncodeTiledFn encode_tiled = nullptr;
-    static EncodeIm2colFn encode_im2col = nullptr;
-    if (!encode_tiled && !driver_entry("cuTensorMapEncodeTiled", reinterpret_cast<void**>(&encode_tiled))) {
-        set_error("lzb_conv: cuTensorMapEncodeTiled unavailable");
-        return LZB_ERR_CUDA;
-    }
-    if (!encode_im2col && !driver_entry("cuTensorMapEncodeIm2col", reinterpret_cast<void**>(&encode_im2col))) {
-        set_error("lzb_conv: cuTensorMapEncodeIm2col unavailable");
-        return LZB_ERR_CUDA;
-    }
-    constexpr int cin = KCH * kKC;
-    alignas(64) CUtensorMap tmA, tmW;
-    {   // activations: (C, W, H, N) bf16, NHWC
-        const cuuint64_t dim[4] = {(cuuint64_t)cin, 6, 6, (cuuint64_t)P.images};
-        const cuuint64_t stride[3] = {(cuuint64_t)cin * 2, (cuuint64_t)cin * 2 * 6, (cuuint64_t)cin * 2 * 36};
-        const int pad = TAPS == 9 ? 1 : 0;
-        const int lower[2] = {-pad, -pad}, upper[2] = {-pad, -pad};   // pad - (filter - 1) * dilation = -pad for 3x3 / 1x1
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
-        const CUresult rc = encode_im2col(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), dim, stride, lower,
-                                          upper, kKC, kTileM, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (rc != CUDA_SUCCESS) { set_error("lzb_conv: cuTensorMapEncodeIm2col failed (%d)", (int)rc); return LZB_ERR_CUDA; }
-    }
-    {   // weights: [tap * 128 + cout][cin] bf16
-        const cuuint64_t dim[2] = {(cuuint64_t)cin, (cuuint64_t)TAPS * kCout};
-        const cuuint64_t stride[1] = {(cuuint64_t)cin * 2};
-        const cuuint32_t box[2] = {kKC, kCout / 2};
-        const cuuint32_t estr[2] = {1, 1};
-        const CUresult rc = encode_tiled(&tmW, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dim, stride, box, estr,
-                                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (rc != CUDA_SUCCESS) { set_error("lzb_conv: cuTensorMapEncodeTiled failed (%d)", (int)rc); return LZB_ERR_CUDA; }
-    }
-    constexpr size_t smem = 1024 + (size_t)kStages * KCH * (kChunkBytes + kWSlotBytes) +
-                            8 * (2 * kStages + 2 * kAccStages) + 32 + 3 * kCout * sizeof(float) + 8 * 32 * 128;
-    // the dynamic shared memory opt-in and the SM count are per DEVICE (a process may drive several GPUs)
-    static int sm_count[64] = {0};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { set_error("lzb_conv: bad current device"); return LZB_ERR_CUDA; }
-    if (sm_count[dev] == 0) {
-        if (cudaFuncSetAttribute(conv_tc_kernel<TAPS, KCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-            set_error("lzb_conv: cannot raise dynamic shared memory to %zu", smem);
-            return LZB_ERR_CUDA;
-        }
-        int n = 0;
-        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n < 2) n = kNumSMs;
-        sm_count[dev] = n;
-    }
-    const int64_t pair_tiles = P.rows / (2 * kTileM);
-    const int clusters = (int)(pair_tiles < sm_count[dev] / 2 ? pair_tiles : sm_count[dev] / 2);
-    static const bool pdl = !(getenv("LZB_CONV_PDL") && atoi(getenv("LZB_CONV_PDL")) == 0);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * clusters);
-    cfg.blockDim = dim3(kConvThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    if (cudaLaunchKernelEx(&cfg, conv_tc_kernel<TAPS, KCH>, tmA, tmW, P) != cudaSuccess) return check_launch("conv_tc_kernel");
-    return check_launch("conv_tc_kernel");
 }
 
 template <int TAPS, int KCH>
@@ -793,7 +361,6 @@ int launch_conv_pad(const void* x, const void* w, const ConvParams& P, cudaStrea
     }
     const int64_t pair_tiles = (P.images + 2 * kBoards - 1) / (2 * kBoards);
     const int clusters = (int)(pair_tiles < sm_count[dev] / 2 ? pair_tiles : sm_count[dev] / 2);
-    static const bool pdl = !(getenv("LZB_CONV_PDL") && atoi(getenv("LZB_CONV_PDL")) == 0);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2 * clusters);
     cfg.blockDim = dim3(kConvThreads);
@@ -803,7 +370,7 @@ int launch_conv_pad(const void* x, const void* w, const ConvParams& P, cudaStrea
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     if (cudaLaunchKernelEx(&cfg, conv_pad_kernel<TAPS, KCH>, tmA, tmW, P) != cudaSuccess) return check_launch("conv_pad_kernel");
     return check_launch("conv_pad_kernel");
 }
@@ -812,13 +379,6 @@ int launch_conv_pad(const void* x, const void* w, const ConvParams& P, cudaStrea
 }  // namespace lzb
 
 // x bf16 [n,6,6,cin] (NHWC), w bf16 [taps][128][cin], outputs bf16 [n,6,6,128]; n must be a multiple of 64.
-// debug: copy the clock64 trace of the last launches (LZB_CONV_DEBUG & 8) to host memory (8192 u64)
-static unsigned long long* g_trace_buf = nullptr;
-extern "C" __attribute__((visibility("default"))) int lzb_conv_debug_trace(unsigned long long* host_out) {
-    if (!g_trace_buf) return LZB_ERR_INVALID_ARGUMENT;
-    return cudaMemcpy(host_out, g_trace_buf, 8192 * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? LZB_OK : LZB_ERR_CUDA;
-}
-
 extern "C" int lzb_conv_bf16(const void* x, const void* w, int64_t n, int32_t cin, int32_t taps, const float* bias,
                              const void* residual, const float* scale, const float* shift, int32_t relu1, void* out1,
                              void* out2, void* stream) {
@@ -832,18 +392,7 @@ extern "C" int lzb_conv_bf16(const void* x, const void* w, int64_t n, int32_t ci
     lzb::ConvParams P;
     P.bias = bias; P.residual = reinterpret_cast<const __nv_bfloat16*>(residual); P.scale = scale; P.shift = shift;
     P.out1 = reinterpret_cast<__nv_bfloat16*>(out1); P.out2 = reinterpret_cast<__nv_bfloat16*>(out2);
-    P.rows = n * 36; P.relu1 = relu1; P.images = (int)n;
-    static const int debug = getenv("LZB_CONV_DEBUG") ? atoi(getenv("LZB_CONV_DEBUG")) : 0;
-    P.debug = debug;
-    if ((debug & 8) && !g_trace_buf) { cudaMalloc(&g_trace_buf, 8192 * 8); cudaMemset(g_trace_buf, 0, 8192 * 8); }
-    P.trace = g_trace_buf;
-    // LZB_CONV_IMPL = 1: the first-generation im2col kernel (one TMA load per tap); default: the padded-board kernel
-    static const int impl = getenv("LZB_CONV_IMPL") ? atoi(getenv("LZB_CONV_IMPL")) : 2;
-    if (impl == 1) {
-        if (cin == 64) return lzb::launch_conv<9, 1>(x, w, P, (cudaStream_t)stream);
-        if (taps == 9) return lzb::launch_conv<9, 2>(x, w, P, (cudaStream_t)stream);
-        return lzb::launch_conv<1, 2>(x, w, P, (cudaStream_t)stream);
-    }
+    P.relu1 = relu1; P.images = (int)n;
     if (cin == 64) return lzb::launch_conv_pad<9, 1>(x, w, P, (cudaStream_t)stream);
     if (taps == 9) return lzb::launch_conv_pad<9, 2>(x, w, P, (cudaStream_t)stream);
     return lzb::launch_conv_pad<1, 2>(x, w, P, (cudaStream_t)stream);

@@ -105,8 +105,6 @@ struct HeadsParams {
     const __nv_bfloat16* pv; int64_t n; int pc, vc, mlp, bins;
     const float *wgl_t, *bn2_scale, *bn2_shift, *wout, *wfc1_t, *bfc1, *wfc2_t, *bfc2;
     const uint64_t* states; float *priors, *values, *log_heads, *value_logits;
-    int* tile_done;      // optional (overlapped launch): per-3-board completion flags of pv's producer + a block counter
-    int trace;           // debug (LZB_OVERLAP_TRACE=1): globaltimer of every block's start into tile_done[4096 + 2 b]
 };
 
 __device__ __forceinline__ uint32_t to_tf32(float x) {
@@ -151,31 +149,9 @@ heads_tail_kernel(HeadsParams P) {
         wpol[2][i] = P.wout[i]; wpol[3][i] = P.wout[pc + i]; wpol[4][i] = P.wout[2 * pc + i];
     }
     const int64_t num_tiles = (P.n + kTile - 1) / kTile;
-    if (P.trace && P.tile_done && t == 0 && blockIdx.x < 1024) {
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        reinterpret_cast<unsigned long long*>(P.tile_done + 4096)[blockIdx.x] = gt;
-    }
     for (int64_t tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         const int64_t base = tile * kTile;
         const int ns = (int)min((int64_t)kTile, P.n - base);
-        if (P.tile_done) {
-            // overlapped launch: this kernel may run while the trunk kernel is still producing other tiles of pv.  Wait for
-            // the flags of the 3-board producer tiles that cover states [base, base + ns): acquire, then the block barrier
-            // below orders every thread's loads after it.  Bounded spin: a lost flag traps instead of hanging the GPU.
-            const int f0 = (int)(base / 3), f1 = (int)((base + ns - 1) / 3);
-            if (t <= f1 - f0) {
-                const int* flag = P.tile_done + f0 + t;
-                int v = 0;
-                const long long t0 = clock64();
-                while (true) {
-                    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-                    if (v != 0) break;
-                    __nanosleep(200);
-                    if (clock64() - t0 > (1ll << 32)) { printf("heads_tail: producer flag %d never set\n", f0 + t); __trap(); }
-                }
-            }
-        }
         __syncthreads();
         // 1. global pooling per (state, channel): mean / max / std (biased variance + 1e-6)  neural_network.py:68-81
         //    thread -> (state, channel octet, half of the board): 18 independent 16-byte loads, one pass (sum, sum of
@@ -401,52 +377,16 @@ heads_tail_kernel(HeadsParams P) {
             }
         }
     }
-    if (P.tile_done) {
-        // the last block to finish hands the flag array back all zero (the state the next producer launch expects)
-        __shared__ int is_last;
-        const int nf = (int)((P.n + 2) / 3);
-        __syncthreads();
-        if (t == 0) is_last = atomicAdd(P.tile_done + nf, 1) == (int)gridDim.x - 1;
-        __syncthreads();
-        if (is_last)
-            for (int i = t; i <= nf; i += kHeadsThreads) P.tile_done[i] = 0;
-    }
 }
 
 }  // namespace
 }  // namespace lzb
 
-static int heads_launch(const void* pv, int64_t n, int32_t pc, int32_t vc, int32_t mlp, int32_t bins,
-                        const float* wgl_t, const float* bn2_scale, const float* bn2_shift, const float* wout,
-                        const float* wfc1_t, const float* bfc1, const float* wfc2_t, const float* bfc2,
-                        const uint64_t* states, float* priors, float* values, float* log_heads,
-                        float* value_logits, int32_t* tile_done, void* stream);
 extern "C" int lzb_heads_tail(const void* pv, int64_t n, int32_t pc, int32_t vc, int32_t mlp, int32_t bins,
                               const float* wgl_t, const float* bn2_scale, const float* bn2_shift, const float* wout,
                               const float* wfc1_t, const float* bfc1, const float* wfc2_t, const float* bfc2,
                               const uint64_t* states, float* priors, float* values, float* log_heads,
                               float* value_logits, void* stream) {
-    return heads_launch(pv, n, pc, vc, mlp, bins, wgl_t, bn2_scale, bn2_shift, wout, wfc1_t, bfc1, wfc2_t, bfc2, states, priors,
-                        values, log_heads, value_logits, nullptr, stream);
-}
-// lzb_heads_tail launched as a PROGRAMMATIC DEPENDENT of the lzb_trunk_bf16_signal launch that precedes it on the stream:
-// its blocks become resident as trunk CTAs finish and wait, per 8-state tile, for the producer's tile_done flags instead of
-// for the whole trunk kernel -- the heads of finished tiles run under the trunk kernel's tail.  The last block zeroes
-// tile_done (int32[ceil(n / 3) + 1]) again.  Must directly follow the matching lzb_trunk_bf16_signal call on `stream`.
-extern "C" int lzb_heads_tail_overlapped(const void* pv, int64_t n, int32_t pc, int32_t vc, int32_t mlp, int32_t bins,
-                                         const float* wgl_t, const float* bn2_scale, const float* bn2_shift, const float* wout,
-                                         const float* wfc1_t, const float* bfc1, const float* wfc2_t, const float* bfc2,
-                                         const uint64_t* states, float* priors, float* values, float* log_heads,
-                                         float* value_logits, int32_t* tile_done, void* stream) {
-    LZB_REQUIRE(tile_done, "null tile_done");
-    return heads_launch(pv, n, pc, vc, mlp, bins, wgl_t, bn2_scale, bn2_shift, wout, wfc1_t, bfc1, wfc2_t, bfc2, states, priors,
-                        values, log_heads, value_logits, tile_done, stream);
-}
-static int heads_launch(const void* pv, int64_t n, int32_t pc, int32_t vc, int32_t mlp, int32_t bins,
-                        const float* wgl_t, const float* bn2_scale, const float* bn2_shift, const float* wout,
-                        const float* wfc1_t, const float* bfc1, const float* wfc2_t, const float* bfc2,
-                        const uint64_t* states, float* priors, float* values, float* log_heads,
-                        float* value_logits, int32_t* tile_done, void* stream) {
     LZB_REQUIRE(n >= 0, "bad batch");
     LZB_REQUIRE(pc >= 1 && pc <= lzb::kMaxHeadCh && vc >= 1 && vc <= lzb::kMaxHeadCh, "head channels must be in [1, 64]");
     LZB_REQUIRE(mlp >= 1 && mlp <= lzb::kMaxMlp && bins >= 2 && bins <= lzb::kMaxBins, "value MLP / bins too large");
@@ -458,23 +398,9 @@ static int heads_launch(const void* pv, int64_t n, int32_t pc, int32_t vc, int32
     P.pv = reinterpret_cast<const __nv_bfloat16*>(pv); P.n = n; P.pc = pc; P.vc = vc; P.mlp = mlp; P.bins = bins;
     P.wgl_t = wgl_t; P.bn2_scale = bn2_scale; P.bn2_shift = bn2_shift; P.wout = wout; P.wfc1_t = wfc1_t; P.bfc1 = bfc1;
     P.wfc2_t = wfc2_t; P.bfc2 = bfc2; P.states = states; P.priors = priors; P.values = values;
-    P.log_heads = log_heads; P.value_logits = value_logits; P.tile_done = tile_done;
-    static const int overlap_trace = getenv("LZB_OVERLAP_TRACE") ? atoi(getenv("LZB_OVERLAP_TRACE")) : 0;
-    P.trace = overlap_trace;
+    P.log_heads = log_heads; P.value_logits = value_logits;
     const int64_t tiles = (n + lzb::kTile - 1) / lzb::kTile;
     const int64_t blocks = tiles < (int64_t)lzb::kNumSMs * 4 ? tiles : (int64_t)lzb::kNumSMs * 4;
-    if (tile_done) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)blocks); cfg.blockDim = dim3(lzb::kHeadsThreads); cfg.dynamicSmemBytes = 0;
-        cfg.stream = (cudaStream_t)stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        cudaError_t le = cudaLaunchKernelEx(&cfg, lzb::heads_tail_kernel, P);
-        (void)le;
-    } else {
-        lzb::heads_tail_kernel<<<(int)blocks, lzb::kHeadsThreads, 0, (cudaStream_t)stream>>>(P);
-    }
+    lzb::heads_tail_kernel<<<(int)blocks, lzb::kHeadsThreads, 0, (cudaStream_t)stream>>>(P);
     return lzb::check_launch("heads_tail_kernel");
 }

@@ -1,5 +1,5 @@
 // lz_tc.cuh -- PTX wrappers for the Blackwell tensor path (tcgen05 / TMEM / TMA / mbarrier / clusters) shared by the
-// fused-trunk kernel (lz_trunk.cu).  Same wrappers as in lz_conv.cu (kept there verbatim for the per-layer kernels).
+// fused-trunk kernel (lz_trunk.cu) and the per-layer convolution kernels (lz_conv.cu).
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -44,7 +44,7 @@ __device__ __forceinline__ uint32_t mbar_try_wait(uint32_t bar, uint32_t parity)
                  : "=r"(done) : "r"(bar), "r"(parity) : "memory");
     return done;
 }
-__device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity) {
+static __device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity) {
     const long long t0 = clock64();
     while (!mbar_try_wait(bar, parity)) {
         if ((uint64_t)(clock64() - t0) > kWatchdogCycles) {
@@ -76,17 +76,6 @@ __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* m) {
 }
 constexpr uint64_t kL2Default = 0x1000000000000000ull;   // the default L2 cache-hint descriptor
 
-// im2col load of [128 pixels x 64 ch] starting at base pixel (w, h, n) with filter offsets (off_w, off_h); the
-// transaction bytes are signalled on `bar` (an address in the LEADER CTA's window: cta_group::2).
-__device__ __forceinline__ void tma_im2col_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c, int w, int h, int n,
-                                               uint16_t off_w, uint16_t off_h) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.im2col.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-        " [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8}, %9;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h),
-          "l"(kL2Default)
-        : "memory");
-}
 __device__ __forceinline__ void tma_tile2d_2sm(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
     asm volatile(
         "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
@@ -142,36 +131,12 @@ __device__ __forceinline__ void tma_tile4d_2sm(uint32_t dst, const CUtensorMap* 
         ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c), "r"(w), "r"(h), "r"(n), "l"(kL2Default)
         : "memory");
 }
-// arrive with RELEASE semantics at cluster scope on a barrier in another CTA of the cluster: publishes this thread's
-// (already proxy-fenced) shared-memory writes to the thread that waits with acquire.cluster
-__device__ __forceinline__ void mbar_arrive_release_cluster(uint32_t cluster_bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-// The same signal with the default semantics (release at CTA scope: MEMBAR.ALL.CTA, i.e. this warp's shared-memory
-// stores have been performed, then the arrive leaves the SM).  `release.cluster` above compiles to MEMBAR.ALL.GPU +
-// ERRBAR + CGAERRBAR (~1,000 cycles per use, measured with the trunk kernel's clock64 trace).  This is the form
-// CUTLASS's ClusterBarrier::arrive(cta_id) uses for every cross-CTA pipeline hand-off.
+// Arrive on a barrier in another CTA of the cluster with the default semantics (release at CTA scope: MEMBAR.ALL.CTA,
+// i.e. this warp's shared-memory stores have been performed, then the arrive leaves the SM).  An arrive with
+// `.release.cluster` would compile to MEMBAR.ALL.GPU + ERRBAR + CGAERRBAR (~1,000 cycles per use, measured in the trunk
+// kernel).  This is the form CUTLASS's ClusterBarrier::arrive(cta_id) uses for every cross-CTA pipeline hand-off.
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_bar) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
-}
-__device__ __forceinline__ uint32_t mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    return done;
-}
-__device__ __noinline__ void mbar_wait_cluster_slow(uint32_t bar, uint32_t parity) {
-    const long long t0 = clock64();
-    while (!mbar_try_wait_cluster(bar, parity)) {
-        if ((uint64_t)(clock64() - t0) > kWatchdogCycles) {
-            printf("lz_trunk: mbarrier (cluster) wait timed out (block %d thread %d bar 0x%x parity %u)\n", (int)blockIdx.x,
-                   (int)threadIdx.x, bar, parity);
-            __trap();
-        }
-    }
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-    if (!mbar_try_wait_cluster(bar, parity)) mbar_wait_cluster_slow(bar, parity);
 }
 __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32]) {
     asm volatile(

@@ -20,12 +20,11 @@
 //   * epilogue warps (8): TMEM -> registers -> bias / BatchNorm / ReLU -> bf16 -> the three shifted copies in shared
 //     memory (swizzled 16-byte stores), 64 channels at a time: the next layer's MMAs on channels 0-63 start while the
 //     epilogue still produces channels 64-127 (K-chunk pipelining).
-//   * weights: one (tap, 64-channel chunk) slice (8 KB per CTA) per pipeline stage, streamed by TMA through a 12-stage
+//   * weights: one tap (this CTA's 64 couts x 128 cin, 16 KB) per pipeline stage, streamed by TMA through a kWStages
 //     ring across layer and tile boundaries.
 // Per layer and tile: 72 MMAs (36 for the stem, 8 for the 1x1 heads conv); junk accumulator rows (the pad row between
 // boards, 20 of 128) are the price of serving all taps from one resident tile.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "lz_common.cuh"
 #include "lz_tc.cuh"
@@ -52,11 +51,6 @@ struct TrunkParams {
     __nv_bfloat16* out;        // [images * 36][128] : relu(heads conv + bias), the input of heads_tail_kernel
     int images;
     int blocks;                // residual blocks; layers = 2 * blocks + 2
-    int debug;
-    int w_copies;              // the trunk weight tensor is stored w_copies times back to back; cluster c reads copy c % w_copies
-    int w_stages;              // weight ring depth actually used (<= kWStages; fewer = latency experiment)
-    int* tile_done;            // optional: tile_done[i] = 1 once boards [3 i, 3 i + 3) of `out` are complete (heads overlap)
-    unsigned long long* trace;   // debug bit 8: clock64 stamps of cluster 0's leader CTA ([0,4096) MMA thread, [4096,8192) epilogue warp 2)
 };
 
 // Per-layer epilogue parameters in CONSTANT memory (warp-uniform reads through the constant cache: no shared-memory
@@ -83,16 +77,6 @@ __device__ __forceinline__ void mbar_arrive_n(uint32_t bar, uint32_t n) {
 // layer 0 of slot 0, layer 0 of slot 1, layer 1 of slot 0, ...: while the tensor core works on one slot, the epilogue
 // warps turn the other slot's accumulator into its next operand.  Operand copies are numbered in consumption order
 // (3 per job, 1 for the 1x1 heads layer) and live in ring buffer number (copy index % 4).
-// 2-D tiled load multicast to the CTAs of `mask` (same shared-memory offset in each); with cta_group::2 the bytes are
-// signalled on the barrier at this offset in the LEADER of each destination CTA's pair
-__device__ __forceinline__ void tma_tile2d_2sm_mc(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster.L2::cache_hint"
-        " [%0], [%1, {%4, %5}], [%2], %3, %6;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "h"(mask), "r"(c0), "r"(c1), "l"(kL2Default)
-        : "memory");
-}
-
 struct Sched {
     int layers;
     __device__ __forceinline__ int ncopies(int l) const { return l == layers - 1 ? 1 : 3; }
@@ -103,14 +87,10 @@ struct Sched {
     __device__ __forceinline__ int round_total(int ns) const { return ns * (3 * (layers - 1) + 1); }
 };
 
-// CS = CTAs per cluster: 2 (one MMA pair) or 4 (two MMA pairs that walk the same weight stream in lockstep: every weight
-// box is fetched from L2 ONCE per cluster and multicast to the CTA of each pair that needs it -- the weight stream, not the
-// tensor core, bounds the 2-CTA variant: profiles/r02_trunk_decompose_*.txt).  The cluster size is set at launch.
-template <int CS>
+// One cluster = one MMA pair (2 CTAs, set at launch); rank 0 is the pair's leader.
 __global__ void __launch_bounds__(kTrunkThreads, 1)
 trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ CUtensorMap tmW0,
              const __grid_constant__ CUtensorMap tmW1, const TrunkParams P) {
-    constexpr int kPairs = CS / 2;                                   // MMA pairs per cluster
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t a_smem = base;                                    // kCopyBufs copy buffers x 2 chunks
@@ -123,7 +103,6 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
     const uint32_t accfull_bar = wempty_bar + 8 * kWStages;          // [2] both  : a slot's accumulator is complete
     const uint32_t epidone_bar = accfull_bar + 16;                   // [2] leader: a slot's last accumulator drained (16 arrivals)
     const uint32_t tmem_slot = epidone_bar + 16;
-    const uint32_t dummy_bar = tmem_slot + 8;                        // timing experiments only (debug bit 64)
     uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
     volatile uint32_t* tmem_slot_p = reinterpret_cast<volatile uint32_t*>(gen + (tmem_slot - base));
 
@@ -131,38 +110,25 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
     // Copy hand-off epilogue -> MMA thread.  The operand copies are written with st.shared by the CTA whose OWN tensor
     // core reads them (cta_group::2: every CTA's A rows come from its own shared memory), so what has to hold is that the
     // stores were performed and fenced into the async proxy before the arrive leaves the SM: fence.proxy.async +
-    // an arrive with the default (release, CTA-scope) semantics = MEMBAR.ALL.CTA.  debug bit 256 switches back to
-    // release.cluster / acquire.cluster (MEMBAR.ALL.GPU + CCTL.IVALL: ~1,000 cycles per copy, 3 copies per job).
-    const bool strict_sync = (P.debug & 256) != 0;
-    const uint32_t crank = cluster_ctarank();                        // rank in the cluster
-    const uint32_t rank = crank & 1u;                                // rank in the MMA pair
-    const uint32_t lead_rank = crank & ~1u;                          // the pair's leader CTA
-    const uint32_t pair_in_cluster = crank >> 1;
+    // an arrive with the default (release, CTA-scope) semantics = MEMBAR.ALL.CTA.  (release.cluster / acquire.cluster
+    // would cost MEMBAR.ALL.GPU + CCTL.IVALL: ~1,000 cycles per copy, 3 copies per job.)
+    const uint32_t rank = cluster_ctarank();                         // rank in the MMA pair
     const bool leader = rank == 0;
-    // "cluster_id" below is the index of this MMA PAIR, "num_clusters" the number of pairs: tiles are dealt to pairs
-    const int cluster_id = (int)(blockIdx.x / CS) * kPairs + (int)pair_in_cluster, num_clusters = (int)(gridDim.x / CS) * kPairs;
+    const int cluster_id = blockIdx.x >> 1, num_clusters = gridDim.x >> 1;
     const int64_t pair_tiles = (P.images + 2 * kBoards - 1) / (2 * kBoards);
-    // pair tiles of this pair; in a 4-CTA cluster both pairs run the SAME number of jobs (lockstep on the weight stream):
-    // the surplus ones are dummy tiles (boards beyond the batch: zero input, no output)
-    const int ntiles = CS == 2 ? (int)((pair_tiles - cluster_id + num_clusters - 1) / num_clusters)
-                               : (int)((pair_tiles + num_clusters - 1) / num_clusters);
+    const int ntiles = (int)((pair_tiles - cluster_id + num_clusters - 1) / num_clusters);
     const int rounds = (ntiles + 1) / 2;
-    const uint16_t pair_mask = (uint16_t)(3u << (2 * pair_in_cluster));      // commit multicast: the two CTAs of this pair
-    const uint16_t all_mask = (uint16_t)((1u << CS) - 1u);
     Sched sch;
     sch.layers = 2 * P.blocks + 2;
     const int layers = sch.layers;
-    // Tap order (copy order and dy order inside a copy).  A per-cluster rotation was tried (so that the 74 clusters, which
-    // run nearly in lockstep, do not all ask the L2 for the same 32 KB weight tap at the same moment): no gain (877 us
-    // either way), and it made a board's fp32 summation order -- hence its low-order bits -- depend on WHERE in the batch
-    // it sits, which breaks the equality of compacted and full-batch searches.  Fixed order: results are position-free.
-    const int rot_c = 0, rot_d = 0;
+    // Tap order (copy order, and dy order inside a copy) is the same for every cluster: it fixes the fp32 summation
+    // order of every board, so a board's result does not depend on where in the batch it sits (compacted and
+    // full-batch searches must agree bit for bit).
 
     if (threadIdx.x == 0) {
         prefetch_tmap(&tmIn); prefetch_tmap(&tmW0); prefetch_tmap(&tmW1);
         for (int i = 0; i < kCopyBufs; ++i) { mbar_init(full_bar + 8 * i, 16); mbar_init(empty_bar + 8 * i, 1); }
-        for (int i = 0; i < kWStages; ++i) { mbar_init(wfull_bar + 8 * i, 1); mbar_init(wempty_bar + 8 * i, kPairs); }
-        mbar_init(dummy_bar, 1);
+        for (int i = 0; i < kWStages; ++i) { mbar_init(wfull_bar + 8 * i, 1); mbar_init(wempty_bar + 8 * i, 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(accfull_bar + 8 * i, 1); mbar_init(epidone_bar + 8 * i, 16); }
         fence_barrier_init();
     }
@@ -184,11 +150,9 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
 
     if (warp == 0) {
         // ===================== TMA producer (both CTAs): stem input copies + every weight tap, in MMA order =============
-        const uint32_t full_leader = mapa_rank(full_bar, lead_rank), wfull_leader = mapa_rank(wfull_bar, lead_rank);
+        const uint32_t full_leader = mapa_rank(full_bar, 0), wfull_leader = mapa_rank(wfull_bar, 0);
         uint32_t wst = 0, wph = 0;
         int g_round = 0;                                             // copies before this round
-        // replicated weights: clusters are spread over the copies so that fewer SMs pull the same L2 lines at once
-        const int w_row0 = (cluster_id % P.w_copies) * (P.blocks * 18 + 1) * 128;
         for (int r = 0; r < rounds; ++r) {
             const int ns = ntiles - 2 * r >= 2 ? 2 : 1;
             for (int l = 0; l < layers; ++l) {
@@ -206,54 +170,29 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                                     mbar_arrive_expect_tx(full_bar + 8 * buf, 2 * kBoxBytes);
                                     mbar_arrive_n(full_bar + 8 * buf, 15);
                                 }
-                                tma_tile4d_2sm(a_smem + buf * kCopyBytes, &tmIn, full_leader + 8 * buf, 0, (c + rot_c) % 3 - 1, -1, board0);
+                                tma_tile4d_2sm(a_smem + buf * kCopyBytes, &tmIn, full_leader + 8 * buf, 0, c - 1, -1, board0);
                             }
                             __syncwarp();
                         }
                     }
                     const int tap_base = l == 0 ? 0 : (l - 1) * 9;
                     for (int t = 0; t < taps; ++t) {
-                        // MMA order: copy-major, dy-minor (both rotated per cluster); tap index in the weight tensor =
-                        // (dy + 1) * 3 + (dx + 1)
-                        const int tap = taps == 9 ? ((t % 3 + rot_d) % 3) * 3 + (t / 3 + rot_c) % 3 : 0;
+                        // MMA order: copy-major, dy-minor; tap index in the weight tensor = (dy + 1) * 3 + (dx + 1)
+                        const int tap = taps == 9 ? (t % 3) * 3 + t / 3 : 0;
                         mbar_wait(wempty_bar + 8 * wst, wph ^ 1);
                         if (elect_one()) {
                             const uint32_t dstw = w_smem + wst * kWStageBytes;
-                            if (P.debug & 32) {          // timing experiment: no weight loads, the MMAs read whatever is there
-                                if (leader) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(wfull_bar + 8 * wst) : "memory");
-                            } else if (CS == 2) {
-                                if (l == 0) {
-                                    if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * 8192);
-                                    tma_tile2d_2sm(dstw, &tmW0, wfull_leader + 8 * wst, 0, tap * 128 + (int)rank * 64);
-                                } else {
-                                    if (P.debug & 128) {   // timing experiment: half the weight bytes (results are garbage)
-                                        if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * 8192);
-                                        tma_tile2d_2sm(dstw, &tmW1, wfull_leader + 8 * wst, 0, w_row0 + (tap_base + tap) * 128 + (int)rank * 64);
-                                    } else {
-                                    if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * kWStageBytes);
-                                    tma_tile2d_2sm(dstw, &tmW1, wfull_leader + 8 * wst, 0, w_row0 + (tap_base + tap) * 128 + (int)rank * 64);
-                                    tma_tile2d_2sm(dstw + 8192, &tmW1, wfull_leader + 8 * wst, 64, w_row0 + (tap_base + tap) * 128 + (int)rank * 64);
-                                    }
-                                }
+                            if (l == 0) {
+                                if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * 8192);
+                                tma_tile2d_2sm(dstw, &tmW0, wfull_leader + 8 * wst, 0, tap * 128 + (int)rank * 64);
                             } else {
-                                // 4-CTA cluster: the 64-cout half this CTA needs is also needed by the CTA of the same parity in
-                                // the other pair.  Each of the two loads HALF of it (32 couts = box rows [32 q, 32 q + 32), q =
-                                // pair index) and multicasts to both; the bytes are counted on each destination pair's leader.
-                                const uint16_t mc = (uint16_t)(5u << rank);          // CTAs {rank, rank + 2}
-                                const int row_half = (int)rank * 64 + (int)pair_in_cluster * 32;
-                                const uint32_t dsth = dstw + pair_in_cluster * 4096;
-                                if (l == 0) {
-                                    if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * 8192);
-                                    tma_tile2d_2sm_mc(dsth, &tmW0, wfull_leader + 8 * wst, 0, tap * 128 + row_half, mc);
-                                } else {
-                                    if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * kWStageBytes);
-                                    tma_tile2d_2sm_mc(dsth, &tmW1, wfull_leader + 8 * wst, 0, w_row0 + (tap_base + tap) * 128 + row_half, mc);
-                                    tma_tile2d_2sm_mc(dsth + 8192, &tmW1, wfull_leader + 8 * wst, 64, w_row0 + (tap_base + tap) * 128 + row_half, mc);
-                                }
+                                if (leader) mbar_arrive_expect_tx(wfull_bar + 8 * wst, 2 * kWStageBytes);
+                                tma_tile2d_2sm(dstw, &tmW1, wfull_leader + 8 * wst, 0, (tap_base + tap) * 128 + (int)rank * 64);
+                                tma_tile2d_2sm(dstw + 8192, &tmW1, wfull_leader + 8 * wst, 64, (tap_base + tap) * 128 + (int)rank * 64);
                             }
                         }
                         __syncwarp();
-                        if (++wst == (uint32_t)P.w_stages) { wst = 0; wph ^= 1; }
+                        if (++wst == (uint32_t)kWStages) { wst = 0; wph ^= 1; }
                     }
                 }
             }
@@ -265,7 +204,6 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
             uint32_t wst = 0, wph = 0;
             uint32_t acc_tile_ph[2] = {0, 0};
             int g = 0;                                               // next copy to consume
-            int tr_m = 0;
             for (int r = 0; r < rounds; ++r) {
                 const int ns = ntiles - 2 * r >= 2 ? 2 : 1;
                 for (int l = 0; l < layers; ++l) {
@@ -273,27 +211,21 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                     const bool conv2 = l >= 2 && l < layers - 1 && (l & 1) == 0;     // accumulates onto the residual stream
                     for (int s = 0; s < ns; ++s) {
                         if (l == 0) {                                // acc_h of this slot's previous tile has been drained
-                            if (strict_sync) mbar_wait_cluster(epidone_bar + 8 * s, acc_tile_ph[s] ^ 1);
-                            else mbar_wait(epidone_bar + 8 * s, acc_tile_ph[s] ^ 1);
+                            mbar_wait(epidone_bar + 8 * s, acc_tile_ph[s] ^ 1);
                             acc_tile_ph[s] ^= 1;
                         }
                         const uint32_t d_tmem = tmem_base + (uint32_t)s * 256u + (conv2 ? kAccX : kAccH);
                         const int nc = sch.ncopies(l);
                         for (int c = 0; c < nc; ++c, ++g) {
                             const int buf = g & 3;
-                            const int dxi = nc == 3 ? c : 1;
-                            if (P.trace && blockIdx.x == 0 && lane == 0 && tr_m < 4090) P.trace[tr_m++] = clock64();   // before the copy wait
-                            if (strict_sync) mbar_wait_cluster(full_bar + 8 * buf, ((uint32_t)g >> 2) & 1u);
-                            else mbar_wait(full_bar + 8 * buf, ((uint32_t)g >> 2) & 1u);
+                            mbar_wait(full_bar + 8 * buf, ((uint32_t)g >> 2) & 1u);
                             tc_fence_after();
-                            if (P.trace && blockIdx.x == 0 && lane == 0 && tr_m < 4090) P.trace[tr_m++] = clock64();   // copy ready
                             for (int d = 0; d < nc; ++d) {            // nc = 3: three dy taps per copy; heads conv: one tap (dy = 0)
-                                const int dyi = nc == 3 ? (d + rot_d) % 3 : 1;
+                                const int dyi = nc == 3 ? d : 1;
                                 mbar_wait(wfull_bar + 8 * wst, wph);
                                 tc_fence_after();
                                 if (elect_one()) {
                                     const bool first_tap = c == 0 && d == 0;
-                                    const int stem_ksteps = (P.debug & 512) ? 4 : 1;      // debug bit 512: all four (A/B timing)
                                     const bool last_tap = c == nc - 1 && d == nc - 1;
 #pragma unroll
                                     for (int kc = 0; kc < 2; ++kc) {
@@ -306,24 +238,18 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                                             // step contributes (9 MMAs instead of 36 for the layer)
 #pragma unroll
                                             for (int k = 0; k < 4; ++k)
-                                                if (!(P.debug & 4) && (k < stem_ksteps || l != 0))
+                                                if (k == 0 || l != 0)
                                                     umma_2sm(d_tmem, adesc + 2 * k, bdesc + 2 * k,
                                                              (uint32_t)(conv2 || !first_tap || (kc | k) != 0));
                                         }
                                     }
-                                    umma_commit_2sm(wempty_bar + 8 * wst, all_mask);             // every CTA that holds this stage
-                                    if (P.debug & 64) {   // timing experiment: what does a commit cost the issue stream?
-                                        umma_commit_2sm(dummy_bar, all_mask);
-                                        umma_commit_2sm(dummy_bar, all_mask);
-                                    }
-                                    if (d == nc - 1) umma_commit_2sm(empty_bar + 8 * buf, pair_mask);   // copy consumed
-                                    if (last_tap) umma_commit_2sm(accfull_bar + 8 * s, pair_mask);
-                                    (void)dxi;
+                                    umma_commit_2sm(wempty_bar + 8 * wst, 3);                    // both CTAs hold this stage
+                                    if (d == nc - 1) umma_commit_2sm(empty_bar + 8 * buf, 3);    // copy consumed
+                                    if (last_tap) umma_commit_2sm(accfull_bar + 8 * s, 3);
                                 }
                                 __syncwarp();
-                                if (++wst == (uint32_t)P.w_stages) { wst = 0; wph ^= 1; }
+                                if (++wst == (uint32_t)kWStages) { wst = 0; wph ^= 1; }
                             }
-                            if (P.trace && blockIdx.x == 0 && lane == 0 && tr_m < 4090) P.trace[tr_m++] = clock64();   // taps of this copy issued
                         }
                     }
                 }
@@ -351,9 +277,8 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
             rowoff[dxi] = (uint32_t)rho * 128u;
             swz[dxi] = (uint32_t)(rho & 7);
         }
-        const uint32_t full_leader = mapa_rank(full_bar, lead_rank), epidone_leader = mapa_rank(epidone_bar, lead_rank);
+        const uint32_t full_leader = mapa_rank(full_bar, 0), epidone_leader = mapa_rank(epidone_bar, 0);
         uint32_t acc_ph[2] = {0, 0};
-        int tr_e = 0;
         int g_round = 0;
         for (int r = 0; r < rounds; ++r) {
             const int ns = ntiles - 2 * r >= 2 ? 2 : 1;
@@ -367,11 +292,9 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                     const uint32_t acc_col = conv2 ? kAccX : kAccH;
                     const int64_t pt = cluster_id + (int64_t)(2 * r + s) * num_clusters;
                     const int board0 = (int)(2 * pt + rank) * kBoards;
-                    if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 4090) P.trace[4096 + tr_e++] = clock64();   // waiting
                     mbar_wait(accfull_bar + 8 * s, acc_ph[s]);
                     acc_ph[s] ^= 1;
                     tc_fence_after();
-                    if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 4090) P.trace[4096 + tr_e++] = clock64();   // accumulator ready
                     // 1. the whole accumulator row segment (64 channels) -> registers -> bias / BatchNorm / ReLU -> bf16, ONCE:
                     //    after this the accumulator is dead, so the slot's next MMAs may overwrite it at any time
                     uint32_t pk[2][16];
@@ -420,11 +343,10 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                         }
                     }
                     if (stem) tmem_st_wait();
-                    if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 4090) P.trace[4096 + tr_e++] = clock64();   // phase 1 done
                     // 2. the operand copies of this slot's NEXT layer, in ring order, as their buffers become free -- or,
                     //    after the last layer, the rows of the output tensor
                     if (last) {
-                        if (row_ok && board0 + b < P.images && !(P.debug & 1)) {
+                        if (row_ok && board0 + b < P.images) {
 #pragma unroll
                             for (int hh = 0; hh < 2; ++hh) {
                                 uint4* o = reinterpret_cast<uint4*>(P.out + ((int64_t)(board0 + b) * 36 + rem) * 128 + col_half * 64 + hh * 32);
@@ -437,11 +359,10 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                         const int nc = sch.ncopies(l + 1);
                         const int g0 = g_round + sch.before(l + 1, s, ns);
                         for (int c = 0; c < nc; ++c) {
-                            const int dxi = nc == 3 ? (c + rot_c) % 3 : 1;
+                            const int dxi = nc == 3 ? c : 1;
                             const int g = g0 + c, buf = g & 3;
                             mbar_wait(empty_bar + 8 * buf, (((uint32_t)g >> 2) & 1u) ^ 1u);      // its previous readers are done
-                            if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 4090) P.trace[4096 + tr_e++] = clock64();   // buffer free
-                            if (row_ok && !(P.debug & 16)) {
+                            if (row_ok) {
                                 // copy dx index is a loop variable: select this thread's row offset / swizzle / zero flag
                                 const uint32_t ro = dxi == 0 ? rowoff[0] : dxi == 1 ? rowoff[1] : rowoff[2];
                                 const uint32_t sw = dxi == 0 ? swz[0] : dxi == 1 ? swz[1] : swz[2];
@@ -459,30 +380,14 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
                             fence_proxy_async();          // generic-proxy stores -> visible to the tensor core (async proxy)
                             tc_fence_before();
                             __syncwarp();
-                            if (lane == 0) {
-                                if (strict_sync) mbar_arrive_release_cluster(full_leader + 8 * buf);
-                                else mbar_arrive_remote(full_leader + 8 * buf);
-                            }
-                            if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 4090) P.trace[4096 + tr_e++] = clock64();   // copy published
+                            if (lane == 0) mbar_arrive_remote(full_leader + 8 * buf);
                         }
-                    }
-                    if (last && P.tile_done) {
-                        // the tile's rows of `out` are complete once all eight epilogue warps have stored their part: publish
-                        // it to the overlapped heads kernel (which acquires the flag before reading the rows)
-                        __threadfence();
-                        asm volatile("bar.sync 1, 256;" ::: "memory");
-                        if (warp == 2 && lane == 0 && board0 < P.images)
-                            asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(P.tile_done + board0 / kBoards), "r"(1) : "memory");
                     }
                     if (last) {                           // acc_h has been read: this slot's next tile may overwrite it
                         tc_fence_before();
                         __syncwarp();
-                        if (lane == 0) {
-                            if (strict_sync) mbar_arrive_release_cluster(epidone_leader + 8 * s);
-                            else mbar_arrive_remote(epidone_leader + 8 * s);
-                        }
+                        if (lane == 0) mbar_arrive_remote(epidone_leader + 8 * s);
                     }
-                    if (P.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && tr_e < 4090) P.trace[4096 + tr_e++] = clock64();   // job done
                 }
             }
             g_round += sch.round_total(ns);
@@ -495,11 +400,6 @@ trunk_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_constant__ C
     if (warp == 1) {
         asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTrunkTmemCols) : "memory");
     }
-    if ((P.debug & 1024) && P.tile_done && threadIdx.x == 0 && blockIdx.x < 512) {   // debug: when did this CTA finish?
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        reinterpret_cast<unsigned long long*>(P.tile_done + 4096 + 2048)[blockIdx.x] = gt;
-    }
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -509,37 +409,15 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 }  // namespace
 }  // namespace lzb
 
-static unsigned long long* g_trunk_trace = nullptr;
-// debug: copy the clock64 trace of the last launch (LZB_TRUNK_DEBUG & 8) to host memory (8192 u64)
-extern "C" __attribute__((visibility("default"))) int lzb_trunk_debug_trace(unsigned long long* host_out) {
-    if (!g_trunk_trace) return LZB_ERR_INVALID_ARGUMENT;
-    return cudaMemcpy(host_out, g_trunk_trace, 8192 * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? LZB_OK : LZB_ERR_CUDA;
-}
-
 // planes bf16 [n,6,6,64] (channel-padded input), w_stem bf16 [9][128][64], w_trunk bf16 [2*blocks*9 + 1][128][128]
 // (conv1_0, conv2_0, ..., conv2_{blocks-1}, heads 1x1; BatchNorm folded where it follows a conv), params f32 (DEVICE
 // memory, compact: stem bias | scale | shift (384), then per block conv1 bias (128) + conv2 scale | shift (256), then the
 // heads conv bias (128)), out bf16 [n,6,6,128] = relu(heads conv + bias).  blocks <= 10.
-static int trunk_launch(const void* planes, int64_t n, const void* w_stem, const void* w_trunk, int32_t w_copies,
-                        const float* params, int32_t blocks, void* out, int32_t* tile_done, void* stream);
-extern "C" int lzb_trunk_bf16(const void* planes, int64_t n, const void* w_stem, const void* w_trunk, int32_t w_copies,
-                              const float* params, int32_t blocks, void* out, void* stream) {
-    return trunk_launch(planes, n, w_stem, w_trunk, w_copies, params, blocks, out, nullptr, stream);
-}
-// The same launch that additionally publishes per-tile completion: tile_done (device, int32[ceil(n / 3) + 1], ALL ZERO on
-// entry) -- entry i becomes 1 when boards [3 i, 3 i + 3) of `out` are complete.  Consumed (and zeroed again) by
-// lzb_heads_tail_overlapped, which may then start on SMs whose trunk CTA has finished while other CTAs still run.
-extern "C" int lzb_trunk_bf16_signal(const void* planes, int64_t n, const void* w_stem, const void* w_trunk, int32_t w_copies,
-                                     const float* params, int32_t blocks, void* out, int32_t* tile_done, void* stream) {
-    LZB_REQUIRE(tile_done, "null tile_done");
-    return trunk_launch(planes, n, w_stem, w_trunk, w_copies, params, blocks, out, tile_done, stream);
-}
-static int trunk_launch(const void* planes, int64_t n, const void* w_stem, const void* w_trunk, int32_t w_copies,
-                        const float* params, int32_t blocks, void* out, int32_t* tile_done, void* stream) {
+extern "C" int lzb_trunk_bf16(const void* planes, int64_t n, const void* w_stem, const void* w_trunk, const float* params,
+                              int32_t blocks, void* out, void* stream) {
     using namespace lzb;
     LZB_REQUIRE(n > 0 && n < (1ll << 30), "bad batch size");
     LZB_REQUIRE(blocks >= 1 && blocks <= kMaxBlocks, "blocks must be in [1, 10]");
-    LZB_REQUIRE(w_copies >= 1 && w_copies <= 64, "w_copies must be in [1, 64]");
     LZB_REQUIRE(planes && w_stem && w_trunk && params && out, "null pointer");
     LZB_REQUIRE(((reinterpret_cast<uintptr_t>(planes) | reinterpret_cast<uintptr_t>(w_stem) | reinterpret_cast<uintptr_t>(w_trunk) |
                   reinterpret_cast<uintptr_t>(out)) & 15) == 0, "pointers must be 16-byte aligned");
@@ -554,9 +432,6 @@ static int trunk_launch(const void* planes, int64_t n, const void* w_stem, const
         }
         encode_tiled = reinterpret_cast<EncodeTiledFn>(fn);
     }
-    // LZB_TRUNK_CLUSTER = 2 (default): clusters are single MMA pairs; 4: two pairs per cluster share one multicast
-    // weight stream (33 such clusters fit a B200: 132 of 148 SMs)
-    static const int cs = (getenv("LZB_TRUNK_CLUSTER") && atoi(getenv("LZB_TRUNK_CLUSTER")) == 4) ? 4 : 2;
     alignas(64) CUtensorMap tmIn, tmW0, tmW1;
     {
         const cuuint64_t dim[4] = {64, 6, 6, (cuuint64_t)n};
@@ -570,10 +445,10 @@ static int trunk_launch(const void* planes, int64_t n, const void* w_stem, const
     }
     for (int which = 0; which < 2; ++which) {
         const cuuint64_t cin = which == 0 ? 64 : 128;
-        const cuuint64_t rows = which == 0 ? 9 * 128 : ((cuuint64_t)blocks * 18 + 1) * 128 * (cuuint64_t)w_copies;
+        const cuuint64_t rows = which == 0 ? 9 * 128 : ((cuuint64_t)blocks * 18 + 1) * 128;
         const cuuint64_t dim[2] = {cin, rows};
         const cuuint64_t stride[1] = {cin * 2};
-        const cuuint32_t box[2] = {64, (cuuint32_t)(cs == 4 ? 32 : 64)};      // 4-CTA clusters: each CTA loads half a box and multicasts
+        const cuuint32_t box[2] = {64, 64};
         const cuuint32_t estr[2] = {1, 1};
         const CUresult rc = encode_tiled(which == 0 ? &tmW0 : &tmW1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2,
                                          const_cast<void*>(which == 0 ? w_stem : w_trunk), dim, stride, box, estr,
@@ -583,45 +458,21 @@ static int trunk_launch(const void* planes, int64_t n, const void* w_stem, const
     }
     constexpr size_t smem = 1024 + (size_t)kCopyBufs * kCopyBytes + (size_t)kWStages * kWStageBytes +
                             8 * (2 * kCopyBufs + 2 * kWStages + 4) + 32 + 256;
+    // the dynamic shared memory opt-in and the SM count are per DEVICE (a process may drive several GPUs)
     static int max_clusters[64] = {0};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { set_error("lzb_trunk: bad current device"); return LZB_ERR_CUDA; }
-    const void* kfn = cs == 4 ? (const void*)trunk_kernel<4> : (const void*)trunk_kernel<2>;
-    cudaLaunchConfig_t cfg = {};
-    cfg.blockDim = dim3(kTrunkThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
     if (max_clusters[dev] == 0) {
-        if (cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+        if (cudaFuncSetAttribute(trunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
             set_error("lzb_trunk: cannot raise dynamic shared memory to %zu", smem);
             return LZB_ERR_CUDA;
         }
         int sms = 0;
         if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms < 2) sms = kNumSMs;
-        int nc = sms / cs;
-        if (cs == 4) {      // how many 4-CTA clusters of this size are co-resident (GPC boundaries strand some SMs)
-            cfg.gridDim = dim3(sms / cs * cs);
-            cfg.numAttrs = 1;
-            int q = 0;
-            if (cudaOccupancyMaxActiveClusters(&q, kfn, &cfg) == cudaSuccess && q > 0) nc = q;
-        }
-        max_clusters[dev] = nc;
+        max_clusters[dev] = sms / 2;
     }
     TrunkParams P;
-    P.out = reinterpret_cast<__nv_bfloat16*>(out); P.images = (int)n; P.blocks = blocks; P.w_copies = w_copies;
-    P.tile_done = tile_done;
-    static const int debug = getenv("LZB_TRUNK_DEBUG") ? atoi(getenv("LZB_TRUNK_DEBUG")) : 0;
-    P.debug = debug;
-    static const int w_stages = getenv("LZB_TRUNK_W_STAGES") ? atoi(getenv("LZB_TRUNK_W_STAGES")) : kWStages;
-    P.w_stages = w_stages >= 1 && w_stages <= kWStages ? w_stages : kWStages;
-    if ((debug & 8) && !g_trunk_trace) { cudaMalloc(&g_trunk_trace, 8192 * 8); cudaMemset(g_trunk_trace, 0, 8192 * 8); }
-    P.trace = g_trunk_trace;
+    P.out = reinterpret_cast<__nv_bfloat16*>(out); P.images = (int)n; P.blocks = blocks;
     // the parameter table goes to constant memory in stream order (device -> constant copy; a memcpy node under capture),
     // so every launch -- also a graph replay after an in-place weight refresh, or another network on this stream -- sees
     // its own current parameters
@@ -631,13 +482,19 @@ static int trunk_launch(const void* planes, int64_t n, const void* w_stem, const
         return LZB_ERR_CUDA;
     }
     const int64_t pair_tiles = (n + 2 * kBoards - 1) / (2 * kBoards);
-    const int64_t clusters_needed = (pair_tiles + cs / 2 - 1) / (cs / 2);
-    const int clusters = (int)(clusters_needed < max_clusters[dev] ? clusters_needed : max_clusters[dev]);
-    cfg.gridDim = dim3(cs * clusters);
+    const int clusters = (int)(pair_tiles < max_clusters[dev] ? pair_tiles : max_clusters[dev]);
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2 * clusters);
+    cfg.blockDim = dim3(kTrunkThreads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute attr[2];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[1].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
     cfg.numAttrs = 2;
-    cudaError_t le;
-    if (cs == 4) le = cudaLaunchKernelEx(&cfg, trunk_kernel<4>, tmIn, tmW0, tmW1, P);
-    else le = cudaLaunchKernelEx(&cfg, trunk_kernel<2>, tmIn, tmW0, tmW1, P);
-    (void)le;
+    (void)cudaLaunchKernelEx(&cfg, trunk_kernel, tmIn, tmW0, tmW1, P);
     return check_launch("trunk_kernel");
 }

@@ -14,8 +14,6 @@ from __future__ import annotations
 
 from typing import Dict, Optional, Tuple
 
-import os
-
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -225,8 +223,7 @@ class FusedTrunk:
         self.use_cudnn_fused = True
         # our tcgen05 implicit-GEMM conv covers the 128-channel trunk; other widths keep the cuDNN path
         self.use_tc = (model.stem_conv.out_channels == 128 and model.stem_conv.in_channels <= 64 and len(model.blocks) > 0
-                       and model.stem_conv.weight.dtype == torch.bfloat16
-                       and os.environ.get("LZB_DISABLE_TC_CONV", "0") != "1")
+                       and model.stem_conv.weight.dtype == torch.bfloat16)
         self.refresh()
         if not self.use_tc:
             self._probe()
@@ -383,7 +380,7 @@ class FusedHeads:
         self._set("bn1_scale", torch.cat([s1, s2]))
         self._set("bn1_shift", torch.cat([t1, t2]))
         self.use_tc = (self.pc + self.vc == 128 and ph.conv1.in_channels == 128
-                       and ph.conv1.weight.dtype == torch.bfloat16 and os.environ.get("LZB_DISABLE_TC_CONV", "0") != "1")
+                       and ph.conv1.weight.dtype == torch.bfloat16)
         if self.use_tc:     # both heads' 1x1 convs + their BatchNorm + ReLU as ONE launch of our tcgen05 conv
             wf = torch.cat([ph.conv1.weight.detach(), vh.conv1.weight.detach()], 0).float()
             self._set("conv_wp", pack_conv_weight(wf * torch.cat([s1, s2]).view(-1, 1, 1, 1)))
@@ -400,8 +397,7 @@ class FusedHeads:
         self._set("bfc2", f(vh.fc2.bias))
 
     def __call__(self, a: Optional[torch.Tensor], states: Optional[torch.Tensor] = None, *, priors_out=None,
-                 values_out=None, want_raw: bool = False, pv: Optional[torch.Tensor] = None,
-                 tile_done: Optional[torch.Tensor] = None):
+                 values_out=None, want_raw: bool = False, pv: Optional[torch.Tensor] = None):
         """a: trunk output bf16 [n,C,6,6] channels-last.  With `states` (packed int64[n,4]) returns
         (priors f32[n,220], values f32[n]); with want_raw returns (log_p1, log_p2, log_pmc, value_logits) fp32."""
         import ctypes
@@ -432,17 +428,14 @@ class FusedHeads:
                 priors_out = torch.empty((n, 220), dtype=torch.float32, device=dev)
             if values_out is None:
                 values_out = torch.empty((n,), dtype=torch.float32, device=dev)
-        args = (ptr(pv), i64(n), ctypes.c_int32(self.pc), ctypes.c_int32(self.vc),
-                ctypes.c_int32(self.mlp), ctypes.c_int32(self.bins), ptr(t["wgl_t"]),
-                ptr(t["bn2_scale"]), ptr(t["bn2_shift"]), ptr(t["wout"]), ptr(t["wfc1_t"]),
-                ptr(t["bfc1"]), ptr(t["wfc2_t"]), ptr(t["bfc2"]),
-                ptr(states if states is not None else None),
-                ptr(priors_out if states is not None else None),
-                ptr(values_out if states is not None else None), ptr(log_heads), ptr(value_logits))
-        if tile_done is not None:     # overlapped with the tail of the trunk kernel that was launched with the same flags
-            check(lib().lzb_heads_tail_overlapped(*args, ptr(tile_done), stream_ptr(dev)))
-        else:
-            check(lib().lzb_heads_tail(*args, stream_ptr(dev)))
+        check(lib().lzb_heads_tail(ptr(pv), i64(n), ctypes.c_int32(self.pc), ctypes.c_int32(self.vc),
+                                   ctypes.c_int32(self.mlp), ctypes.c_int32(self.bins), ptr(t["wgl_t"]),
+                                   ptr(t["bn2_scale"]), ptr(t["bn2_shift"]), ptr(t["wout"]), ptr(t["wfc1_t"]),
+                                   ptr(t["bfc1"]), ptr(t["wfc2_t"]), ptr(t["bfc2"]),
+                                   ptr(states if states is not None else None),
+                                   ptr(priors_out if states is not None else None),
+                                   ptr(values_out if states is not None else None), ptr(log_heads), ptr(value_logits),
+                                   stream_ptr(dev)))
         if want_raw:
             return log_heads[:, 0], log_heads[:, 1], log_heads[:, 2], value_logits
         return priors_out, values_out
@@ -479,15 +472,10 @@ class InferenceNet:
             self.trunk.use_tc = False            # the tcgen05 path is all or nothing (trunk and heads convolutions)
             self.trunk._probe()
         self.flops_per_state = flops_per_state(self.model)
-        # LZB_TRUNK_IMPL: 1 (default) = the whole trunk + heads conv as ONE persistent kernel (csrc/lz_trunk.cu: activations
-        # stay in shared memory / TMEM across all layers); 0 = one kernel launch per convolution (csrc/lz_conv.cu)
-        # LZB_HEADS_OVERLAP=1: the heads kernel starts under the trunk kernel's tail (per-tile completion flags + a
-        # programmatic dependent launch) instead of after it
-        self.heads_overlap = os.environ.get("LZB_HEADS_OVERLAP", "0") == "1"
-        self._flags: dict = {}
+        # the whole trunk + heads conv as ONE persistent kernel (csrc/lz_trunk.cu: activations stay in shared memory /
+        # TMEM across all layers) where the net fits it; otherwise one kernel launch per convolution (csrc/lz_conv.cu)
         self.fused_trunk = (self._tc_ready() and len(self.model.blocks) <= 10
-                            and self.model.num_input_channels <= 16      # the kernel's stem multiplies 16 input channels
-                            and os.environ.get("LZB_TRUNK_IMPL", "1") != "0")
+                            and self.model.num_input_channels <= 16)     # the kernel's stem multiplies 16 input channels
         self._ft = {}
         self._pv = {}
         if self.fused_trunk:
@@ -527,8 +515,7 @@ class InferenceNet:
             parts += [t[f"bf1_{i}"], t[sn], t[tn]]                   # conv1: bias; conv2: scale | shift
         ws.append(h["conv_wp"])
         parts.append(h["conv_bias"])                                 # heads conv: bias
-        self.w_copies = max(1, int(os.environ.get("LZB_TRUNK_W_COPIES", "1")))
-        w_trunk = torch.cat(ws * self.w_copies, 0).contiguous()
+        w_trunk = torch.cat(ws, 0).contiguous()
         params = torch.cat([p_.float().reshape(-1) for p_ in parts]).to(dev).contiguous()
         for name, val in (("w_trunk", w_trunk), ("params", params)):
             if name in self._ft:
@@ -536,17 +523,7 @@ class InferenceNet:
             else:
                 self._ft[name] = val.clone()
 
-    def _tile_flags(self, n: int) -> Optional[torch.Tensor]:
-        """Completion flags shared by the trunk kernel and the overlapped heads kernel (LZB_HEADS_OVERLAP=1), or None."""
-        if not self.heads_overlap:
-            return None
-        f = self._flags.get(n)
-        if f is None:
-            extra = 4096 + 4096 if os.environ.get("LZB_OVERLAP_TRACE") else 0       # debug: block start / CTA end stamps
-            f = self._flags[n] = torch.zeros(((n + 2) // 3 + 1 + extra,), dtype=torch.int32, device=self.device)
-        return f
-
-    def _trunk_heads_conv(self, x: torch.Tensor, tile_done: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def _trunk_heads_conv(self, x: torch.Tensor) -> torch.Tensor:
         """planes bf16 [n,64,6,6] channels-last -> relu(bn(conv1)) of both heads, bf16 [n,128,6,6] channels-last: stem,
         every residual block and the heads' 1x1 conv in ONE kernel launch (lzb_trunk_bf16)."""
         import ctypes
@@ -561,12 +538,9 @@ class InferenceNet:
         if pv is None:
             pv = self._pv[n] = torch.empty((n, 128, 6, 6), dtype=torch.bfloat16, device=x.device,
                                            memory_format=torch.channels_last)
-        args = (ptr(x), i64(n), ptr(self.trunk._t["stem_wp"]), ptr(self._ft["w_trunk"]), ctypes.c_int32(self.w_copies),
-                ptr(self._ft["params"]), ctypes.c_int32(len(self.model.blocks)), ptr(pv))
-        if tile_done is not None:
-            check(lib().lzb_trunk_bf16_signal(*args, ptr(tile_done), stream_ptr(x.device)))
-        else:
-            check(lib().lzb_trunk_bf16(*args, stream_ptr(x.device)))
+        check(lib().lzb_trunk_bf16(ptr(x), i64(n), ptr(self.trunk._t["stem_wp"]), ptr(self._ft["w_trunk"]),
+                                   ptr(self._ft["params"]), ctypes.c_int32(len(self.model.blocks)), ptr(pv),
+                                   stream_ptr(x.device)))
         return pv
 
     def load_state_dict(self, state_dict) -> None:
@@ -589,8 +563,7 @@ class InferenceNet:
         if self.trunk is not None:
             with torch.cuda.device(self.device):
                 if self.fused_trunk:
-                    fl = self._tile_flags(x.size(0))
-                    return self.heads(None, want_raw=True, pv=self._trunk_heads_conv(x, fl), tile_done=fl)
+                    return self.heads(None, want_raw=True, pv=self._trunk_heads_conv(x))
                 a = self.trunk(x)
                 if self.heads is not None:
                     return self.heads(a, want_raw=True)
@@ -606,9 +579,8 @@ class InferenceNet:
         (priors f32[n,220] = softmax over each state's legal actions, values f32[n] = bucket expectation)."""
         with torch.cuda.device(self.device):
             if self.fused_trunk:
-                fl = self._tile_flags(x.size(0))
                 return self.heads(None, states, priors_out=priors_out, values_out=values_out,
-                                  pv=self._trunk_heads_conv(x, fl), tile_done=fl)
+                                  pv=self._trunk_heads_conv(x))
             if self.trunk is not None and self.heads is not None:
                 return self.heads(self.trunk(x), states, priors_out=priors_out, values_out=values_out)
             from .tree import heads_to_priors

@@ -137,7 +137,7 @@ _LIBRARY_CONV = ("cudnn", "convolve", "nvjet", "cutlass", "xmma", "gemm", "impli
 
 def test_no_library_convolution_for_any_batch_size():
     """One convolution path: batches that are not multiples of 64 (a `_split_games` share of 65,311 positions through
-    the drop-in `InferenceNet.forward`, a 4,000-game tree search) run on `conv_tc_kernel` with padded tiles -- not a
+    the drop-in `InferenceNet.forward`, a 4,000-game tree search) run on `trunk_kernel` with padded tiles -- not a
     single cuDNN / cuBLAS / CUTLASS kernel is launched (kernel names from torch.profiler)."""
     from liuzhou_b200 import native
     from liuzhou_b200.net import ChessNet, InferenceNet
