@@ -237,25 +237,23 @@ typedef struct {
 
 /* Reset the arena to `num_trees` unexpanded roots (PortableTreeBatch ctor, :443-459). active u8[T] or NULL. */
 LZB_API int lzb_tree_init_roots(const lzb_tree *tree, const uint64_t *root_states, const uint8_t *active, void *stream);
-/* prepare_roots / select_leaves (:483-552): per slot (tree*K + k): leaf_node i32 (-1 if none), leaf_status i32
- * (0 = evaluate, 1 = terminal/inactive, already backed up, 2 = duplicate of a pending leaf), leaf_states u64[.,4].
+/* select_leaves (:515-552) or, with roots_only = 1, prepare_roots (:483-513).  Per slot (tree*K + k): leaf_node i32
+ * (-1 if none), leaf_status i32 (0 = evaluate, 1 = terminal/inactive, already backed up, 2 = duplicate of a pending leaf),
+ * leaf_states u64[.,4].
  * leaf_path i32[slots][LZB_TREE_PATH_STRIDE] (optional, may be NULL): the descent's node path ([0,32) node per depth,
  * [32] depth or -1 if deeper than 32, [33] colour bits) so that lzb_tree_expand_backup can back up the whole path in
- * one memory round trip instead of walking the parent chain. */
+ * one memory round trip instead of walking the parent chain.
+ * roots_only = 1 (requires K = 1; leaf_path and virtual_loss are ignored, and exploration_weight has no effect because
+ * nothing is descended): one slot per tree; only an UNEXPANDED, non-terminal, active root becomes a pending leaf
+ * (status 0) -- a root that kept its subtree through lzb_tree_advance_roots is left alone (status 1).
+ * inputs_c64 (optional, may be NULL; 16-byte aligned): bf16 [slots,6,6,64] channels-last; the kernel also writes the
+ * network input of every status-0 slot, the planes of lzb_encode_inputs_packed layout 2, which saves a separate
+ * encoding launch per simulation wave.  Only channels 0..15 of those rows are written: channels 16..63 must already be
+ * zero (the caller zero-fills the buffer once), and the rows of all other slots are left untouched. */
 #define LZB_TREE_PATH_STRIDE 34
 LZB_API int lzb_tree_select(const lzb_tree *tree, int32_t K, double exploration_weight, double virtual_loss,
                             int32_t *leaf_node, int32_t *leaf_status, uint64_t *leaf_states, int32_t *leaf_path,
-                            void *stream);
-/* lzb_tree_select (roots_only = 0) or lzb_tree_prepare_roots (roots_only = 1, K = 1) that ALSO writes the network input
- * of every status-0 slot: inputs_c64 = bf16 [slots,6,6,64] channels-last, the planes of lzb_encode_inputs_packed
- * layout 2 (rows of other slots are left untouched) -- saves the separate encoding launch in every simulation wave. */
-LZB_API int lzb_tree_select_encode(const lzb_tree *tree, int32_t K, double exploration_weight, double virtual_loss,
-                                   int32_t *leaf_node, int32_t *leaf_status, uint64_t *leaf_states, int32_t *leaf_path,
-                                   int32_t roots_only, void *inputs_c64, void *stream);
-/* prepare_roots proper (:483-513): one slot per tree; only an UNEXPANDED, non-terminal, active root becomes a pending
- * leaf (status 0) -- a root that kept its subtree through lzb_tree_advance_roots is left alone (status 1). */
-LZB_API int lzb_tree_prepare_roots(const lzb_tree *tree, int32_t *leaf_node, int32_t *leaf_status, uint64_t *leaf_states,
-                                   void *stream);
+                            int32_t roots_only, void *inputs_c64, void *stream);
 /* advance_roots (:739-768) + the start of new games, with subtree reuse: for every tree the child reached by
  * actions[t] (i32, an action index in [0,220)) becomes the root and keeps its subtree; actions[t] < 0 or an inactive
  * tree keeps the tree unchanged; reset_mask[t] != 0 (optional, with reset_states u64[T,4]) replaces the tree by a
@@ -275,7 +273,7 @@ LZB_API int lzb_tree_expand_backup(const lzb_tree *tree, int32_t K, const int32_
 /* complete_pending of wave w + select_leaves of wave w + 1 in ONE launch (trees are independent, so each warp expands,
  * backs up and descends again without a grid-wide barrier): same arguments as the two calls; leaf_node / leaf_status /
  * leaf_states / leaf_path are read (wave w) and then rewritten (wave w + 1); inputs_c64 (optional, may be NULL) receives
- * the new leaves' network input as in lzb_tree_select_encode. */
+ * the new leaves' network input as in lzb_tree_select, with the same zero-padding precondition. */
 LZB_API int lzb_tree_expand_select(const lzb_tree *tree, int32_t K, int32_t *leaf_node, int32_t *leaf_status,
                                    const float *priors, const float *values, double exploration_weight, double virtual_loss,
                                    uint64_t *leaf_states, int32_t *leaf_path, void *inputs_c64, void *stream);

@@ -25,15 +25,6 @@ using namespace lz;
 namespace lzb {
 namespace {
 
-// Debug timeline (LZB_TREE_TRACE=1): clock64 stamps of lane 0 of the first warp of blocks 0, 64, 128, ... (8 warps x 32
-// stamps) inside tree_expand_select_kernel; read back with lzb_tree_debug_trace.  nullptr in normal runs.
-__device__ unsigned long long* d_tree_trace = nullptr;
-#define LZB_TSTAMP(i)                                                                                   \
-    do {                                                                                                \
-        if (d_tree_trace && lane == 0 && (threadIdx.x >> 5) == 0 && (blockIdx.x & 63) == 0 && blockIdx.x < 512) \
-            d_tree_trace[(blockIdx.x >> 6) * 32 + (i)] = clock64();                                     \
-    } while (0)
-
 constexpr int32_t kFlagArena = 1, kFlagIllegalAdvance = 2, kFlagBadNetwork = 4;   // sticky bits of counters[1]
 constexpr uint32_t kInfoActionMask = 0xFFu;
 constexpr uint32_t kInfoTerminal = 1u << 16;
@@ -188,7 +179,6 @@ __device__ __forceinline__ void select_tree(const lzb_tree& A, int64_t t, int K,
             // SelectPath :862-874.  One dependent HBM round trip per level: the sibling scan also fetches each
             // child's first_child / info / visit, so the next level needs nothing else from the chosen child.
             int fc = A.first_child[node], nv = A.visit[node];
-            LZB_TSTAMP(8);
             int depth = 0, path_node = lane == 0 ? node : -1, scanned = 0;
             bool path_white = lane == 0 && (inf & kInfoWhite);
             while ((inf & kInfoExpanded) && info_nchild(inf) > 0 && !(inf & kInfoTerminal)) {
@@ -238,9 +228,7 @@ __device__ __forceinline__ void select_tree(const lzb_tree& A, int64_t t, int K,
                 fc = __shfl_sync(0xffffffffu, b_fc, owner);
                 ++depth;
                 if (depth < kPathLanes && lane == depth) { path_node = node; path_white = (inf & kInfoWhite) != 0; }
-                if (depth <= 8) LZB_TSTAMP(8 + depth);
             }
-            LZB_TSTAMP(20);
             const bool recorded = depth < kPathLanes;
             if (lane == 0 && depth > 0) { atomicAdd(&A.counters[4], scanned); atomicAdd(&A.counters[5], depth); }
             const uint32_t white_mask = __ballot_sync(0xffffffffu, path_white);
@@ -289,9 +277,6 @@ __device__ __forceinline__ void select_tree(const lzb_tree& A, int64_t t, int K,
             }
             if (lane == 0) { leaf_node[slot] = status == kLeafEval ? node : -1; leaf_status[slot] = status; }
             __syncwarp();
-            LZB_TSTAMP(21);
-            if (d_tree_trace && lane == 0 && (threadIdx.x >> 5) == 0 && (blockIdx.x & 63) == 0 && blockIdx.x < 512)
-                d_tree_trace[(blockIdx.x >> 6) * 32 + 22] = (unsigned long long)depth;
         }
     }
 }
@@ -307,9 +292,9 @@ tree_select_kernel(lzb_tree A, int K, double c_puct, double vl, int32_t* __restr
         select_tree(A, t, K, c_puct, vl, leaf_node, leaf_status, leaf_states, leaf_path, roots_only, enc_out, lane);
 }
 
-#ifndef LZB_EXPAND_MIN_BLOCKS
-#define LZB_EXPAND_MIN_BLOCKS 3
-#endif
+// Both expand kernels ask for 3 blocks of 8 warps per SM; tree_expand_select_kernel says why.
+constexpr int kExpandMinBlocks = 3;
+
 // Expand (portable_mcts.cpp:894-939) + Backup for every evaluated leaf slot of a tree, sequentially in slot
 // order (deterministic).  priors f32[slots,220] dense over the 220-d action space, values f32[slots].
 // (spri = this warp's 220-float staging row in shared memory)
@@ -326,7 +311,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
         }
         for (int k = 0; k < K; ++k) {
             const int64_t slot = base * K + k;
-            LZB_TSTAMP(0);
             // Everything whose address depends only on the slot is requested in ONE round trip, before the status is
             // looked at (all of it is valid memory for any slot): status, node, value, this lane's 7 prior entries, the
             // descent's path.  The second round trip fetches what hangs off the node / the path.
@@ -348,7 +332,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
             }
             if (st != kLeafEval) continue;
             const int node = node_raw;
-            LZB_TSTAMP(1);
             // statistics of the path nodes for the backup at the end: only this warp touches this tree, so they cannot
             // change in between -- except through this warp's own virtual-loss bookkeeping (K > 1), which re-reads
             const bool pre_backup = do_backup && path_depth >= 0 && !(K > 1 && vl > 0.0);
@@ -362,7 +345,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
             const int n = legal_count(L);
             double value = (double)value_f;
             const uint32_t inf = A.info[node] & ~kInfoPending;
-            LZB_TSTAMP(2);
             if (lane == 0 && K > 1 && vl > 0.0) virtual_loss_path(A, node, vl, -1);
             __syncwarp();
             // CompletePending / Expand throw on a non-finite value or a negative / non-finite prior
@@ -382,7 +364,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
             }
             __syncwarp();                         // staging writes visible to lane 0's sequential sum below
             bad = __any_sync(0xffffffffu, bad);
-            LZB_TSTAMP(3);
             if (bad) {
                 if (lane == 0) { A.info[node] = inf; atomicOr(&A.counters[1], kFlagBadNetwork); }
                 __syncwarp();
@@ -421,7 +402,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
                             if (j0 + j < m) prior_sum = __dadd_rn(prior_sum, (double)v[j]);
                     }
                 }
-                LZB_TSTAMP(4);
                 if (lane == 0) {
                     // the bump pointer only grows: after the first failure every later allocation fails too, so
                     // [num_trees, first failed index) is exactly the set of valid nodes (advance_roots relies on it)
@@ -429,7 +409,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
                     else atomicAdd(&A.counters[2], 1);
                 }
                 fc = __shfl_sync(0xffffffffu, fc, 0);
-                LZB_TSTAMP(5);
                 if (fc >= 0) {
                     const bool uniform = !(prior_sum > 0.0) || isinf(prior_sum);      // :919
                     for (int i = lane, r = 0; i < n; i += 32, ++r) {   // child i <-> i-th legal action in ascending index order
@@ -458,7 +437,6 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
                 }
             }
             __syncwarp();
-            LZB_TSTAMP(6);
             if (do_backup) {
                 if (pre_backup) {                 // backup_recorded with the statistics fetched at the top: stores only
                     if (lane <= path_depth) {
@@ -470,12 +448,11 @@ __device__ __forceinline__ void expand_tree(const lzb_tree& A, int64_t t, int K,
                 else if (lane == 0) backup_path(A, node, value);
             }
             __syncwarp();
-            LZB_TSTAMP(7);
         }
     }
 }
 
-__global__ void __launch_bounds__(kThreads, LZB_EXPAND_MIN_BLOCKS)
+__global__ void __launch_bounds__(kThreads, kExpandMinBlocks)
 tree_expand_kernel(lzb_tree A, int K, const int32_t* __restrict__ leaf_node, const int32_t* __restrict__ leaf_status,
                    const float* __restrict__ priors, const float* __restrict__ values, int do_backup, double vl,
                    const int32_t* __restrict__ leaf_path) {
@@ -491,17 +468,16 @@ tree_expand_kernel(lzb_tree A, int K, const int32_t* __restrict__ leaf_node, con
 // latency chains of a warp run back to back without a grid-wide barrier between them, and a simulation wave needs one
 // tree kernel instead of two (select -> network -> expand becomes network -> expand+select).  The warp's own writes
 // (children, statistics along the path) are ordered before its reads by __syncwarp().
-// WPB warps per block, at least MINB blocks per SM: 4,096 trees are 4,096 warps = 27.7 per SM; <8, 3> (80 registers) keeps
-// only 24 resident, so 13 % of the blocks wait for a second round and the kernel lasts two latency chains.
-template <int WPB, int MINB>
-__global__ void __launch_bounds__(WPB * 32, MINB)
+// 4,096 trees are 4,096 warps = 27.7 per SM; 3 blocks of 8 warps (80 registers) keep only 24 resident, so 13 % of the
+// blocks wait for a second round and the kernel lasts two latency chains.
+__global__ void __launch_bounds__(kThreads, kExpandMinBlocks)
 tree_expand_select_kernel(lzb_tree A, int K, int32_t* __restrict__ leaf_node, int32_t* __restrict__ leaf_status,
                           const float* __restrict__ priors, const float* __restrict__ values, double c_puct, double vl,
                           uint64_t* __restrict__ leaf_states, int32_t* __restrict__ leaf_path, uint4* __restrict__ enc_out) {
-    __shared__ float s_pri[WPB][kActionDim];
+    __shared__ float s_pri[kWarpsPerBlock][kActionDim];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int64_t warp = (int64_t)blockIdx.x * WPB + w;
-    const int64_t nwarps = (int64_t)gridDim.x * WPB;
+    const int64_t warp = (int64_t)blockIdx.x * kWarpsPerBlock + w;
+    const int64_t nwarps = (int64_t)gridDim.x * kWarpsPerBlock;
     for (int64_t t = warp; t < A.num_trees; t += nwarps) {
         expand_tree(A, t, K, leaf_node, leaf_status, priors, values, 1, vl, leaf_path, s_pri[w], lane);
         __syncwarp();
@@ -891,41 +867,19 @@ extern "C" int lzb_tree_init_roots(const lzb_tree* tree, const uint64_t* root_st
 }
 
 extern "C" int lzb_tree_select(const lzb_tree* tree, int32_t K, double c_puct, double virtual_loss, int32_t* leaf_node,
-                               int32_t* leaf_status, uint64_t* leaf_states, int32_t* leaf_path, void* stream) {
+                               int32_t* leaf_status, uint64_t* leaf_states, int32_t* leaf_path, int32_t roots_only,
+                               void* inputs_c64, void* stream) {
     int rc = check_tree(tree);
     if (rc) return rc;
     LZB_REQUIRE(K >= 1 && K <= 64, "leaves per tree per wave must be in [1, 64]");
     LZB_REQUIRE(c_puct >= 0.0 && c_puct == c_puct, "exploration_weight must be finite and non-negative");
     LZB_REQUIRE(leaf_node && leaf_status && leaf_states, "null output");
-    tree_select_kernel<<<warp_grid(tree->num_trees), kThreads, 0, (cudaStream_t)stream>>>(
-        *tree, K, c_puct, virtual_loss, leaf_node, leaf_status, leaf_states, leaf_path, 0, nullptr);
-    return check_launch("tree_select_kernel");
-}
-
-extern "C" int lzb_tree_select_encode(const lzb_tree* tree, int32_t K, double c_puct, double virtual_loss, int32_t* leaf_node,
-                                      int32_t* leaf_status, uint64_t* leaf_states, int32_t* leaf_path, int32_t roots_only,
-                                      void* inputs_c64, void* stream) {
-    int rc = check_tree(tree);
-    if (rc) return rc;
-    LZB_REQUIRE(K >= 1 && K <= 64, "leaves per tree per wave must be in [1, 64]");
-    LZB_REQUIRE(c_puct >= 0.0 && c_puct == c_puct, "exploration_weight must be finite and non-negative");
-    LZB_REQUIRE(leaf_node && leaf_status && leaf_states && inputs_c64, "null output");
     LZB_REQUIRE(!roots_only || K == 1, "prepare_roots uses one slot per tree");
     LZB_REQUIRE((reinterpret_cast<uintptr_t>(inputs_c64) & 15) == 0, "inputs must be 16-byte aligned");
     tree_select_kernel<<<warp_grid(tree->num_trees), kThreads, 0, (cudaStream_t)stream>>>(
         *tree, K, c_puct, roots_only ? 0.0 : virtual_loss, leaf_node, leaf_status, leaf_states, roots_only ? nullptr : leaf_path,
         roots_only ? 1 : 0, reinterpret_cast<uint4*>(inputs_c64));
-    return check_launch("tree_select_kernel(+encode)");
-}
-
-extern "C" int lzb_tree_prepare_roots(const lzb_tree* tree, int32_t* leaf_node, int32_t* leaf_status,
-                                      uint64_t* leaf_states, void* stream) {
-    int rc = check_tree(tree);
-    if (rc) return rc;
-    LZB_REQUIRE(leaf_node && leaf_status && leaf_states, "null output");
-    tree_select_kernel<<<warp_grid(tree->num_trees), kThreads, 0, (cudaStream_t)stream>>>(
-        *tree, 1, 0.0, 0.0, leaf_node, leaf_status, leaf_states, nullptr, 1, nullptr);
-    return check_launch("tree_select_kernel(roots)");
+    return check_launch("tree_select_kernel");
 }
 
 extern "C" int lzb_tree_advance_roots(const lzb_tree* tree, const lzb_tree* scratch, const int32_t* actions,
@@ -963,13 +917,6 @@ extern "C" int lzb_tree_expand_backup(const lzb_tree* tree, int32_t K, const int
     return check_launch("tree_expand_kernel");
 }
 
-static unsigned long long* g_tree_trace_buf = nullptr;
-// debug: copy the stamps of the last tree_expand_select_kernel launch (LZB_TREE_TRACE=1) to host memory (256 u64)
-extern "C" __attribute__((visibility("default"))) int lzb_tree_debug_trace(unsigned long long* host_out) {
-    if (!g_tree_trace_buf) return LZB_ERR_INVALID_ARGUMENT;
-    return cudaMemcpy(host_out, g_tree_trace_buf, 256 * 8, cudaMemcpyDeviceToHost) == cudaSuccess ? LZB_OK : LZB_ERR_CUDA;
-}
-
 extern "C" int lzb_tree_expand_select(const lzb_tree* tree, int32_t K, int32_t* leaf_node, int32_t* leaf_status,
                                       const float* priors, const float* values, double c_puct, double virtual_loss,
                                       uint64_t* leaf_states, int32_t* leaf_path, void* inputs_c64, void* stream) {
@@ -979,25 +926,9 @@ extern "C" int lzb_tree_expand_select(const lzb_tree* tree, int32_t K, int32_t* 
     LZB_REQUIRE(c_puct >= 0.0 && c_puct == c_puct, "exploration_weight must be finite and non-negative");
     LZB_REQUIRE(leaf_node && leaf_status && priors && values && leaf_states && leaf_path, "null pointer");
     LZB_REQUIRE((reinterpret_cast<uintptr_t>(inputs_c64) & 15) == 0, "inputs must be 16-byte aligned");
-    static const int variant = getenv("LZB_TREE_VARIANT") ? atoi(getenv("LZB_TREE_VARIANT")) : 0;
-    static const bool trace = getenv("LZB_TREE_TRACE") && atoi(getenv("LZB_TREE_TRACE")) != 0;
-    if (trace && !g_tree_trace_buf) {
-        cudaMalloc(&g_tree_trace_buf, 256 * 8);
-        cudaMemset(g_tree_trace_buf, 0, 256 * 8);
-        cudaMemcpyToSymbol(d_tree_trace, &g_tree_trace_buf, sizeof(g_tree_trace_buf));
-    }
-    uint4* enc = reinterpret_cast<uint4*>(inputs_c64);
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t T = tree->num_trees;
-    if (variant == 1)
-        tree_expand_select_kernel<8, 4><<<warp_grid(T), 256, 0, s>>>(*tree, K, leaf_node, leaf_status, priors, values, c_puct,
-                                                                     virtual_loss, leaf_states, leaf_path, enc);
-    else if (variant == 2)
-        tree_expand_select_kernel<4, 7><<<(unsigned)((T + 3) / 4), 128, 0, s>>>(*tree, K, leaf_node, leaf_status, priors, values,
-                                                                                c_puct, virtual_loss, leaf_states, leaf_path, enc);
-    else
-        tree_expand_select_kernel<8, 3><<<warp_grid(T), 256, 0, s>>>(*tree, K, leaf_node, leaf_status, priors, values, c_puct,
-                                                                     virtual_loss, leaf_states, leaf_path, enc);
+    tree_expand_select_kernel<<<warp_grid(tree->num_trees), kThreads, 0, (cudaStream_t)stream>>>(
+        *tree, K, leaf_node, leaf_status, priors, values, c_puct, virtual_loss, leaf_states, leaf_path,
+        reinterpret_cast<uint4*>(inputs_c64));
     return check_launch("tree_expand_select_kernel");
 }
 

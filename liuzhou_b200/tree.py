@@ -105,32 +105,18 @@ class DeviceTreeBatch:
     def _select(self, k: int, roots_only: bool, encode_out: Optional[torch.Tensor]) -> None:
         node, status, states = ((self.root_leaf_node, self.root_leaf_status, self.root_leaf_states) if roots_only
                                 else (self.leaf_node, self.leaf_status, self.leaf_states))
+        _check_encode_out(encode_out, self.num_trees * k)
         with torch.cuda.device(self.device):
-            if encode_out is not None:
-                # fused: the kernel also writes the bf16 [slots,6,6,64] network input of every pending leaf
-                slots = self.num_trees * k
-                if (encode_out.dtype != torch.bfloat16 or encode_out.dim() != 4 or encode_out.size(0) < slots
-                        or tuple(encode_out.shape[1:]) != (64, 6, 6)
-                        or not encode_out.is_contiguous(memory_format=torch.channels_last)):
-                    raise RuntimeError(f"encode_out must be bfloat16 [>={slots},64,6,6] in channels_last memory format")
-                check(lib().lzb_tree_select_encode(
-                    ctypes.byref(self._struct), ctypes.c_int32(k), ctypes.c_double(self.exploration_weight),
-                    ctypes.c_double(self.virtual_loss), ptr(node), ptr(status), ptr(states),
-                    ptr(None if roots_only else self.leaf_path), ctypes.c_int32(1 if roots_only else 0), ptr(encode_out),
-                    stream_ptr(self.device)))
-            elif roots_only:
-                check(lib().lzb_tree_prepare_roots(ctypes.byref(self._struct), ptr(node), ptr(status), ptr(states),
-                                                   stream_ptr(self.device)))
-            else:
-                check(lib().lzb_tree_select(ctypes.byref(self._struct), ctypes.c_int32(k),
-                                            ctypes.c_double(self.exploration_weight), ctypes.c_double(self.virtual_loss),
-                                            ptr(node), ptr(status), ptr(states), ptr(self.leaf_path),
-                                            stream_ptr(self.device)))
+            check(lib().lzb_tree_select(ctypes.byref(self._struct), ctypes.c_int32(k),
+                                        ctypes.c_double(self.exploration_weight), ctypes.c_double(self.virtual_loss),
+                                        ptr(node), ptr(status), ptr(states), ptr(None if roots_only else self.leaf_path),
+                                        ctypes.c_int32(1 if roots_only else 0), ptr(encode_out), stream_ptr(self.device)))
 
     def prepare_roots(self, encode_out: Optional[torch.Tensor] = None) -> None:
         """Unexpanded, non-terminal, active roots become the pending leaves (one slot per tree, whatever K is);
         roots that kept their subtree through advance_roots() need no evaluation (portable_mcts.cpp:483-513).
-        ``encode_out`` (bf16 [T,64,6,6] channels-last): also write the pending roots' network input in the same launch."""
+        ``encode_out`` (bf16 [T,64,6,6] channels-last): also write the pending roots' network input in the same launch
+        (channels 0..15 of the pending rows; channels 16..63 must already be zero, other rows are left untouched)."""
         self._select(1, True, encode_out)
         self._pending_is_root = True
 
@@ -215,7 +201,8 @@ class DeviceTreeBatch:
                 "moves_since_capture": ((meta >> 22) & 63).to(torch.int32), "game_over": over}
 
     def select_leaves(self, encode_out: Optional[torch.Tensor] = None) -> None:
-        """One descent per leaf slot; ``encode_out`` (bf16 [T*K,64,6,6] channels-last) fuses the input encoding in."""
+        """One descent per leaf slot; ``encode_out`` (bf16 [T*K,64,6,6] channels-last) fuses the input encoding in: channels
+        0..15 of the pending rows are written, channels 16..63 must already be zero, other rows are left untouched."""
         self._select(self.k, False, encode_out)
         self._pending_is_root = False
 
@@ -255,7 +242,8 @@ class DeviceTreeBatch:
                             encode_out: Optional[torch.Tensor] = None) -> None:
         """``complete_pending`` of the current wave followed by ``select_leaves`` of the next one in ONE launch
         (``lzb_tree_expand_select``): trees are independent, so every warp expands, backs up and descends again without a
-        grid-wide barrier in between.  Only after ``select_leaves`` (not after ``prepare_roots``)."""
+        grid-wide barrier in between.  Only after ``select_leaves`` (not after ``prepare_roots``).  ``encode_out`` as in
+        ``select_leaves``: channels 16..63 must already be zero."""
         if self._pending_is_root:
             raise RuntimeError("complete_and_select follows select_leaves, not prepare_roots")
         slots = self.num_trees * self.k
@@ -264,10 +252,7 @@ class DeviceTreeBatch:
         require_cuda(priors, "priors")
         p = priors.to(torch.float32).contiguous()
         v = values.to(torch.float32).contiguous()
-        if encode_out is not None and (encode_out.dtype != torch.bfloat16 or encode_out.dim() != 4
-                                       or encode_out.size(0) < slots or tuple(encode_out.shape[1:]) != (64, 6, 6)
-                                       or not encode_out.is_contiguous(memory_format=torch.channels_last)):
-            raise RuntimeError(f"encode_out must be bfloat16 [>={slots},64,6,6] in channels_last memory format")
+        _check_encode_out(encode_out, slots)
         with torch.cuda.device(self.device):
             check(lib().lzb_tree_expand_select(ctypes.byref(self._struct), ctypes.c_int32(self.k), ptr(self.leaf_node),
                                                ptr(self.leaf_status), ptr(p), ptr(v),
@@ -351,6 +336,14 @@ class DeviceTreeBatch:
 
     def check_capacity(self) -> None:
         self._raise_flags(int(self.counters[1].item()))
+
+
+def _check_encode_out(encode_out: Optional[torch.Tensor], slots: int) -> None:
+    """The fused select kernels write the network input of every pending slot as bf16 channels-last [slots,6,6,64]."""
+    if encode_out is not None and (encode_out.dtype != torch.bfloat16 or encode_out.dim() != 4
+                                   or encode_out.size(0) < slots or tuple(encode_out.shape[1:]) != (64, 6, 6)
+                                   or not encode_out.is_contiguous(memory_format=torch.channels_last)):
+        raise RuntimeError(f"encode_out must be bfloat16 [>={slots},64,6,6] in channels_last memory format")
 
 
 def encode_inputs(packed: torch.Tensor, layout: str = "f32_nchw", out: Optional[torch.Tensor] = None) -> torch.Tensor:

@@ -7,7 +7,6 @@ evaluate -> expand + backup) -> root outputs -> policy from visit counts.
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass
 from typing import Optional
 
@@ -51,6 +50,13 @@ class TreeSearchOutput:
     chosen_action_indices: torch.Tensor   # int64[T], -1 for terminal roots
 
 
+def _capture_graph(graph: torch.cuda.CUDAGraph, pool=None) -> torch.cuda.graph:
+    """Capture checked on this thread only: other threads may keep using CUDA meanwhile.  The shard writer's thread
+    (``AsyncShardWriter``) waits on its copies of the previous group of games while the next group's engine captures;
+    torch's default "global" mode fails that wait with cudaErrorStreamCaptureUnsupported."""
+    return torch.cuda.graph(graph, pool=pool, capture_error_mode="thread_local")
+
+
 class TreeMCTS:
     def __init__(self, net: InferenceNet, num_trees: int, config: TreeMCTSConfig, device=None):
         self.net = net
@@ -78,8 +84,6 @@ class TreeMCTS:
         self._root_val = torch.zeros((tp,), dtype=torch.float32, device=dev)
         self._wave_pri = self._root_pri if k == 1 else torch.zeros((sp, ACTION_DIM), dtype=torch.float32, device=dev)
         self._wave_val = self._root_val if k == 1 else torch.zeros((sp,), dtype=torch.float32, device=dev)
-        self._unroll = max(1, int(os.environ.get("LZB_WAVE_UNROLL", "1")))
-        self._unrolled: dict = {}
         self._wave_graph: Optional[torch.cuda.CUDAGraph] = None
         self._root_graph: Optional[torch.cuda.CUDAGraph] = None
         self.root_graph_launches = self.wave_graph_launches = self.search_extra_launches = 0
@@ -122,7 +126,6 @@ class TreeMCTS:
             return
         for b in self.bucket_ladder():
             self._graphs_for(b)
-            self._unrolled_for(b)
         self._buckets_warm = True
 
     def set_live(self, active: Optional[torch.Tensor]) -> None:
@@ -138,10 +141,10 @@ class TreeMCTS:
         self._live_set = True
 
     # one network evaluation of the pending leaves + expansion (+ backup).  On the tcgen05 path the network input is
-    # the channel-padded bf16 [n,64,6,6] tensor and the select kernel writes it itself (one launch less per wave).
+    # the channel-padded bf16 [n,64,6,6] tensor and the select kernel writes it itself (one launch less per wave); other
+    # nets (allow_library_convs) take the 11-channel input, written by a separate encoding launch.
     def _fused_encode(self, x: torch.Tensor) -> bool:
-        return (x.dim() == 4 and x.size(1) == 64 and x.dtype == torch.bfloat16
-                and os.environ.get("LZB_FUSED_ENCODE", "1") != "0")
+        return x.dim() == 4 and x.size(1) == 64 and x.dtype == torch.bfloat16
 
     def _eval_pending(self, root: bool, encoded: bool) -> None:
         tree = self.tree
@@ -200,32 +203,12 @@ class TreeMCTS:
             torch.cuda.current_stream(dev).wait_stream(side)
             torch.cuda.synchronize(dev)
             g_mid, g_last = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g_mid, pool=self._root_graph.pool()):
+            with _capture_graph(g_mid, pool=self._root_graph.pool()):
                 self._wave_mid(bucket)
-            with torch.cuda.graph(g_last, pool=self._root_graph.pool()):
+            with _capture_graph(g_last, pool=self._root_graph.pool()):
                 self._wave_last(bucket)
             pair = self._bucket_graphs[bucket] = (g_mid, g_last)
         return pair
-
-    def _unrolled_for(self, bucket: int):
-        """A graph of ``_unroll`` consecutive waves (kernel -> kernel edges inside one graph are cheaper than graph -> graph
-        launches), or None when unrolling is off."""
-        if self._unroll <= 1:
-            return None
-        g = self._unrolled.get(bucket)
-        if g is None:
-            self._graphs_for(bucket)                 # warm-up at this size + the single-wave graphs for the remainder
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g, pool=self._root_graph.pool()):
-                for _ in range(self._unroll):
-                    self._wave_mid(None if bucket >= self.num_trees else bucket)
-            self._unrolled[bucket] = g
-        return g
-
-    def _wave_step(self) -> None:
-        """One stand-alone wave (select -> network -> expand + backup); used by tools and the tree-kernel timing."""
-        self._first_select()
-        self._wave_last()
 
     def _capture(self) -> None:
         dev = self.device
@@ -243,19 +226,19 @@ class TreeMCTS:
         # kernels of OURS inside each graph (every replay launches them again; bench.py's gpu_launches)
         c0 = launch_count()
         self._root_graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self._root_graph):
+        with _capture_graph(self._root_graph):
             self._root_step()
         c1 = launch_count()
         self._first_graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self._first_graph, pool=self._root_graph.pool()):
+        with _capture_graph(self._first_graph, pool=self._root_graph.pool()):
             self._first_select()
         c2 = launch_count()
         self._wave_graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self._wave_graph, pool=self._root_graph.pool()):
+        with _capture_graph(self._wave_graph, pool=self._root_graph.pool()):
             self._wave_mid()
         c3 = launch_count()
         self._last_graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self._last_graph, pool=self._root_graph.pool()):
+        with _capture_graph(self._last_graph, pool=self._root_graph.pool()):
             self._wave_last()
         c4 = launch_count()
         self.root_graph_launches, self.wave_graph_launches = c1 - c0, c3 - c2
@@ -322,14 +305,8 @@ class TreeMCTS:
             self._apply_root_noise()
         if use_graph:
             g_mid, g_last = self._graphs_for(bucket)
-            g_many = self._unrolled_for(bucket)
             self._first_graph.replay()
-            left = self.waves - 1
-            if g_many is not None:
-                for _ in range(left // self._unroll):
-                    g_many.replay()
-                left %= self._unroll
-            for _ in range(left):
+            for _ in range(self.waves - 1):
                 g_mid.replay()
             g_last.replay()
         else:

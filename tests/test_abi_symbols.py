@@ -1,5 +1,5 @@
-"""The C-ABI shared library loads on a CPU-only box and exports every symbol include/liuzhou_b200.h declares
-(no compute calls without a GPU)."""
+"""The C-ABI shared library loads on a CPU-only box and exports exactly the lzb_* symbols include/liuzhou_b200.h
+declares (no compute calls without a GPU)."""
 import ctypes
 import re
 from pathlib import Path
@@ -14,6 +14,9 @@ def _declared():
 
 
 def test_library_exports_every_declared_symbol():
+    import shutil
+    import subprocess
+
     from liuzhou_b200 import build
 
     lib_path = build.build()
@@ -24,6 +27,13 @@ def test_library_exports_every_declared_symbol():
     assert not missing, f"declared in include/liuzhou_b200.h but not exported: {missing}"
     lib.lzb_version.restype = ctypes.c_char_p
     assert b"sm_100a" in lib.lzb_version()
+    # and the reverse: nothing callable is exported that the header does not document
+    nm = shutil.which("nm") or str(Path(build.nvcc()).with_name("nm"))
+    out = subprocess.run([nm, "-D", "--defined-only", str(lib_path)], capture_output=True, text=True, check=True).stdout
+    exported = set(re.findall(r"^\S+\s+\w\s+(lzb_[a-z0-9_]+)$", out, flags=re.M))
+    assert set(names) <= exported, "nm output was not parsed"
+    undeclared = sorted(exported - set(names))
+    assert not undeclared, f"exported but not declared in include/liuzhou_b200.h: {undeclared}"
 
 
 def test_library_is_sm100a_only():
