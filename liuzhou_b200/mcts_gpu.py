@@ -154,10 +154,7 @@ class V1RootMCTS:
 
     # -- network -------------------------------------------------------------------------------------
     def _forward_model(self, inputs_f32: torch.Tensor):
-        if self.net._tc_ready():          # chunked, padded batches straight onto our tcgen05 convolutions
-            return self.net.forward(inputs_f32)
-        x = inputs_f32.to(dtype=self.net.dtype).contiguous(memory_format=torch.channels_last)
-        return self.net.forward(x)
+        return self.net.forward(inputs_f32)
 
     def _evaluate_batch(self, batch: GpuStateBatch):
         inputs = states_to_model_input(batch)

@@ -3,25 +3,37 @@ bf16 inference wrapper the search engines use.
 
 The architecture (11 -> 128-channel stem, 10 pre-activation residual blocks, three-head policy with global
 pooling, 101-bucket value head) and every parameter name are the reference's, so its checkpoints
-(``{"model_state_dict": ...}``, v1/train.py:2556) load unchanged.  north_star keeps this one dense contraction
-in PyTorch (cuDNN / cuBLAS on the tensor cores); what is ours is everything around it: inputs are written by our
-kernels directly as bf16 channels-last planes, outputs are consumed by our fused head kernel, and the whole
-forward is replayed from a CUDA graph at fixed batch sizes.
+(``{"model_state_dict": ...}``, v1/train.py:2556) load unchanged.
+
+``InferenceNet`` runs a net on one of four forward paths, chosen once from its shape and dtype (``network_path``):
+  * trunk   -- the product path (128-wide trunk, 64 + 64 head channels, bf16, 1..10 blocks, <= 16 input channels):
+               stem, blocks and heads conv in ONE persistent tcgen05 kernel (csrc/lz_trunk.cu), then heads_tail_kernel;
+  * layered -- the same shape with more blocks or 17..64 input channels: one tcgen05 conv launch per layer
+               (csrc/lz_conv.cu), then heads_tail_kernel;
+  * library -- opt-in (``allow_library_convs``), other bf16 nets of a width divisible by 8: cuDNN convolutions and our
+               bn_relu pass, then heads_tail_kernel (csrc/lz_nn.cu) or, where the heads do not fit it, PyTorch's heads;
+  * module  -- opt-in: the plain ``ChessNet`` module, any dtype.
+Inputs are written by our kernels directly as bf16 channels-last planes (zero-padded to 64 channels on the tcgen05
+paths), and the whole forward is replayed from a CUDA graph at fixed batch sizes.
 
 FLOPs per evaluated state (forward, 2 x MAC): stem 0.91 M + 20 convs x 10.62 M + heads ~1.29 M = 214.5 MFLOP.
 """
 from __future__ import annotations
 
+import copy
+import ctypes
 from typing import Dict, Optional, Tuple
 
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
+from ._lib import check, i64, lib, ptr, require_cuda, stream_ptr
+from .tree import heads_to_priors
+
 NUM_INPUT_CHANNELS = 11
 VALUE_BUCKET_BINS = 101
 BOARD_SIZE = 6
-FLOPS_PER_STATE = 214.5e6
 
 
 class GlobalPool(nn.Module):
@@ -151,11 +163,49 @@ def flops_per_state(model: ChessNet) -> float:
     return total
 
 
+PATHS = ("trunk", "layered", "library", "module")      # a net runs its default path or any later one
+
+
+def heads_kernel_fits(model: ChessNet) -> bool:
+    """Whether heads_tail_kernel (csrc/lz_nn.cu) takes this net's heads."""
+    pc, vc = model.policy_head.conv1.out_channels, model.value_head.conv1.out_channels
+    vh = model.value_head
+    return (pc <= 64 and vc <= 64 and (pc + vc) % 8 == 0 and vh.fc1.out_features <= 128
+            and 2 <= vh.fc2.out_features <= 128)
+
+
+def network_path(model: ChessNet, dtype: torch.dtype = torch.bfloat16, path: Optional[str] = None) -> str:
+    """The forward path (module docstring) of `model` run in `dtype`: with ``path=None`` the default for its shape,
+    otherwise `path` itself, which must be the default or a later entry of PATHS.  Reads only the shape (no GPU)."""
+    width, cin, nb = model.stem_conv.out_channels, model.num_input_channels, len(model.blocks)
+    heads = model.policy_head.conv1.out_channels + model.value_head.conv1.out_channels
+    if dtype != torch.bfloat16 or width % 8 != 0:         # our epilogue kernels work on bf16 in 8-channel vectors
+        default = "module"
+    elif width == heads == 128 and nb >= 1 and cin <= 64 and heads_kernel_fits(model):
+        default = "trunk" if nb <= 10 and cin <= 16 else "layered"    # the trunk kernel's stem multiplies 16 channels
+    else:
+        default = "library"
+    if path is None:
+        return default
+    if path not in PATHS or PATHS.index(path) < PATHS.index(default):
+        raise ValueError(f"network path {path!r} is not available for this ChessNet shape / dtype; it can run "
+                         f"{', '.join(PATHS[PATHS.index(default):])}")
+    return path
+
+
 def _fold_bn(bn: nn.BatchNorm2d):
     """eval-mode BatchNorm as y = scale * x + shift (fp32 vectors)."""
     scale = (bn.weight.float() / torch.sqrt(bn.running_var.float() + bn.eps)).contiguous()
     shift = (bn.bias.float() - bn.running_mean.float() * scale).contiguous()
     return scale, shift
+
+
+def _set(store: Dict[str, torch.Tensor], values: Dict[str, torch.Tensor]) -> None:
+    for name, value in values.items():
+        if name in store:
+            store[name].copy_(value)          # in place: captured CUDA graphs stay valid
+        else:
+            store[name] = value.clone()
 
 
 def pack_conv_weight(w: torch.Tensor) -> torch.Tensor:
@@ -185,10 +235,6 @@ def conv_bf16(x: torch.Tensor, w_packed: torch.Tensor, *, bias: Optional[torch.T
               want_out2: bool = False, out1: Optional[torch.Tensor] = None, out2: Optional[torch.Tensor] = None):
     """Our tcgen05 implicit-GEMM convolution with the fused residual / BatchNorm / ReLU epilogue (lzb_conv_bf16).
     x bf16 [n,128,6,6] channels-last with n % 64 == 0; returns (out1, out2) (None where not requested)."""
-    import ctypes
-
-    from ._lib import check, i64, lib, ptr, require_cuda, stream_ptr
-
     require_cuda(x, "x")
     n, cin, h, w = x.shape
     if (h, w) != (6, 6) or x.dtype != torch.bfloat16 or not x.is_contiguous(memory_format=torch.channels_last):
@@ -206,33 +252,31 @@ def conv_bf16(x: torch.Tensor, w_packed: torch.Tensor, *, bias: Optional[torch.T
     return (out1 if want_out1 else None), (out2 if want_out2 else None)
 
 
-class FusedTrunk:
-    """The ChessNet trunk (src/neural_network.py:250-254) with
-      * cuDNN convolutions (bf16 channels-last implicit GEMMs on the tensor cores, cutlass sm100 kernels),
-      * BatchNorm folded INTO the convolution wherever a BN directly follows a conv (stem_bn -> stem_conv, bn2 ->
-        conv1 of each block) and applied by cuDNN's fused conv + bias + ReLU epilogue (free on B200: same time as
-        the bare conv),
-      * OUR fused kernel (csrc/lz_nn.cu) for the one pass cuDNN cannot absorb: residual add + next block's
-        BatchNorm + ReLU with both the sum and the activation written.
-    Per residual block: 2 tensor-core kernels + 1 HBM-bound pass (PyTorch eager: 2 + ~7)."""
+def bn_relu(u: torch.Tensor, v: Optional[torch.Tensor], scale: torch.Tensor, shift: torch.Tensor, want_sum: bool):
+    """Our eval BatchNorm + ReLU pass (lzb_bn_relu_bf16) on bf16 channels-last [n,C,6,6]: x = u (+ v) ->
+    (x if v is given and want_sum else None, relu(scale * x + shift))."""
+    n, c, h, w = u.shape
+    out_act = torch.empty_like(u)
+    out_sum = torch.empty_like(u) if (v is not None and want_sum) else None
+    check(lib().lzb_bn_relu_bf16(ptr(u), ptr(v), ptr(scale), ptr(shift), i64(n * h * w), ctypes.c_int32(c),
+                                 ptr(out_sum), ptr(out_act), stream_ptr(u.device)))
+    return out_sum, out_act
 
-    def __init__(self, model: "ChessNet"):
+
+class FusedTrunk:
+    """The ChessNet trunk (src/neural_network.py:250-254) with eval BatchNorm folded INTO the conv it follows (stem_bn
+    -> stem_conv, bn2 -> conv1 of each block), on one of two bodies fixed at construction.  ``tc`` (trunk and layered
+    paths): one launch of our tcgen05 conv (csrc/lz_conv.cu) per layer, whose epilogue also does the residual add and
+    the next BatchNorm + ReLU.  Library: cuDNN's fused conv + bias + ReLU (or conv + our bn_relu pass where cuDNN has no
+    engine for the shape), and our bn_relu pass for residual add + next BatchNorm + ReLU."""
+
+    def __init__(self, model: "ChessNet", tc: bool):
         self.model = model
+        self.use_tc = tc
         self._t = {}
         self._act = {}
-        self.use_cudnn_fused = True
-        # our tcgen05 implicit-GEMM conv covers the 128-channel trunk; other widths keep the cuDNN path
-        self.use_tc = (model.stem_conv.out_channels == 128 and model.stem_conv.in_channels <= 64 and len(model.blocks) > 0
-                       and model.stem_conv.weight.dtype == torch.bfloat16)
         self.refresh()
-        if not self.use_tc:
-            self._probe()
-
-    def _set(self, name: str, value: torch.Tensor) -> None:
-        if name in self._t:
-            self._t[name].copy_(value)          # in place: captured CUDA graphs stay valid
-        else:
-            self._t[name] = value.clone()
+        self.use_cudnn_fused = not tc and self._probe()
 
     @staticmethod
     def _fold_into_conv(conv: nn.Conv2d, bn: nn.BatchNorm2d):
@@ -241,39 +285,29 @@ class FusedTrunk:
         return w.contiguous(memory_format=torch.channels_last), shift.to(conv.weight.dtype).contiguous()
 
     def refresh(self) -> None:
-        m = self.model
+        m, v = self.model, {}
         w, b = self._fold_into_conv(m.stem_conv, m.stem_bn)
-        self._set("stem_w", w)
-        self._set("stem_b", b)
-        if self.use_tc and m.stem_conv.in_channels <= 64:     # stem as a K = 64 tcgen05 conv on zero-padded channels
+        if self.use_tc:     # stem as a K = 64 tcgen05 conv on zero-padded channels
             w64 = torch.zeros((w.size(0), 64, 3, 3), dtype=w.dtype, device=w.device)
             w64[:, :m.stem_conv.in_channels] = w
-            self._set("stem_wp", pack_conv_weight(w64))
-            self._set("stem_bf", b.float())
+            v["stem_wp"], v["stem_bf"] = pack_conv_weight(w64), b.float()
+        else:
+            v["stem_w"], v["stem_b"] = w, b
+            v["stem_s"], v["stem_t"] = _fold_bn(m.stem_bn)
         for i, blk in enumerate(m.blocks):
             w, b = self._fold_into_conv(blk.conv1, blk.bn2)
-            self._set(f"w1_{i}", w)
-            self._set(f"b1_{i}", b)
-            if self.use_tc:      # layouts of our tcgen05 convolution (csrc/lz_conv.cu)
-                self._set(f"wp1_{i}", pack_conv_weight(w))
-                self._set(f"bf1_{i}", b.float())
-                self._set(f"wp2_{i}", pack_conv_weight(blk.conv2.weight))
-            s, t = _fold_bn(blk.bn1)
-            self._set(f"s1_{i}", s)
-            self._set(f"t1_{i}", t)
-            s, t = _fold_bn(blk.bn2)
-            self._set(f"s2_{i}", s)
-            self._set(f"t2_{i}", t)
-        s, t = _fold_bn(m.stem_bn)
-        self._set("stem_s", s)
-        self._set("stem_t", t)
-        s, t = _fold_bn(m.trunk_bn)
-        self._set("trunk_s", s)
-        self._set("trunk_t", t)
+            if self.use_tc:     # layouts of our tcgen05 convolution (csrc/lz_conv.cu)
+                v[f"wp1_{i}"], v[f"bf1_{i}"] = pack_conv_weight(w), b.float()
+                v[f"wp2_{i}"] = pack_conv_weight(blk.conv2.weight)
+            else:
+                v[f"w1_{i}"], v[f"b1_{i}"] = w, b
+                v[f"s2_{i}"], v[f"t2_{i}"] = _fold_bn(blk.bn2)
+            v[f"s1_{i}"], v[f"t1_{i}"] = _fold_bn(blk.bn1)
+        v["trunk_s"], v["trunk_t"] = _fold_bn(m.trunk_bn)
+        _set(self._t, v)
 
-    def _probe(self) -> None:
-        """cuDNN's fused conv+bias+ReLU needs engine support for this shape / dtype; fall back to conv + our
-        bn_relu pass if it is not available."""
+    def _probe(self) -> bool:
+        """Whether cuDNN has a fused conv+bias+ReLU engine for this shape / dtype (else: conv + our bn_relu pass)."""
         m = self.model
         try:
             dev = m.stem_conv.weight.device
@@ -283,142 +317,117 @@ class FusedTrunk:
             if len(m.blocks):
                 torch.cudnn_convolution_relu(y, self._t["w1_0"], self._t["b1_0"], [1, 1], [1, 1], [1, 1], 1)
         except Exception:
-            self.use_cudnn_fused = False
-
-    @staticmethod
-    def _bn_relu(u, v, scale, shift, want_sum: bool):
-        import ctypes
-
-        from ._lib import check, i64, lib, ptr, stream_ptr
-
-        n, c, h, w = u.shape
-        out_act = torch.empty_like(u)
-        out_sum = torch.empty_like(u) if (v is not None and want_sum) else None
-        check(lib().lzb_bn_relu_bf16(ptr(u), ptr(v), ptr(scale), ptr(shift), i64(n * h * w), ctypes.c_int32(c),
-                                     ptr(out_sum), ptr(out_act), stream_ptr(u.device)))
-        return out_sum, out_act
+            return False
+        return True
 
     def _conv_bn_relu(self, x, conv: nn.Conv2d, wname: str, bname: str, sname: str, tname: str):
         t = self._t
         if self.use_cudnn_fused:
             return torch.cudnn_convolution_relu(x, t[wname], t[bname], [1, 1], [1, 1], [1, 1], 1)
-        c = F.conv2d(x, conv.weight, None, 1, 1)
-        return self._bn_relu(c, None, t[sname], t[tname], False)[1]
+        return bn_relu(F.conv2d(x, conv.weight, None, 1, 1), None, t[sname], t[tname], False)[1]
 
     def __call__(self, x: torch.Tensor) -> torch.Tensor:
+        return self._forward_tc(x) if self.use_tc else self._forward_library(x)
+
+    def _forward_tc(self, x: torch.Tensor) -> torch.Tensor:
+        # no library fallback: callers pad to 64 channels and 64-board tiles (InferenceNet.new_input), or this raises
+        if not (x.size(1) == 64 and x.size(0) % 64 == 0):
+            raise RuntimeError("the tcgen05 network path takes bf16 [n,64,6,6] channel-padded inputs with n % 64 == 0 "
+                               f"(got {tuple(x.shape)}); use InferenceNet.new_input / InferenceNet.forward, which pad")
+        t, nb = self._t, len(self.model.blocks)
+        # Three persistent activation buffers per batch size -- X (residual stream, updated IN PLACE by conv2's
+        # epilogue: every element is read and rewritten by the same thread), A (the next conv's activated input)
+        # and H (conv1's output) -- so the working set of the trunk is 3 x n x 9.2 KB (113 MB at 4,096 boards)
+        # and stays inside the 126 MB L2 instead of cycling through fresh allocations.
+        n = x.size(0)
+        bufs = self._act.get(n)
+        if bufs is None:
+            bufs = self._act[n] = tuple(torch.empty((n, 128, 6, 6), dtype=torch.bfloat16, device=x.device,
+                                                    memory_format=torch.channels_last) for _ in range(3))
+        bx, ba, bh = bufs
+        # stem conv + stem_bn + ReLU and the first block's bn1 + ReLU in ONE launch (x0 and a0 = the two outputs)
+        conv_bf16(x, t["stem_wp"], bias=t["stem_bf"], relu1=True, scale=t["s1_0"], shift=t["t1_0"], want_out2=True,
+                  out1=bx, out2=ba)
+        for i in range(nb):
+            conv_bf16(ba, t[f"wp1_{i}"], bias=t[f"bf1_{i}"], relu1=True, out1=bh)
+            last = i == nb - 1
+            sn, tn = ("trunk_s", "trunk_t") if last else (f"s1_{i + 1}", f"t1_{i + 1}")
+            conv_bf16(bh, t[f"wp2_{i}"], residual=bx, scale=t[sn], shift=t[tn], want_out1=not last, want_out2=True,
+                      out1=bx, out2=ba)
+        return ba
+
+    def _forward_library(self, x: torch.Tensor) -> torch.Tensor:
         m, t = self.model, self._t
         nb = len(m.blocks)
-        if self.use_tc:
-            # ONE convolution path for the 128-channel network: our tcgen05 kernel, on channel-padded inputs
-            # (InferenceNet.new_input) in whole 64-board tiles.  No library fallback: callers pad, or this raises.
-            if not (x.size(1) == 64 and "stem_wp" in t and nb > 0 and x.size(0) % 64 == 0):
-                raise RuntimeError("the tcgen05 network path takes bf16 [n,64,6,6] channel-padded inputs with n % 64 == 0 "
-                                   f"(got {tuple(x.shape)}); use InferenceNet.new_input / InferenceNet.forward, which pad")
-            # Three persistent activation buffers per batch size -- X (residual stream, updated IN PLACE by conv2's
-            # epilogue: every element is read and rewritten by the same thread), A (the next conv's activated input)
-            # and H (conv1's output) -- so the working set of the trunk is 3 x n x 9.2 KB (113 MB at 4,096 boards)
-            # and stays inside the 126 MB L2 instead of cycling through fresh allocations.
-            n = x.size(0)
-            bufs = self._act.get(n)
-            if bufs is None:
-                bufs = self._act[n] = tuple(torch.empty((n, 128, 6, 6), dtype=torch.bfloat16, device=x.device,
-                                                        memory_format=torch.channels_last) for _ in range(3))
-            bx, ba, bh = bufs
-            # stem conv + stem_bn + ReLU and the first block's bn1 + ReLU in ONE launch (x0 and a0 = the two outputs)
-            conv_bf16(x, t["stem_wp"], bias=t["stem_bf"], relu1=True, scale=t["s1_0"], shift=t["t1_0"], want_out2=True,
-                      out1=bx, out2=ba)
-            for i in range(nb):
-                conv_bf16(ba, t[f"wp1_{i}"], bias=t[f"bf1_{i}"], relu1=True, out1=bh)
-                last = i == nb - 1
-                sn, tn = ("trunk_s", "trunk_t") if last else (f"s1_{i + 1}", f"t1_{i + 1}")
-                conv_bf16(bh, t[f"wp2_{i}"], residual=bx, scale=t[sn], shift=t[tn], want_out1=not last, want_out2=True,
-                          out1=bx, out2=ba)
-            return ba
-        else:
-            xr = self._conv_bn_relu(x, m.stem_conv, "stem_w", "stem_b", "stem_s", "stem_t")  # x0 = relu(stem_bn(conv))
-            if nb == 0:
-                return self._bn_relu(xr, None, t["trunk_s"], t["trunk_t"], False)[1]
-            _, a = self._bn_relu(xr, None, t["s1_0"], t["t1_0"], False)                       # a0 = relu(bn1_0(x0))
+        xr = self._conv_bn_relu(x, m.stem_conv, "stem_w", "stem_b", "stem_s", "stem_t")  # x0 = relu(stem_bn(conv))
+        if nb == 0:
+            return bn_relu(xr, None, t["trunk_s"], t["trunk_t"], False)[1]
+        _, a = bn_relu(xr, None, t["s1_0"], t["t1_0"], False)                            # a0 = relu(bn1_0(x0))
         for i, blk in enumerate(m.blocks):
             h = self._conv_bn_relu(a, blk.conv1, f"w1_{i}", f"b1_{i}", f"s2_{i}", f"t2_{i}")  # relu(bn2(conv1(a)))
             c2 = F.conv2d(h, blk.conv2.weight, None, 1, 1)
             last = i == nb - 1
             sn, tn = ("trunk_s", "trunk_t") if last else (f"s1_{i + 1}", f"t1_{i + 1}")
-            xr, a = self._bn_relu(xr, c2, t[sn], t[tn], not last)       # x' = x + conv2 ; a = relu(bn_next(x'))
+            xr, a = bn_relu(xr, c2, t[sn], t[tn], not last)       # x' = x + conv2 ; a = relu(bn_next(x'))
         return a
 
 
 class FusedHeads:
-    """PolicyHead + ValueHead as ONE cuDNN 1x1 convolution (both heads' conv1 stacked) + our bn_relu epilogue + ONE
-    fused kernel for everything after it (csrc/lz_nn.cu: heads_tail_kernel), optionally fused with the masked
-    softmax over legal actions and the bucket expectation."""
+    """PolicyHead + ValueHead for nets whose heads fit heads_tail_kernel (``heads_kernel_fits``): both heads' 1x1
+    conv1 stacked into ONE convolution with their bn1 + ReLU -- our tcgen05 conv with the BatchNorm folded in, or (not
+    ``tc``) a cuDNN conv + our bn_relu pass -- then ONE fused kernel for everything after it (csrc/lz_nn.cu:
+    heads_tail_kernel), optionally fused with the masked softmax over legal actions and the bucket expectation."""
 
-    def __init__(self, model: "ChessNet"):
+    def __init__(self, model: "ChessNet", tc: bool):
         self.model = model
+        self.use_tc = tc
         ph, vh = model.policy_head, model.value_head
         self.pc, self.vc = ph.conv1.out_channels, vh.conv1.out_channels
         self.mlp, self.bins = vh.fc1.out_features, vh.fc2.out_features
-        self.supported = (self.pc <= 64 and self.vc <= 64 and self.mlp <= 128 and 2 <= self.bins <= 128
-                          and (self.pc + self.vc) % 8 == 0)
         self._t = {}
-        if self.supported:
-            self.refresh()
-
-    def _set(self, name: str, value: torch.Tensor) -> None:
-        if name in self._t:
-            self._t[name].copy_(value)
-        else:
-            self._t[name] = value.contiguous().clone()
+        self.refresh()
 
     def refresh(self) -> None:
         ph, vh = self.model.policy_head, self.model.value_head
         f = lambda x: x.detach().float()  # noqa: E731
-        self._set("conv_w", torch.cat([ph.conv1.weight.detach(), vh.conv1.weight.detach()], 0).contiguous(
-            memory_format=torch.channels_last))
         s1, t1 = _fold_bn(ph.bn1)
         s2, t2 = _fold_bn(vh.bn1)
-        self._set("bn1_scale", torch.cat([s1, s2]))
-        self._set("bn1_shift", torch.cat([t1, t2]))
-        self.use_tc = (self.pc + self.vc == 128 and ph.conv1.in_channels == 128
-                       and ph.conv1.weight.dtype == torch.bfloat16)
+        v = {}
         if self.use_tc:     # both heads' 1x1 convs + their BatchNorm + ReLU as ONE launch of our tcgen05 conv
             wf = torch.cat([ph.conv1.weight.detach(), vh.conv1.weight.detach()], 0).float()
-            self._set("conv_wp", pack_conv_weight(wf * torch.cat([s1, s2]).view(-1, 1, 1, 1)))
-            self._set("conv_bias", torch.cat([t1, t2]).float())
-        self._set("wgl_t", pack_mma_b(f(ph.gpool_linear.weight)))
-        sb, tb = _fold_bn(ph.bn2)
-        self._set("bn2_scale", sb)
-        self._set("bn2_shift", tb)
-        self._set("wout", torch.stack([f(ph.out_pos1.weight).view(-1), f(ph.out_pos2.weight).view(-1),
-                                       f(ph.out_mark.weight).view(-1)]))
-        self._set("wfc1_t", pack_mma_b(f(vh.fc1.weight)))
-        self._set("bfc1", f(vh.fc1.bias))
-        self._set("wfc2_t", pack_mma_b(f(vh.fc2.weight)))
-        self._set("bfc2", f(vh.fc2.bias))
+            v["conv_wp"] = pack_conv_weight(wf * torch.cat([s1, s2]).view(-1, 1, 1, 1))
+            v["conv_bias"] = torch.cat([t1, t2]).float()
+        else:
+            v["conv_w"] = torch.cat([ph.conv1.weight.detach(), vh.conv1.weight.detach()], 0).contiguous(
+                memory_format=torch.channels_last)
+            v["bn1_scale"], v["bn1_shift"] = torch.cat([s1, s2]), torch.cat([t1, t2])
+        v["wgl_t"] = pack_mma_b(f(ph.gpool_linear.weight))
+        v["bn2_scale"], v["bn2_shift"] = _fold_bn(ph.bn2)
+        v["wout"] = torch.stack([f(ph.out_pos1.weight).view(-1), f(ph.out_pos2.weight).view(-1),
+                                 f(ph.out_mark.weight).view(-1)])
+        v["wfc1_t"], v["bfc1"] = pack_mma_b(f(vh.fc1.weight)), f(vh.fc1.bias)
+        v["wfc2_t"], v["bfc2"] = pack_mma_b(f(vh.fc2.weight)), f(vh.fc2.bias)
+        _set(self._t, v)
 
-    def __call__(self, a: Optional[torch.Tensor], states: Optional[torch.Tensor] = None, *, priors_out=None,
-                 values_out=None, want_raw: bool = False, pv: Optional[torch.Tensor] = None):
-        """a: trunk output bf16 [n,C,6,6] channels-last.  With `states` (packed int64[n,4]) returns
-        (priors f32[n,220], values f32[n]); with want_raw returns (log_p1, log_p2, log_pmc, value_logits) fp32."""
-        import ctypes
-
-        from ._lib import check, i64, lib, ptr, stream_ptr
-
+    def __call__(self, a: torch.Tensor, states: Optional[torch.Tensor] = None, *, priors_out=None, values_out=None,
+                 want_raw: bool = False):
+        """a: trunk output bf16 [n,C,6,6] channels-last -> ``tail`` of relu(bn1(conv1(a))) of both heads."""
         t = self._t
-        src = pv if pv is not None else a
-        n = src.size(0)
-        dev = src.device
-        if pv is not None:
-            pass                    # relu(bn1(conv1(a))) of both heads already computed (the fused trunk kernel's last layer)
-        elif self.use_tc:
-            if n % 64 != 0:
+        if self.use_tc:
+            if a.size(0) % 64 != 0:
                 raise RuntimeError("the tcgen05 network path works on whole 64-board tiles (n % 64 == 0)")
             pv, _ = conv_bf16(a, t["conv_wp"], bias=t["conv_bias"], relu1=True)
         else:
-            c = F.conv2d(a, t["conv_w"], None, 1, 0)
-            pv = torch.empty_like(c)
-            check(lib().lzb_bn_relu_bf16(ptr(c), ptr(None), ptr(t["bn1_scale"]), ptr(t["bn1_shift"]), i64(n * 36),
-                                         ctypes.c_int32(self.pc + self.vc), ptr(None), ptr(pv), stream_ptr(dev)))
+            pv = bn_relu(F.conv2d(a, t["conv_w"], None, 1, 0), None, t["bn1_scale"], t["bn1_shift"], False)[1]
+        return self.tail(pv, states, priors_out=priors_out, values_out=values_out, want_raw=want_raw)
+
+    def tail(self, pv: torch.Tensor, states: Optional[torch.Tensor] = None, *, priors_out=None, values_out=None,
+             want_raw: bool = False):
+        """pv: relu(bn1(conv1)) of both heads, bf16 [n,pc+vc,6,6] channels-last.  With `states` (packed int64[n,4])
+        returns (priors f32[n,220], values f32[n]); with want_raw (log_p1, log_p2, log_pmc, value_logits) fp32."""
+        t = self._t
+        n = pv.size(0)
+        dev = pv.device
         log_heads = value_logits = None
         if want_raw:
             log_heads = torch.empty((n, 3, 36), dtype=torch.float32, device=dev)
@@ -442,56 +451,67 @@ class FusedHeads:
 
 
 class InferenceNet:
-    """bf16 / channels-last / CUDA-graph inference wrapper around a ChessNet on one GPU.
+    """bf16 / channels-last / CUDA-graph inference wrapper around a ChessNet on one GPU, on the forward path ``path``
+    (module docstring), fixed at construction.
 
-    ``forward(inputs)`` takes bf16 channels-last planes [n,11,6,6] (as written by ``lzb_encode_inputs_packed``)
-    and returns fp32 (log_p1, log_p2, log_pmc, value_logits).  For batch sizes registered with ``capture``
-    the forward is a graph replay on static buffers (returned tensors alias those buffers)."""
+    ``forward(inputs)`` takes planes [n,C,6,6] (C = the net's input channels, as ``lzb_encode_inputs_packed`` writes
+    them; any float dtype) and returns fp32 (log_p1, log_p2, log_pmc, value_logits).  For batch sizes registered with
+    ``capture`` the forward is a graph replay on static buffers (returned tensors alias those buffers)."""
 
-    def __init__(self, model: ChessNet, device, dtype: torch.dtype = torch.bfloat16, fused: bool = True,
+    def __init__(self, model: ChessNet, device, dtype: torch.dtype = torch.bfloat16, *, path: Optional[str] = None,
                  allow_library_convs: bool = False):
-        """``allow_library_convs``: the product network path is our tcgen05 convolution kernel, which covers the
-        reference's default architecture (128-channel trunk, 64 + 64 head channels, bf16).  Any other ChessNet shape
-        (the tiny nets of unit tests, fp32 parity runs, ``fused=False``) can only run on PyTorch's library convolutions;
-        that is refused unless the caller opts in explicitly -- there is no silent dispatch between the two."""
+        """``path``: None for the default of the net's shape and dtype, or any later path of PATHS (``network_path``).
+        The product paths run our tcgen05 kernels, which cover the reference's default architecture; the library and
+        module paths (the only ones for other shapes: the tiny nets of unit tests, fp32 parity runs) run PyTorch's
+        library convolutions and are refused without ``allow_library_convs``: no silent dispatch between the two."""
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("InferenceNet needs a CUDA device")
         if dev.index is None:
             dev = torch.device("cuda", torch.cuda.current_device())
+        default = network_path(model, dtype)
+        self.path = network_path(model, dtype, path)
+        if self.library_convs and not allow_library_convs:
+            raise RuntimeError(
+                "liuzhou_b200.InferenceNet: this ChessNet shape / dtype / path is not covered by the tcgen05 "
+                "convolution kernel (needs trunk_channels = 128, policy_channels + value_channels = 128, >= 1 block, "
+                "bf16, path 'trunk' or 'layered'); pass allow_library_convs=True to run it on PyTorch's cuDNN "
+                "convolutions instead (tests / parity only)")
         self.device = dev
         self.dtype = dtype
         self.model = self._clone_for_inference(model, dev, dtype)
-        # fused epilogue kernels need bf16 and a channel count that is a multiple of 8
-        self.fused = bool(fused) and dtype == torch.bfloat16 and self.model.stem_conv.out_channels % 8 == 0
-        self.trunk = FusedTrunk(self.model) if self.fused else None
-        self.heads = FusedHeads(self.model) if self.fused else None
-        if self.heads is not None and not self.heads.supported:
-            self.heads = None
-        if self.trunk is not None and self.trunk.use_tc and not (self.heads is not None and self.heads.use_tc):
-            self.trunk.use_tc = False            # the tcgen05 path is all or nothing (trunk and heads convolutions)
-            self.trunk._probe()
+        self.trunk = self.heads = None
+        if self.path != "module":
+            self.trunk = FusedTrunk(self.model, self.padded_input)
+            if heads_kernel_fits(self.model):
+                # a 128 -> 64 + 64 heads conv stays on tcgen05 where library is the default path (no blocks, or > 64
+                # input channels); path="library" on a net the tcgen05 kernels can run puts every conv on cuDNN
+                heads = self.model.policy_head.conv1.out_channels + self.model.value_head.conv1.out_channels
+                tc = self.padded_input or (default == "library" and self.model.stem_conv.out_channels == heads == 128)
+                self.heads = FusedHeads(self.model, tc)
         self.flops_per_state = flops_per_state(self.model)
-        # the whole trunk + heads conv as ONE persistent kernel (csrc/lz_trunk.cu: activations stay in shared memory /
-        # TMEM across all layers) where the net fits it; otherwise one kernel launch per convolution (csrc/lz_conv.cu)
-        self.fused_trunk = (self._tc_ready() and len(self.model.blocks) <= 10
-                            and self.model.num_input_channels <= 16)     # the kernel's stem multiplies 16 input channels
         self._ft = {}
         self._pv = {}
-        if self.fused_trunk:
+        if self.path == "trunk":
             self._pack_fused_trunk()
-        self.library_convs = not self._tc_ready()
-        if self.library_convs and not allow_library_convs:
-            raise RuntimeError(
-                "liuzhou_b200.InferenceNet: this ChessNet shape / dtype is not covered by the tcgen05 convolution kernel "
-                "(needs trunk_channels = 128, policy_channels + value_channels = 128, >= 1 block, bf16, fused=True); "
-                "pass allow_library_convs=True to run it on PyTorch's cuDNN convolutions instead (tests / parity only)")
         self._graphs: Dict[int, Tuple[torch.cuda.CUDAGraph, torch.Tensor, Tuple[torch.Tensor, ...]]] = {}
+
+    @property
+    def fused_trunk(self) -> bool:
+        """Trunk + heads conv run as ONE kernel launch (lzb_trunk_bf16): the trunk path."""
+        return self.path == "trunk"
+
+    @property
+    def library_convs(self) -> bool:
+        return self.path in ("library", "module")
+
+    @property
+    def padded_input(self) -> bool:
+        """Inputs are planes zero-padded to 64 channels, in whole 64-board tiles (``new_input``): the tcgen05 paths."""
+        return self.path in ("trunk", "layered")
 
     @staticmethod
     def _clone_for_inference(model: ChessNet, dev, dtype):
-        import copy
-
         m = copy.deepcopy(model).to(device=dev, dtype=dtype)
         m = m.to(memory_format=torch.channels_last)
         m.eval()
@@ -506,7 +526,6 @@ class InferenceNet:
         and conv2_i (bn1_{i+1} or trunk_bn: scale | shift), then the heads conv (bn1 folded: bias)."""
         t, h = self.trunk._t, self.heads._t
         nb = len(self.model.blocks)
-        dev = self.device
         ws = []
         parts = [t["stem_bf"], t["s1_0"], t["t1_0"]]               # stem: bias | scale | shift
         for i in range(nb):
@@ -515,21 +534,12 @@ class InferenceNet:
             parts += [t[f"bf1_{i}"], t[sn], t[tn]]                   # conv1: bias; conv2: scale | shift
         ws.append(h["conv_wp"])
         parts.append(h["conv_bias"])                                 # heads conv: bias
-        w_trunk = torch.cat(ws, 0).contiguous()
-        params = torch.cat([p_.float().reshape(-1) for p_ in parts]).to(dev).contiguous()
-        for name, val in (("w_trunk", w_trunk), ("params", params)):
-            if name in self._ft:
-                self._ft[name].copy_(val)          # in place: captured CUDA graphs stay valid
-            else:
-                self._ft[name] = val.clone()
+        _set(self._ft, {"w_trunk": torch.cat(ws, 0).contiguous(),
+                        "params": torch.cat([p_.float().reshape(-1) for p_ in parts]).to(self.device).contiguous()})
 
     def _trunk_heads_conv(self, x: torch.Tensor) -> torch.Tensor:
         """planes bf16 [n,64,6,6] channels-last -> relu(bn(conv1)) of both heads, bf16 [n,128,6,6] channels-last: stem,
         every residual block and the heads' 1x1 conv in ONE kernel launch (lzb_trunk_bf16)."""
-        import ctypes
-
-        from ._lib import check, i64, lib, ptr, stream_ptr
-
         n = x.size(0)
         if not (x.size(1) == 64 and x.dtype == torch.bfloat16 and x.is_contiguous(memory_format=torch.channels_last)):
             raise RuntimeError("the fused trunk takes bf16 [n,64,6,6] channel-padded planes in channels_last format "
@@ -550,49 +560,45 @@ class InferenceNet:
             for k, v in state_dict.items():
                 if k in own:
                     own[k].copy_(v.to(device=self.device, dtype=own[k].dtype))
-        if self.trunk is not None:
-            self.trunk.refresh()
-        if self.heads is not None:
-            self.heads.refresh()
-        if self.fused_trunk:
+        for part in (self.trunk, self.heads):
+            if part is not None:
+                part.refresh()
+        if self.path == "trunk":
             self._pack_fused_trunk()
 
     @torch.no_grad()
     def _forward_eager(self, x: torch.Tensor):
         """-> fp32 (log_p1 [n,36], log_p2, log_pmc, value_logits [n,bins])."""
-        if self.trunk is not None:
+        if self.path == "module":
+            lp1, lp2, lpm, vl = self.model(x)
+        else:
             with torch.cuda.device(self.device):
-                if self.fused_trunk:
-                    return self.heads(None, want_raw=True, pv=self._trunk_heads_conv(x))
+                if self.path == "trunk":
+                    return self.heads.tail(self._trunk_heads_conv(x), want_raw=True)
                 a = self.trunk(x)
                 if self.heads is not None:
                     return self.heads(a, want_raw=True)
                 lp1, lp2, lpm = self.model.policy_head(a)
                 vl = self.model.value_head(a)
-        else:
-            lp1, lp2, lpm, vl = self.model(x)
         return lp1.float(), lp2.float(), lpm.float(), vl.float()
 
     @torch.no_grad()
     def forward_priors(self, x: torch.Tensor, states: torch.Tensor, priors_out=None, values_out=None):
-        """Network + head post-processing for the tree search: bf16 planes [n,11,6,6] + packed states int64[n,4] ->
+        """Network + head post-processing for the tree search: planes from ``new_input`` + packed states int64[n,4] ->
         (priors f32[n,220] = softmax over each state's legal actions, values f32[n] = bucket expectation)."""
         with torch.cuda.device(self.device):
-            if self.fused_trunk:
-                return self.heads(None, states, priors_out=priors_out, values_out=values_out,
-                                  pv=self._trunk_heads_conv(x))
-            if self.trunk is not None and self.heads is not None:
+            if self.path == "trunk":
+                return self.heads.tail(self._trunk_heads_conv(x), states, priors_out=priors_out, values_out=values_out)
+            if self.heads is not None:
                 return self.heads(self.trunk(x), states, priors_out=priors_out, values_out=values_out)
-            from .tree import heads_to_priors
-
             lp1, lp2, lpm, vl = self._forward_eager(x)
             return heads_to_priors(states, lp1, lp2, lpm, vl, priors_out=priors_out, values_out=values_out)
 
     def new_input(self, n: int) -> torch.Tensor:
-        """Input buffer for ``encode_inputs(..., "bf16_nhwc", out=...)``: [n,11,6,6] channels-last, or -- when the
-        whole network runs on our tcgen05 convs -- the same planes zero-padded to 64 channels ([n,64,6,6])."""
+        """Input buffer for ``encode_inputs(..., "bf16_nhwc", out=...)``: [n,C,6,6] channels-last, or -- with
+        ``padded_input`` -- the same planes zero-padded to 64 channels ([n,64,6,6])."""
         c = self.model.num_input_channels
-        if self._tc_ready():
+        if self.padded_input:
             if n % 64 != 0:
                 raise RuntimeError(f"the tcgen05 network path works on whole 64-board tiles: pad the batch ({n}) to a "
                                    "multiple of 64")
@@ -617,10 +623,6 @@ class InferenceNet:
             outs = self._forward_eager(x)
         self._graphs[n] = (g, x, outs)
         return x, outs
-
-    def _tc_ready(self) -> bool:
-        return (self.trunk is not None and self.trunk.use_tc and "stem_wp" in self.trunk._t
-                and len(self.model.blocks) > 0 and self.heads is not None and self.heads.use_tc)
 
     @torch.no_grad()
     def _forward_chunked(self, inputs: torch.Tensor, chunk: int = 16384):
@@ -652,13 +654,10 @@ class InferenceNet:
         n = inputs.size(0)
         entry = self._graphs.get(n)
         if entry is None:
-            if self._tc_ready():
-                if n > 0 and inputs.size(1) == self.model.num_input_channels:
-                    return self._forward_chunked(inputs.to(self.device))      # pads rows to 64 and channels to 64
-                x = inputs.to(device=self.device, dtype=self.dtype).contiguous(memory_format=torch.channels_last)
-                return self._forward_eager(x)                                 # already padded, or raises
+            if self.padded_input and n > 0 and inputs.size(1) == self.model.num_input_channels:
+                return self._forward_chunked(inputs.to(self.device))      # pads rows to 64 and channels to 64
             x = inputs.to(device=self.device, dtype=self.dtype).contiguous(memory_format=torch.channels_last)
-            return self._forward_eager(x)
+            return self._forward_eager(x)               # the tcgen05 paths: already padded, or raises
         g, x, outs = entry
         if inputs.data_ptr() != x.data_ptr():
             x.copy_(inputs)

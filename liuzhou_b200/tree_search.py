@@ -140,11 +140,11 @@ class TreeMCTS:
         self._rows.copy_(torch.where(act, rows, torch.full_like(rows, -1)))
         self._live_set = True
 
-    # one network evaluation of the pending leaves + expansion (+ backup).  On the tcgen05 path the network input is
-    # the channel-padded bf16 [n,64,6,6] tensor and the select kernel writes it itself (one launch less per wave); other
-    # nets (allow_library_convs) take the 11-channel input, written by a separate encoding launch.
+    # one network evaluation of the pending leaves + expansion (+ backup).  On the tcgen05 paths (net.padded_input) the
+    # network input x is the channel-padded bf16 [n,64,6,6] tensor and the select kernel writes it itself (one launch
+    # less per wave); other nets (allow_library_convs) take the unpadded input, written by a separate encoding launch.
     def _fused_encode(self, x: torch.Tensor) -> bool:
-        return x.dim() == 4 and x.size(1) == 64 and x.dtype == torch.bfloat16
+        return self.net.padded_input
 
     def _eval_pending(self, root: bool, encoded: bool) -> None:
         tree = self.tree

@@ -69,10 +69,10 @@ def test_conv_is_deterministic_and_border_exact():
     assert torch.equal(y, y2)
 
 
-def test_trunk_and_heads_tc_path_matches_cudnn_path():
+def test_trunk_path_matches_library_path():
     """The whole default ChessNet forward through our tcgen05 convs (20 trunk convs + the heads' 1x1 conv) vs the
-    cuDNN conv + bn_relu path on the same inputs: same folded weights, bf16 activations -> agreement to bf16 noise,
-    and both agree with the fp32 PyTorch module."""
+    same model built with path="library" (cuDNN conv + bn_relu) on the same inputs: same folded weights, bf16
+    activations -> agreement to bf16 noise, and both agree with the fp32 PyTorch module."""
     from liuzhou_b200.net import ChessNet, InferenceNet
 
     torch.manual_seed(5)
@@ -84,7 +84,7 @@ def test_trunk_and_heads_tc_path_matches_cudnn_path():
             m.weight.data.uniform_(0.7, 1.3)
             m.bias.data.normal_(0.0, 0.1)
     net = InferenceNet(model, DEV)
-    assert net.trunk.use_tc and net.heads.use_tc
+    assert net.path == "trunk"
     x64 = net.new_input(128)
     assert x64.size(1) == 64                      # channel-padded input: the stem runs on our conv too
     x = (torch.rand((128, 11, 6, 6), device=DEV) > 0.6).to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
@@ -97,8 +97,8 @@ def test_trunk_and_heads_tc_path_matches_cudnn_path():
     out_pub = net.forward(x.float())                           # the public entry pads rows and channels itself
     for a, b in zip(out_tc, out_pub):
         assert torch.equal(a, b)
-    net.trunk.use_tc = net.heads.use_tc = net.fused_trunk = False
-    out_cudnn = [o.clone() for o in net._forward_eager(x)]
+    cudnn = InferenceNet(model, DEV, path="library", allow_library_convs=True)
+    out_cudnn = [o.clone() for o in cudnn._forward_eager(x)]
     ref = model.to(DEV).float().eval()
     with torch.no_grad():
         out_ref = ref(x.float())
@@ -177,10 +177,11 @@ def test_no_library_convolution_for_any_batch_size():
 
 
 @pytest.mark.parametrize("n,blocks", [(64, 1), (192, 2), (4096, 10), (130 * 64, 3)])
-def test_fused_trunk_kernel_matches_per_layer_path_and_fp32(n, blocks):
+def test_trunk_path_matches_layered_path_and_fp32(n, blocks):
     """lzb_trunk_bf16 (whole trunk + heads conv in one persistent kernel, activations resident in shared memory / TMEM,
-    fp32 residual stream) against the per-layer tcgen05 path (bf16 residual stream) and the fp32 PyTorch module on the
-    same positions: the fused kernel must be at least as close to fp32 as the per-layer path."""
+    fp32 residual stream) against the same model built with path="layered" (one tcgen05 conv per layer, bf16 residual
+    stream) and the fp32 PyTorch module on the same positions: the fused kernel must be at least as close to fp32 as
+    the per-layer path."""
     from liuzhou_b200.net import ChessNet, InferenceNet
 
     torch.manual_seed(17)
@@ -200,8 +201,7 @@ def test_fused_trunk_kernel_matches_per_layer_path_and_fp32(n, blocks):
     again = [o.clone() for o in net._forward_eager(x)]
     for a, b in zip(fused, again):
         assert torch.equal(a, b)                                  # deterministic
-    net.fused_trunk = False
-    layered = [o.clone() for o in net._forward_eager(x)]
+    layered = [o.clone() for o in InferenceNet(model, DEV, path="layered")._forward_eager(x)]
     ref = model.to(DEV).float().eval()
     with torch.no_grad():
         out_ref = [o.float() for o in ref(planes.float())]

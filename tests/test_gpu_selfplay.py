@@ -227,9 +227,10 @@ def test_self_play_entry_format_and_determinism(backend):
     assert torch.equal(batch.state_tensors, b2.state_tensors)
 
 
-def test_fused_trunk_matches_pytorch_forward():
-    """Our fused BatchNorm+ReLU(+residual add) epilogue kernels around the cuDNN convolutions reproduce the plain
-    PyTorch bf16 forward (bf16 rounding tolerance), with non-trivial BatchNorm statistics."""
+def test_library_path_matches_module_path():
+    """The library path -- our fused BatchNorm+ReLU(+residual add) epilogue kernels around the cuDNN convolutions --
+    reproduces the plain PyTorch bf16 forward of the module path (bf16 rounding tolerance), with non-trivial
+    BatchNorm statistics."""
     from liuzhou_b200.net import ChessNet, InferenceNet
 
     torch.manual_seed(3)
@@ -240,8 +241,8 @@ def test_fused_trunk_matches_pytorch_forward():
             m.running_var.uniform_(0.5, 1.5)
             m.weight.data.uniform_(0.5, 1.5)
             m.bias.data.normal_(0.0, 0.2)
-    fused = InferenceNet(model, DEV, fused=True, allow_library_convs=True)
-    plain = InferenceNet(model, DEV, fused=False, allow_library_convs=True)
+    fused = InferenceNet(model, DEV, allow_library_convs=True)
+    plain = InferenceNet(model, DEV, path="module", allow_library_convs=True)
     assert fused.trunk is not None and plain.trunk is None
     x = fused.new_input(257)
     x.copy_((torch.rand(257, 11, 6, 6, device=DEV) > 0.6).to(torch.bfloat16))

@@ -7,7 +7,7 @@ import torch
 import torch.nn.functional as F
 
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
-from liuzhou_b200.net import FusedTrunk, conv_bf16, pack_conv_weight  # noqa: E402
+from liuzhou_b200.net import bn_relu, conv_bf16, pack_conv_weight  # noqa: E402
 
 
 def timeit(fn, reps=50):
@@ -44,7 +44,7 @@ for n in ns:
     print(f"n={n} cuDNN conv+bias+relu          : {t:7.1f} us  {flop / t / 1e6:6.0f} TFLOP/s")
     t = timeit(lambda: conv_bf16(x, wp, bias=bf, relu1=True, out1=o1))
     print(f"n={n} ours  conv+bias+relu          : {t:7.1f} us  {flop / t / 1e6:6.0f} TFLOP/s")
-    t = timeit(lambda: FusedTrunk._bn_relu(res, F.conv2d(x, w, None, 1, 1), sc, sh, True))
+    t = timeit(lambda: bn_relu(res, F.conv2d(x, w, None, 1, 1), sc, sh, True))
     print(f"n={n} cuDNN conv + bn_relu(add,dual): {t:7.1f} us")
     t = timeit(lambda: conv_bf16(x, wp, residual=res, scale=sc, shift=sh, want_out2=True, out1=o1, out2=o2))
     print(f"n={n} ours  conv+residual+bn+relu x2: {t:7.1f} us  {flop / t / 1e6:6.0f} TFLOP/s")
@@ -54,5 +54,5 @@ for n in ns:
         conv_bf16(h, wp, residual=res, scale=sc, shift=sh, want_out2=True, out1=o2, out2=o1)
     def block_cudnn():
         h = torch.cudnn_convolution_relu(x, w, b, [1, 1], [1, 1], [1, 1], 1)
-        FusedTrunk._bn_relu(res, F.conv2d(h, w, None, 1, 1), sc, sh, True)
+        bn_relu(res, F.conv2d(h, w, None, 1, 1), sc, sh, True)
     print(f"n={n} residual block: cuDNN path {timeit(block_cudnn):7.1f} us   ours {timeit(block_ours):7.1f} us")

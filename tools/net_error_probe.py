@@ -1,6 +1,10 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
-from liuzhou_b200.net import ChessNet, InferenceNet
+import sys
+from pathlib import Path
+
+import torch
+
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
+from liuzhou_b200.net import ChessNet, InferenceNet  # noqa: E402
 DEV = "cuda:0"
 for n, blocks in [(64, 1), (192, 2), (4096, 10), (130 * 64, 3)]:
     torch.manual_seed(17)
@@ -14,8 +18,7 @@ for n, blocks in [(64, 1), (192, 2), (4096, 10), (130 * 64, 3)]:
     planes = (torch.rand((n, 11, 6, 6), device=DEV) > 0.6).to(torch.bfloat16)
     x[:, :11] = planes
     fused = [o.clone() for o in net._forward_eager(x)]
-    net.fused_trunk = False
-    layered = [o.clone() for o in net._forward_eager(x)]
+    layered = [o.clone() for o in InferenceNet(model, DEV, path="layered")._forward_eager(x)]
     ref = model.to(DEV).float().eval()
     with torch.no_grad():
         out_ref = [o.float() for o in ref(planes.float())]

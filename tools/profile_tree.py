@@ -6,7 +6,7 @@ import torch
 
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from liuzhou_b200 import native  # noqa: E402
-from liuzhou_b200.net import ChessNet, InferenceNet  # noqa: E402
+from liuzhou_b200.net import ChessNet, InferenceNet, conv_bf16  # noqa: E402
 from liuzhou_b200.tree import encode_inputs  # noqa: E402
 from liuzhou_b200.tree_search import TreeMCTS, TreeMCTSConfig  # noqa: E402
 
@@ -39,14 +39,9 @@ for w in range(waves):
     timed("encode", lambda: encode_inputs(tree.pending_states, "bf16_nhwc", out=x))
     a = timed("trunk (21 convs)", lambda: net.trunk(x))
     t = net.heads._t
-    from liuzhou_b200.net import conv_bf16
     pv = timed("heads conv1x1", lambda: conv_bf16(a, t["conv_wp"], bias=t["conv_bias"], relu1=True)[0])
-    orig = conv_bf16
-    # heads tail with priors: call through FusedHeads but skip its conv by monkeypatching
-    import liuzhou_b200.net as netmod
-    netmod.conv_bf16 = lambda *aa, **kk: (pv, None)
-    timed("heads_tail (+priors)", lambda: net.heads(a, tree.pending_states, priors_out=m._wave_pri, values_out=m._wave_val))
-    netmod.conv_bf16 = orig
+    timed("heads_tail (+priors)", lambda: net.heads.tail(pv, tree.pending_states, priors_out=m._wave_pri,
+                                                          values_out=m._wave_val))
     timed("expand+backup", lambda: tree.complete_pending(m._wave_pri, m._wave_val))
 torch.cuda.synchronize()
 tot = 0.0
