@@ -154,20 +154,29 @@ heads_tail_kernel(HeadsParams P) {
         const int ns = (int)min((int64_t)kTile, P.n - base);
         __syncthreads();
         // 1. global pooling per (state, channel): mean / max / std (biased variance + 1e-6)  neural_network.py:68-81
-        //    thread -> (state, channel octet, half of the board): 18 independent 16-byte loads, one pass (sum, sum of
-        //    squares, max in fp32); the two halves sit in adjacent lanes and meet by shuffle.
+        //    thread -> (state, channel octet, half of the board): 18 independent 16-byte loads, one pass (max in fp32,
+        //    and the sum and sum of squares of d = x - K in fp32); the two halves sit in adjacent lanes and meet by
+        //    shuffle.  The shift K is the channel's value at cell 0, which both halves load: var = E[d^2] - E[d]^2
+        //    then does not cancel on a channel that is nearly constant over the board (E[x^2] - E[x]^2 loses all of
+        //    its bits there), and since d_0 = 0, E[d]^2 <= 36 var bounds the cancellation everywhere.  For bf16 x,
+        //    x - K is exact unless the two magnitudes are more than 2^16 apart.
         {
             const int octets = c2 >> 3, items = kTile * octets * 2;
             for (int idx0 = 0; idx0 < items; idx0 += kHeadsThreads) {
                 const int idx = idx0 + t;
                 const bool valid = idx < items;
                 const int hf = idx & 1, so = idx >> 1, s = valid ? so / octets : 0, o = valid ? so - s * octets : 0;
-                float sm[8], sq[8], mx[8];
+                float sm[8], sq[8], mx[8], k0[8];
 #pragma unroll
-                for (int c = 0; c < 8; ++c) { sm[c] = 0.0f; sq[c] = 0.0f; mx[c] = -INFINITY; }
+                for (int c = 0; c < 8; ++c) { sm[c] = 0.0f; sq[c] = 0.0f; mx[c] = -INFINITY; k0[c] = 0.0f; }
                 if (valid && s < ns) {
-                    const uint4* src = reinterpret_cast<const uint4*>(P.pv + ((base + s) * 36 + hf * 18) * c2 + o * 8);
+                    const uint4* board = reinterpret_cast<const uint4*>(P.pv + (base + s) * 36 * c2 + o * 8);
                     const int stride = c2 >> 3;                    // uint4 per cell
+                    const uint4 raw0 = __ldg(board);
+                    const uint32_t w0[4] = {raw0.x, raw0.y, raw0.z, raw0.w};
+#pragma unroll
+                    for (int h = 0; h < 4; ++h) { k0[2 * h] = __uint_as_float(w0[h] << 16); k0[2 * h + 1] = __uint_as_float(w0[h] & 0xffff0000u); }
+                    const uint4* src = board + hf * 18 * stride;
 #pragma unroll
                     for (int cell = 0; cell < 18; ++cell) {
                         const uint4 raw = __ldg(src + cell * stride);
@@ -175,8 +184,9 @@ heads_tail_kernel(HeadsParams P) {
 #pragma unroll
                         for (int h = 0; h < 4; ++h) {
                             const float lo = __uint_as_float(wv[h] << 16), hi = __uint_as_float(wv[h] & 0xffff0000u);
-                            sm[2 * h] += lo; sq[2 * h] = fmaf(lo, lo, sq[2 * h]); mx[2 * h] = fmaxf(mx[2 * h], lo);
-                            sm[2 * h + 1] += hi; sq[2 * h + 1] = fmaf(hi, hi, sq[2 * h + 1]); mx[2 * h + 1] = fmaxf(mx[2 * h + 1], hi);
+                            const float dl = lo - k0[2 * h], dh = hi - k0[2 * h + 1];
+                            sm[2 * h] += dl; sq[2 * h] = fmaf(dl, dl, sq[2 * h]); mx[2 * h] = fmaxf(mx[2 * h], lo);
+                            sm[2 * h + 1] += dh; sq[2 * h + 1] = fmaf(dh, dh, sq[2 * h + 1]); mx[2 * h + 1] = fmaxf(mx[2 * h + 1], hi);
                         }
                     }
                 }
@@ -191,9 +201,9 @@ heads_tail_kernel(HeadsParams P) {
 #pragma unroll
                     for (int c = 0; c < 8; ++c) {
                         const int ch = o * 8 + c;
-                        const float mean = sm[c] * (1.0f / 36.0f);
-                        const float var = fmaxf(fmaf(-mean, mean, sq[c] * (1.0f / 36.0f)), 0.0f);
-                        const float r0 = live ? mean : 0.0f, r1 = live ? mx[c] : 0.0f, r2 = live ? sqrtf(var + 1e-6f) : 1e-3f;
+                        const float md = sm[c] * (1.0f / 36.0f);
+                        const float var = fmaxf(fmaf(-md, md, sq[c] * (1.0f / 36.0f)), 0.0f);
+                        const float r0 = live ? k0[c] + md : 0.0f, r1 = live ? mx[c] : 0.0f, r2 = live ? sqrtf(var + 1e-6f) : 1e-3f;
                         if (ch < pc) { poolT_p[ch][s] = r0; poolT_p[pc + ch][s] = r1; poolT_p[2 * pc + ch][s] = r2; }
                         else { const int cv = ch - pc; poolT_v[cv][s] = r0; poolT_v[vc + cv][s] = r1; poolT_v[2 * vc + cv][s] = r2; }
                     }

@@ -230,6 +230,15 @@ def fake_net(model_inputs, legal_masks, salt):
     return pri, val
 
 
+def bf16_ulp(x):
+    """One bf16 step (8 significant bits) at |x|, in fp64; 0 at 0.  x: a torch tensor."""
+    import torch
+
+    a = x.double().abs()
+    e = torch.floor(torch.log2(torch.where(a > 0, a, torch.ones_like(a))))
+    return torch.where(a > 0, torch.exp2(e - 7), torch.zeros_like(a))
+
+
 def load_golden(name: str) -> dict:
     with np.load(GOLDEN / f"{name}.npz") as z:
         return {k: z[k] for k in z.files}

@@ -1,12 +1,16 @@
-"""Our tcgen05 implicit-GEMM convolution (csrc/lz_conv.cu) vs a plain PyTorch fp32 reference of the same op on the
-same bf16 inputs.  Tolerance: the kernel accumulates bf16 x bf16 products in fp32 and rounds the outputs to bf16
-once, so |err| <= 2^-8 relative to the output magnitude (+ summation-order noise): rtol = atol = 2e-2."""
+"""Our tcgen05 implicit-GEMM convolution (csrc/lz_conv.cu) vs an fp64 reference of the same op on the same bf16
+inputs.  The kernel multiplies bf16 x bf16 exactly, accumulates the K = cin x taps products in fp32 and rounds each
+output to bf16 once, so |out - ref| <= 1 bf16 step at the output + K * 2^-24 * sum |x| |w| (c = 1 on both terms).  The
+second output reads the first one back: it must be bf16(relu(fmaf(scale, out1, shift))) within one bf16 step."""
 import pytest
 import torch
 import torch.nn.functional as F
 
+from tests._util import bf16_ulp
+
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
+U_FP32 = 2.0 ** -24
 
 
 def _mk(n, seed):
@@ -20,14 +24,70 @@ def _mk(n, seed):
     return x, w, bias, res, scale, shift
 
 
-@pytest.mark.parametrize("n", [64, 192, 4096])
+def _conv_ref64(x, w, chunk=2048):
+    """fp64 conv2d (stride 1, 'same' padding) and its magnitude sum |x| |w|, both [n, cout, 6, 6]."""
+    k = w.size(-1)
+    w2 = w.double().reshape(w.size(0), -1).t()
+    refs, mags = [], []
+    for s in range(0, x.size(0), chunk):
+        cols = F.unfold(x[s:s + chunk].double().contiguous(), kernel_size=k, padding=k // 2).transpose(1, 2)
+        refs.append((cols @ w2).transpose(1, 2))
+        mags.append((cols.abs() @ w2.abs()).transpose(1, 2))
+    shape = (x.size(0), w.size(0), 6, 6)
+    return torch.cat(refs).reshape(shape), torch.cat(mags).reshape(shape)
+
+
+def _assert_conv_bound(out, ref, mag, k, what):
+    """out (bf16) vs the fp64 ref: one bf16 step of the larger of the two + K * 2^-24 * magnitude."""
+    o = out.double()
+    bound = bf16_ulp(torch.maximum(o.abs(), ref.abs())) + k * U_FP32 * mag
+    diff = (o - ref).abs()
+    assert not (diff > bound).any(), (what, int((diff > bound).sum()), float((diff / bound.clamp_min(1e-300)).max()))
+
+
+def _assert_bn_relu_of(out2, out1, scale, shift, what):
+    """out2 == bf16(relu(fmaf(scale, out1, shift))) within one bf16 step (the fp64 product + sum is exact, so its
+    fp32 rounding is the fma's)."""
+    y = (out1.double() * scale.double().view(1, -1, 1, 1) + shift.double().view(1, -1, 1, 1)).float()
+    exp = torch.relu(y).to(torch.bfloat16).double()
+    diff = (out2.double() - exp).abs()
+    assert not (diff > bf16_ulp(exp)).any(), (what, float(diff.max()))
+
+
+@pytest.mark.parametrize("n", [64, 192, 4096, 4736, 16384])
 def test_conv3x3_bias_relu(n):
     from liuzhou_b200.net import conv_bf16, pack_conv_weight
 
     x, w, bias, _, _, _ = _mk(n, 1)
     y, _ = conv_bf16(x, pack_conv_weight(w), bias=bias, relu1=True)
-    ref = torch.relu(F.conv2d(x.float(), w.float(), bias, 1, 1))
-    torch.testing.assert_close(y.float(), ref, rtol=2e-2, atol=2e-2)
+    ref, mag = _conv_ref64(x, w)
+    b = bias.double().view(1, -1, 1, 1)
+    _assert_conv_bound(y, torch.relu(ref + b), mag + b.abs(), 1152, n)
+
+
+@pytest.mark.parametrize("n", [64, 192, 4736, 16384])
+def test_conv_stem_cin64_dual_output(n):
+    """The cin = 64, 9-tap instantiation (the stem on the layered path) with the stem epilogue: out1 = relu(conv + bias)
+    (stem_bn folded), out2 = relu(bn1_0(out1)).  n = 4,736 is 790 pair tiles of 6 boards over 74 clusters, the last
+    one partial."""
+    from liuzhou_b200.net import conv_bf16, pack_conv_weight
+
+    g = torch.Generator(device="cpu").manual_seed(n)
+    x = torch.randn((n, 64, 6, 6), generator=g)
+    x[:, 40:] = (x[:, 40:] > 0.5).float()                           # part of the planes 0 / 1 like the encoded input
+    x = x.to(DEV).to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+    w = (torch.randn((128, 64, 3, 3), generator=g) * 0.05).to(DEV).to(torch.bfloat16)
+    bias = (torch.randn((128,), generator=g) * 0.5).to(DEV)
+    scale = (torch.rand((128,), generator=g) + 0.5).to(DEV)
+    shift = (torch.randn((128,), generator=g) * 0.3).to(DEV)
+    out1, out2 = conv_bf16(x, pack_conv_weight(w), bias=bias, relu1=True, scale=scale, shift=shift, want_out2=True)
+    ref, mag = _conv_ref64(x, w)
+    b = bias.double().view(1, -1, 1, 1)
+    _assert_conv_bound(out1, torch.relu(ref + b), mag + b.abs(), 576, n)
+    _assert_bn_relu_of(out2, out1, scale, shift, n)
+    only2 = conv_bf16(x, pack_conv_weight(w), bias=bias, relu1=True, scale=scale, shift=shift, want_out1=False,
+                      want_out2=True)[1]
+    assert torch.equal(only2, out2)
 
 
 @pytest.mark.parametrize("n", [64, 1024])
@@ -36,10 +96,9 @@ def test_conv3x3_residual_dual_output(n):
 
     x, w, _, res, scale, shift = _mk(n, 2)
     s, a = conv_bf16(x, pack_conv_weight(w), residual=res, scale=scale, shift=shift, want_out2=True)
-    ref_s = F.conv2d(x.float(), w.float(), None, 1, 1) + res.float()
-    torch.testing.assert_close(s.float(), ref_s, rtol=2e-2, atol=2e-2)
-    ref_a = torch.relu(s.float() * scale.view(1, -1, 1, 1) + shift.view(1, -1, 1, 1))     # BN reads the stored sum
-    torch.testing.assert_close(a.float(), ref_a, rtol=1e-2, atol=1e-2)
+    ref, mag = _conv_ref64(x, w)
+    _assert_conv_bound(s, ref + res.double(), mag + res.double().abs(), 1152, n)
+    _assert_bn_relu_of(a, s, scale, shift, n)                                         # BN reads the stored sum
     only_a = conv_bf16(x, pack_conv_weight(w), residual=res, scale=scale, shift=shift, want_out1=False, want_out2=True)[1]
     assert torch.equal(only_a, a)
 
@@ -50,8 +109,9 @@ def test_conv1x1():
     x, w, bias, _, _, _ = _mk(128, 3)
     w1 = w[:, :, 1:2, 1:2].contiguous()
     y, _ = conv_bf16(x, pack_conv_weight(w1), bias=bias, relu1=True)
-    ref = torch.relu(F.conv2d(x.float(), w1.float(), bias))
-    torch.testing.assert_close(y.float(), ref, rtol=2e-2, atol=2e-2)
+    ref, mag = _conv_ref64(x, w1)
+    b = bias.double().view(1, -1, 1, 1)
+    _assert_conv_bound(y, torch.relu(ref + b), mag + b.abs(), 128, "1x1")
 
 
 def test_conv_is_deterministic_and_border_exact():
