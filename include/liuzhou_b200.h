@@ -348,6 +348,34 @@ LZB_API int lzb_heads_tail(const void *pv, int64_t n, int32_t pc, int32_t vc, in
                            const uint64_t *states, float *priors, float *values, float *log_heads,
                            float *value_logits, void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Refilling self-play actor (csrc/lz_actor.cu, liuzhou_b200/actor.py): per-slot game arenas of fixed rows and a
+ * linear output of finished games.  Row format = liuzhou_b200.compact.compact_rows_fixed (42 x i64 = 336 B): words
+ * 0..3 boards of the side to move + phase << 36, 4..7 legal bits, 8..39 64 x f32 policy in ascending legal order,
+ * 40 value | soft value (f32 pair), 41 flags (bit 0 = not representable).
+ * Arena row of (slot g, ply p) = g * max_plies + p; signs i8 / actions i16 arenas are indexed the same way.
+ * ctl u64[48]: [0] output row cursor, [1] output game cursor, [2] next game serial, [3] sticky overflow flags
+ * (1 output capacity, 2 arena), [4] OR of the flags words emitted, [5] block ticket (0 between launches),
+ * [6..8] black wins / white wins / draws, [9..46) games by piece delta (black - white) clamped to [-18, 18].
+ *
+ * lzb_actor_record: for every slot with active[g] != 0, the row of the state BEFORE its move: planes and the
+ * encode_actions_fast legal bits of states u64[G,4], the policy row f32[G,220], value words NaN; signs = +1 black /
+ * -1 white to move; actions = chosen i64[G] (-1 = no move); nrows i32[G] (rows of the game so far) += 1.
+ * lzb_actor_emit: for every slot with finished[g] != 0, in ascending slot order: its nrows[g] rows with word 40 =
+ * (sign * result[g], sign * soft[g]) (f32 products; result / soft from black's perspective) are appended at the row
+ * cursor of out_rows i64[capacity,42] with 16-byte copies, their actions at the same rows of out_actions
+ * i16[capacity], and one record i64[8] = {serial, slot, length, first output row, step, piece delta of states u64[G,4],
+ * result | soft value (f32 pair), 0} at the game cursor of records i64[capacity,8].  A game that does not fit is not
+ * written and sets ctl[3] bit 0.  nrows of the finished slots is reset to 0.  Offsets come from a scan, not from
+ * atomics: the output is bit-reproducible. */
+LZB_API int lzb_actor_record(const uint64_t *states, const uint8_t *active, const float *policy, const int64_t *chosen,
+                             int64_t G, int32_t max_plies, int32_t *nrows, int64_t *arena, int8_t *signs,
+                             int16_t *actions, uint64_t *ctl, void *stream);
+LZB_API int lzb_actor_emit(const uint8_t *finished, const float *result, const float *soft, const uint64_t *states,
+                           int64_t G, int32_t max_plies, int32_t *nrows, const int64_t *arena, const int8_t *signs,
+                           const int16_t *actions, int64_t *out_rows, int16_t *out_actions, int64_t *records,
+                           int64_t capacity, uint64_t *ctl, int64_t step, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -20,9 +20,9 @@ import torch
 from . import native, v0_core
 from .mcts_gpu import TOTAL_ACTION_DIM, GpuStateBatch, V1RootMCTS, V1RootMCTSConfig
 from .net import InferenceNet
+from .compact import expand_rows_fixed
 from .trajectory_buffer import TensorSelfPlayBatch, TensorTrajectoryBuffer
-from .tree import encode_inputs
-from .tree_search import TreeMCTS, TreeMCTSConfig
+from .tree_search import TreeMCTS
 
 _PIECE_DELTA_MIN, _PIECE_DELTA_MAX = -18, 18
 
@@ -78,124 +78,117 @@ def _popcount36(x: torch.Tensor) -> torch.Tensor:
     return pc(x)
 
 
-class _TreeWaveResult:
-    __slots__ = ("planes", "legal", "policy", "value", "soft", "lengths", "result", "piece_delta", "plies_played")
+@dataclass
+class TreePlyRules:
+    """Per-game schedule of a tree-backend self-play ply (the settings of ``self_play_v1_gpu(search_backend="tree")``)."""
+
+    temperature_init: float
+    temperature_final: float
+    temperature_threshold: int
+    add_dirichlet_noise: bool
+    sample_moves: bool
+    opening_random_n: int
+    max_plies: int
+    soft_value_k: float
 
 
-def _play_wave_tree(tree_mcts: TreeMCTS, wave_games: int, *, temperature_init: float, temperature_final: float,
-                    temperature_threshold: int, add_dirichlet_noise: bool, sample_moves: bool, opening_random_n: int,
-                    max_plies: int, soft_value_k: float, live_check_period: int = 4,
-                    progress: Optional[list] = None) -> _TreeWaveResult:
-    """One wave of ``wave_games`` games from the initial position to the end of every game, on the packed layout, with the
-    reference's wave semantics (self_play_gpu_runner.py:159-256: every live game appends one row per ply, no refill,
-    step / finalise rules of module.cpp:632-871) but WITHOUT a host round trip per ply:
+@dataclass
+class TreePly:
+    """What one ply did.  ``states`` / ``plies`` are the values after the moves; ``result`` / ``soft`` (from black's
+    perspective) are meaningful where ``newly`` (the game ended this ply)."""
 
-    * rows of ply p live in slot block [p * G, (p + 1) * G) of preallocated buffers with a validity flag (= the game was
-      live); the finished batch is one ``nonzero`` + ``index_select`` at the end, which yields exactly the reference's
-      append order (ply-major, live games ascending);
-    * results are recorded per game when it ends and broadcast to its rows at the end (finalize_trajectory_inplace,
-      module.cpp:547-630: value = sign x result_from_black, soft = sign x tanh(k (black - white) / 18));
-    * the host looks at the live-game count only every ``live_check_period`` plies; between checks the last count is an
-      upper bound (games never come back), which is all the search needs to pick its network batch bucket: the
-      simulation waves evaluate ceil(live) leaves, not ``wave_games`` (TreeMCTS.set_live / search(live_rows=...)).
-    """
-    dev, g = tree_mcts.device, int(wave_games)
-    states = native.init_states(g, dev)
-    plies = torch.zeros((g,), dtype=torch.int32, device=dev)
-    done = torch.zeros((g,), dtype=torch.bool, device=dev)
-    result = torch.zeros((g,), dtype=torch.float32, device=dev)
-    soft = torch.zeros((g,), dtype=torch.float32, device=dev)
-    cap = max(1, min(int(max_plies), 176))
+    out: object                      # TreeSearchOutput
+    chosen: torch.Tensor             # int64[G] action played (< 0: none)
+    legal_words: torch.Tensor        # int64[G,4] encode_actions_fast legal bits of the states before the move
+    sign: torch.Tensor               # int8[G] +1 black / -1 white to move before the move
+    states: torch.Tensor
+    plies: torch.Tensor
+    move: torch.Tensor               # bool[G] a move was applied
+    newly: torch.Tensor              # bool[G] the game ended this ply
+    result: torch.Tensor             # f32[G]
+    soft: torch.Tensor               # f32[G]
 
-    def alloc(c):
-        return (torch.empty((c * g, 11, 6, 6), dtype=torch.float32, device=dev),
-                torch.empty((c * g, TOTAL_ACTION_DIM), dtype=torch.bool, device=dev),
-                torch.empty((c * g, TOTAL_ACTION_DIM), dtype=torch.float32, device=dev),
-                torch.empty((c * g,), dtype=torch.int8, device=dev),
-                torch.zeros((c * g,), dtype=torch.bool, device=dev))
 
-    planes, legal, policy, sign, valid = alloc(cap)
-    tree_mcts._advanced = False                      # a new wave of games starts from reset roots
+def tree_ply(tree_mcts: TreeMCTS, states: torch.Tensor, plies: torch.Tensor, active: torch.Tensor, rules: TreePlyRules,
+             *, live_rows: Optional[int] = None, restart_states: Optional[torch.Tensor] = None) -> TreePly:
+    """One ply of every active game on the packed layout, without a host synchronisation: the search (and its RNG draws),
+    the legal rows, the forced-uniform opening picks, the step / finish rules of module.cpp:632-871, result and soft
+    value, and the subtree-reuse advance.  The one implementation of these rules: the wave loop of
+    ``self_play_v1_gpu(search_backend="tree")`` and ``SelfPlayActor`` both call it.
+
+    ``live_rows``: a host-side upper bound of the active games; the simulation waves then evaluate only the live trees'
+    leaves (``TreeMCTS.set_live``).  ``restart_states`` int64[G,4]: the games that end this ply start again from these
+    states in the tree (``TreeMCTS.advance`` restart path); None leaves their trees as they are."""
     mask36 = (1 << 36) - 1
-    live_upper, ply = g, 0
-    while ply < int(max_plies) + 1:
-        if ply > 0 and ply % int(live_check_period) == 0:
-            live_upper = int((~done).sum().item())   # the only host synchronisation of the loop
-            if progress is not None:
-                progress.append((ply, live_upper, time.perf_counter()))
-            if live_upper == 0:
-                break
-        if ply >= cap:                               # rare: a game longer than the preallocated block
-            new_cap = min(int(max_plies) + 1, cap + max(16, cap // 2))
-            bigger = alloc(new_cap)
-            for dst, src in zip(bigger, (planes, legal, policy, sign, valid)):
-                dst[: cap * g].copy_(src)
-            planes, legal, policy, sign, valid = bigger
-            cap = new_cap
-        active = ~done
+    if live_rows is not None:
         tree_mcts.set_live(active)
-        temps = torch.where(plies < int(temperature_threshold), float(temperature_init),
-                            float(temperature_final)).to(torch.float32)
-        out = tree_mcts.search(states, active=active, temperatures=temps, add_dirichlet_noise=add_dirichlet_noise,
-                               sample_moves=sample_moves, live_rows=live_upper)
-        if ply == 0:
-            tree_mcts.warm_buckets()                 # first use of this engine: capture the smaller wave batches once
-        chosen = out.chosen_action_indices
-        # legal-mask rows as the reference stores them: v0_core.encode_actions_fast semantics (no game-over check)
-        legal_now = native.mask_words_to_bool(native.legal_masks(states, scalar_semantics=False)[0])
-        if opening_random_n > 0:
-            force = (plies < opening_random_n) & ~out.terminal_mask & active
-            lm = legal_now.to(torch.float32)
-            tot = lm.sum(dim=1, keepdim=True)
-            uni = torch.where(tot > 0, lm / tot.clamp_min(1.0), torch.full_like(lm, 1.0 / TOTAL_ACTION_DIM))
-            chosen = torch.where(force, torch.multinomial(uni, 1).view(-1), chosen)
-        s0 = ply * g
-        encode_inputs(states, "f32_nchw", out=planes[s0:s0 + g])
-        legal[s0:s0 + g] = legal_now
-        policy[s0:s0 + g] = out.policy_dense
-        white_to_move = (states[:, 0] >> 39) & 1                           # meta bit 3 of w0 >> 36
-        sign_now = (1 - 2 * white_to_move).to(torch.int8)
-        sign[s0:s0 + g] = sign_now
-        valid[s0:s0 + g] = active
-        # self_play_step_inplace (module.cpp:632-871) on the packed layout
-        immediate = active & out.terminal_mask                            # no legal action: the side to move loses
-        move = active & ~out.terminal_mask
-        nxt = native.apply_actions(states, chosen.clamp_min(0).to(torch.int32))
-        states = torch.where(move.view(-1, 1), nxt, states).contiguous()
-        plies = plies + move.to(torch.int32)
-        w0, w1 = states[:, 0], states[:, 1]
-        meta = (w0 >> 36) & 0xFFFFFFF
-        phase = meta & 7
-        black, white = _popcount36(w0 & mask36), _popcount36(w1 & mask36)
-        post = (phase == 4) | (phase == 5) | (phase == 7)
-        winner = torch.where(post & (white < 4), 1, torch.where(post & (black < 4), -1, 0))     # :817-824
-        draw = (((meta >> 14) & 255) >= 144) | (((meta >> 22) & 63) >= 36)
-        fin = move & ((winner != 0) | draw | (plies >= int(max_plies)))
-        newly = immediate | fin
-        res_now = torch.where(immediate, -sign_now.to(torch.float32), winner.to(torch.float32))
-        soft_now = torch.tanh((black - white).to(torch.float32) / 18.0 * float(soft_value_k))
-        result = torch.where(newly, res_now, result)
-        soft = torch.where(newly, soft_now, soft)
-        done = done | newly
-        # subtree reuse (portable_cpp_self_play.py:170): the played child becomes the root; finished games keep -1
-        tree_mcts.advance(torch.where(move & ~fin, chosen, torch.full_like(chosen, -1)))
-        ply += 1
-    tree_mcts.set_live(None)
-    tree_mcts.tree.check_capacity()                  # sticky error flags of the whole wave (one blocking read)
-    used = ply * g
-    idx = valid[:used].nonzero().view(-1)
-    game = idx % g
-    sg = sign.index_select(0, idx).to(torch.float32)
-    r = _TreeWaveResult()
-    r.planes, r.legal, r.policy = planes.index_select(0, idx), legal.index_select(0, idx), policy.index_select(0, idx)
-    r.value = sg * result.index_select(0, game)
-    r.soft = sg * soft.index_select(0, game)
-    r.lengths = valid[:used].view(ply, g).sum(dim=0).to(torch.int64)
-    r.result = result
+    temps = torch.where(plies < int(rules.temperature_threshold), float(rules.temperature_init),
+                        float(rules.temperature_final)).to(torch.float32)
+    out = tree_mcts.search(states, active=active, temperatures=temps, add_dirichlet_noise=rules.add_dirichlet_noise,
+                           sample_moves=rules.sample_moves, live_rows=live_rows)
+    if live_rows is not None:
+        tree_mcts.warm_buckets()         # first compacted search of this engine: capture the smaller wave batches once
+    chosen = out.chosen_action_indices
+    # legal-mask rows as the reference stores them: v0_core.encode_actions_fast semantics (no game-over check)
+    legal_words = native.legal_masks(states, scalar_semantics=False)[0]
+    if rules.opening_random_n > 0:
+        force = (plies < rules.opening_random_n) & ~out.terminal_mask & active
+        lm = native.mask_words_to_bool(legal_words).to(torch.float32)
+        tot = lm.sum(dim=1, keepdim=True)
+        uni = torch.where(tot > 0, lm / tot.clamp_min(1.0), torch.full_like(lm, 1.0 / TOTAL_ACTION_DIM))
+        chosen = torch.where(force, torch.multinomial(uni, 1).view(-1), chosen)
+    white_to_move = (states[:, 0] >> 39) & 1                           # meta bit 3 of w0 >> 36
+    sign_now = (1 - 2 * white_to_move).to(torch.int8)
+    # self_play_step_inplace (module.cpp:632-871) on the packed layout
+    immediate = active & out.terminal_mask                            # no legal action: the side to move loses
+    move = active & ~out.terminal_mask
+    nxt = native.apply_actions(states, chosen.clamp_min(0).to(torch.int32))
+    states = torch.where(move.view(-1, 1), nxt, states).contiguous()
+    plies = plies + move.to(torch.int32)
     w0, w1 = states[:, 0], states[:, 1]
-    r.piece_delta = (_popcount36(w0 & mask36) - _popcount36(w1 & mask36)).to(torch.int64)
-    r.plies_played = ply
-    return r
+    meta = (w0 >> 36) & 0xFFFFFFF
+    phase = meta & 7
+    black, white = _popcount36(w0 & mask36), _popcount36(w1 & mask36)
+    post = (phase == 4) | (phase == 5) | (phase == 7)
+    winner = torch.where(post & (white < 4), 1, torch.where(post & (black < 4), -1, 0))     # :817-824
+    draw = (((meta >> 14) & 255) >= 144) | (((meta >> 22) & 63) >= 36)
+    fin = move & ((winner != 0) | draw | (plies >= int(rules.max_plies)))
+    newly = immediate | fin
+    res_now = torch.where(immediate, -sign_now.to(torch.float32), winner.to(torch.float32))
+    soft_now = torch.tanh((black - white).to(torch.float32) / 18.0 * float(rules.soft_value_k))
+    # subtree reuse (portable_cpp_self_play.py:170): the played child becomes the root; finished games keep -1
+    keep = torch.where(move & ~fin, chosen, torch.full_like(chosen, -1))
+    if restart_states is None:
+        tree_mcts.advance(keep)
+    else:
+        tree_mcts.advance(keep, restart_states, newly)
+    return TreePly(out=out, chosen=chosen, legal_words=legal_words, sign=sign_now, states=states, plies=plies, move=move,
+                   newly=newly, result=res_now, soft=soft_now)
+
+
+def _play_wave_tree(actor, rules: TreePlyRules, progress: Optional[list] = None):
+    """One wave of ``actor.num_games`` games from the initial position to the end of every game, with the reference's
+    wave semantics (self_play_gpu_runner.py:159-256: every live game appends one row per ply, no refill, step / finalise
+    rules of module.cpp:632-871): the actor (``SelfPlayActor``) with ``finish()`` before its first step, so no host round
+    trip per ply and the live-game count read every 4 plies (the simulation waves evaluate only the live trees' leaves).
+    -> (rows int64[n, 42] in the reference's append order -- ply-major, live games ascending --, game records, stats).
+    ``progress`` (optional list) receives (ply, live-game upper bound, time) at every live-game count."""
+    g, max_plies = actor.num_games, int(rules.max_plies)
+    actor.rules = rules
+    actor._allocate(max_plies, g * max_plies)        # every game of the wave fits the output
+    actor.reset()
+    actor.finish()
+    while not actor.idle:
+        actor.step()
+        if progress is not None and actor._finish_plies % 4 == 0:
+            progress.append((actor._finish_plies, actor._live_upper, time.perf_counter()))
+    rows, _, rec, stats = actor._take_output()
+    n = int(rows.shape[0])
+    # emission order (game by game) -> ply-major, slot ascending
+    game = torch.repeat_interleave(torch.arange(rec.shape[0], device=rows.device), rec[:, 2], output_size=n)
+    ply = torch.arange(n, device=rows.device) - rec[:, 3].index_select(0, game)
+    order = torch.argsort(ply * g + rec[:, 1].index_select(0, game))
+    return rows.index_select(0, order), rec, stats
 
 
 def self_play_v1_gpu(
@@ -262,43 +255,45 @@ def self_play_v1_gpu(
     evals = 0
 
     if search_backend == "tree":
-        parts = []
+        from .actor import SelfPlayActor
+
+        parts, actor = [], None
         for wave_base in range(0, int(num_games), wave_size):
             wave_games = min(wave_size, int(num_games) - wave_base)
             cache_key = ("tree", id(net), wave_games, sims, float(exploration_weight), bool(add_dirichlet_noise),
                          float(dirichlet_alpha), float(dirichlet_epsilon), bool(sample_moves), int(leaves_per_wave),
                          bool(tree_reuse), policy_target_temperature, float(policy_target_prior_pseudocount))
             if engine_cache is not None and cache_key in engine_cache:
-                tree_mcts = engine_cache[cache_key]
-            if tree_mcts is None or tree_mcts.num_trees != wave_games:
-                tree_mcts = TreeMCTS(net, wave_games, TreeMCTSConfig(
-                    num_simulations=sims, exploration_weight=float(exploration_weight),
+                actor = engine_cache[cache_key]
+            if actor is None or actor.num_games != wave_games:
+                actor = SelfPlayActor(
+                    net, wave_games, device=dev, mcts_simulations=sims, exploration_weight=float(exploration_weight),
                     add_dirichlet_noise=bool(add_dirichlet_noise), dirichlet_alpha=float(dirichlet_alpha),
                     dirichlet_epsilon=float(dirichlet_epsilon), sample_moves=bool(sample_moves),
-                    leaves_per_wave=int(leaves_per_wave), reuse_subtree=bool(tree_reuse),
+                    leaves_per_wave=int(leaves_per_wave), tree_reuse=bool(tree_reuse),
                     policy_target_temperature=policy_target_temperature,
-                    policy_target_prior_pseudocount=float(policy_target_prior_pseudocount)), dev)
+                    policy_target_prior_pseudocount=float(policy_target_prior_pseudocount), max_game_plies=max_plies,
+                    output_capacity=wave_games * max_plies)
                 if engine_cache is not None:
-                    engine_cache[cache_key] = tree_mcts
-            r = _play_wave_tree(tree_mcts, wave_games, temperature_init=float(temperature_init),
-                                temperature_final=float(temperature_final),
-                                temperature_threshold=int(temperature_threshold),
-                                add_dirichlet_noise=bool(add_dirichlet_noise), sample_moves=bool(sample_moves),
-                                opening_random_n=opening_random_n, max_plies=max_plies, soft_value_k=float(soft_value_k))
-            parts.append(r)
-            game_lengths[wave_base:wave_base + wave_games] = r.lengths
-            outcome_counts += torch.stack([(r.result > 0).sum(), (r.result < 0).sum(), (r.result == 0).sum()])
-            piece_delta_hist += torch.bincount(
-                torch.clamp(r.piece_delta - _PIECE_DELTA_MIN, 0, piece_delta_hist.numel() - 1),
-                minlength=piece_delta_hist.numel())
+                    engine_cache[cache_key] = actor
+            rows, rec, wave_stats = _play_wave_tree(actor, TreePlyRules(
+                temperature_init=float(temperature_init), temperature_final=float(temperature_final),
+                temperature_threshold=int(temperature_threshold), add_dirichlet_noise=bool(add_dirichlet_noise),
+                sample_moves=bool(sample_moves), opening_random_n=opening_random_n, max_plies=max_plies,
+                soft_value_k=float(soft_value_k)))
+            parts.append(rows)
+            game_lengths.index_copy_(0, rec[:, 1] + wave_base, rec[:, 2])
+            outcome_counts += torch.tensor([wave_stats.black_wins, wave_stats.white_wins, wave_stats.draws],
+                                           dtype=torch.int64, device=dev)
+            piece_delta_hist += torch.tensor([wave_stats.piece_delta_buckets[str(d)]
+                                              for d in range(_PIECE_DELTA_MIN, _PIECE_DELTA_MAX + 1)],
+                                             dtype=torch.int64, device=dev)
             if verbose:
                 oc = outcome_counts.tolist()
                 print(f"[v1.self_play] games={min(wave_base + wave_games, num_games)}/{num_games} "
                       f"W/L/D={oc[0]}/{oc[1]}/{oc[2]}")
-        cat = (lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs))
-        batch = TensorSelfPlayBatch(cat([r.planes for r in parts]), cat([r.legal for r in parts]),
-                                    cat([r.policy for r in parts]), cat([r.value for r in parts]),
-                                    cat([r.soft for r in parts]))
+        batch = expand_rows_fixed(parts[0] if len(parts) == 1 else torch.cat(parts), check=False)
+        tree_mcts = actor.mcts
         buffer = None
     else:
         buffer = TensorTrajectoryBuffer(dev, TOTAL_ACTION_DIM, max_steps_hint=min(max_plies, 160),
